@@ -1,6 +1,6 @@
 """bench.py — GCN fwd+bwd throughput on botnet-shaped graph batches (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = forward + cross-entropy + backward (+ gradient all-reduce for N>1) + Adam step of the
 12-layer residual GCN (hidden 32) over one batch of `--graphs` synthetic botnet graphs per GPU
@@ -59,7 +59,14 @@ def parse():
     ap.add_argument("--strong-graphs", default="24,25",
                     help="global batch sizes of the strong-scaling measurement (configs[1]: 25 graphs sharded over "
                          "the GPUs by edge count; 24 divides evenly); empty = skip")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the device-resident measurement, write what its last step computed "
+                         "(mean loss, logits, parameter gradients, updated parameters) as DIR/<name>.npy, rank 0's "
+                         "shard, at most 64 MB (beyond that a fixed, seeded sample of the logits rows)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.config != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs --config 1 --impl ours")
+    return args
 
 
 def _gen(args):
@@ -87,6 +94,35 @@ def b_agg(n, e, h):
 
 def b_step(n, e, h, layers):
     return layers * (2 * b_agg(n, e, h) + 4 * n * h)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, loss, logits, model):
+    """--dump-outputs: the step's mean loss, its logits, every parameter's gradient and the parameters after the
+    optimiser step, each as out_dir/<name>.npy in float32.  The logits take what the others leave of DUMP_BYTES; a
+    larger batch keeps a sample of rows drawn with a fixed seed (same rows for the same shape), listed in
+    logits_rows.npy."""
+    import numpy as np
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        arrays[f"grad.{name}"] = p.grad
+        arrays[f"param.{name}"] = p
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    logits = logits.detach().float().cpu().numpy()
+    header = 128        # bytes of an .npy header
+    room = DUMP_BYTES - sum(a.nbytes + header for a in arrays.values()) - 2 * header
+    if logits.nbytes > room:
+        row_bytes = logits.itemsize * logits.shape[1]
+        rows = np.random.default_rng(0).choice(logits.shape[0], room // (row_bytes + 8), replace=False)
+        rows.sort()
+        arrays["logits_rows"] = rows.astype(np.float64)
+        logits = logits[rows]
+    arrays["logits"] = logits
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -246,12 +282,15 @@ def run_ours(args):
     def crit_sum(out, target):   # nn.CrossEntropyLoss(reduction="sum") as deterministic kernels
         return F_mgcn.cross_entropy(out, target, "sum")
 
+    # logits of the latest forward, for --dump-outputs (under a CUDA graph: its output buffer, rewritten by each replay)
+    latest = {}
+
     # model.forward_loss = model(...) + CrossEntropyLoss(reduction="sum") (train_botnet.py:286-287) with the output
     # layer and the loss in one launch (csrc/head.cu); same values as the two separate calls (tests/test_gpu_head.py)
     def step(batch_dev):
         reducer.zero()
-        loss_sum, _logits = model.forward_loss(batch_dev.x[:, 0].view(-1, 1), batch_dev.edge_index, batch_dev.y.long(),
-                                               deg_K=batch_dev.x[:, 1], reduction="sum")
+        loss_sum, latest["logits"] = model.forward_loss(batch_dev.x[:, 0].view(-1, 1), batch_dev.edge_index,
+                                                        batch_dev.y.long(), deg_K=batch_dev.x[:, 1], reduction="sum")
         loss_sum.backward()
         mean_loss, _ = reducer.reduce_mean(loss_sum, batch_dev.num_nodes)
         opt.step()
@@ -259,8 +298,8 @@ def run_ours(args):
 
     def fwd_loss_bwd(batch_dev):
         reducer.zero()
-        loss_sum, _logits = model.forward_loss(batch_dev.x[:, 0].view(-1, 1), batch_dev.edge_index, batch_dev.y.long(),
-                                               deg_K=batch_dev.x[:, 1], reduction="sum")
+        loss_sum, latest["logits"] = model.forward_loss(batch_dev.x[:, 0].view(-1, 1), batch_dev.edge_index,
+                                                        batch_dev.y.long(), deg_K=batch_dev.x[:, 1], reduction="sum")
         loss_sum.backward()
         return loss_sum
 
@@ -276,10 +315,11 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure_resident(batch, steps):
+    def measure_resident(batch, steps, dump_dir=None):
         """structures built once outside the timed region; forward + loss + backward of the fixed-shape batch replayed
         as ONE CUDA graph (meta_gcn_b200/graphed.py), all-reduce and Adam eager; --no-cuda-graph times the eager
-        step.  Returns (ms per step as max over ranks, libmgcn launches in the timed region, graphed?, last loss)."""
+        step.  Returns (ms per step as max over ranks, libmgcn launches in the timed region, graphed?, last loss).
+        With dump_dir, rank 0 writes what the last timed step computed there (dump_outputs)."""
         batch.structure()      # registers the batch boundaries with the structure cache (ordered batches: no sort)
         structure_of(batch.edge_index, batch.num_nodes).fwd_plain
         structure_of(batch.edge_index, batch.num_nodes).bwd_plain
@@ -319,6 +359,8 @@ def run_ours(args):
         ms_ = max_over_ranks(ev0.elapsed_time(ev1)) / steps
         # kernels of libmgcn.so inside the timed region: host-side launches + those replayed from the graph
         n_launch = (_lib.launch_count() - launches0) + (graph_launches * steps if use_graph else 0)
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, loss, latest["logits"], model)
         return ms_, n_launch, use_graph, float(loss.item())
 
     # ---- device-resident arm (weak scaling: every rank its own batch of --graphs graphs) ----
@@ -328,7 +370,7 @@ def run_ours(args):
     batch.structure().fwd_plain
     if rank == 0:
         sampler.start()
-    ms, launches, use_graph, final_loss = measure_resident(batch, args.steps)
+    ms, launches, use_graph, final_loss = measure_resident(batch, args.steps, args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- strong scaling: one GLOBAL batch of G graphs sharded over the ranks ----

@@ -1,5 +1,5 @@
 import cProfile, pstats, os, sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import CFG, make_graphs
 graphs = make_graphs(list(range(25)), 143107, 1_500_000)
 import torch
