@@ -294,6 +294,14 @@ int mgcn_gcn_first_layer_fwd(const float* s, const float* x, int64_t N, int64_t 
                              float* m_next, uint32_t* hmask, void* stream);
 /* out_scale [N] (may be NULL; only with w_next == NULL): x_next rows leave multiplied by it — the input format of
  * mgcn_gcn_layer_fwd_tc below. */
+/* The same with dropout on h (gcn_model.py:92, before the residual add): keep uint32 [N] = this layer's slice of
+ * mgcn_dropout_keep_bits (one word per row, H = 32), keep_scale = 1 / (1 - p):
+ *     h = bit c of keep[i] ? h * keep_scale : 0   (one rounded fp32 multiply);   hmask bit c = (h > 0) — kept and active
+ * keep == NULL: exactly mgcn_gcn_first_layer_fwd.  keep needs w_next == NULL (the streaming pass); else MGCN_ERR_SHAPE. */
+int mgcn_gcn_first_layer_fwd_ex(const float* s, const float* x, int64_t N, int64_t Hin, const float* w_in,
+                                const float* res_w, const float* res_b, const float* w_next, const float* pre,
+                                const float* post, const float* out_scale, const uint32_t* keep, float keep_scale,
+                                int act_out, int64_t H, float* x_next, float* m_next, uint32_t* hmask, void* stream);
 
 /* One residual GCN layer forward at hidden 32, AGGREGATE-THEN-TRANSFORM, on tcgen05.mma / tensor memory
  * (csrc/gcn_fwd_tc.cu) — the default of the hidden-32 stack.  Same reference lines as mgcn_gcn_layer_fwd
@@ -311,6 +319,15 @@ int mgcn_gcn_layer_fwd_tc(const mgcn_csr_t* g, const float* z, int64_t n_in, con
                           const float* res_b, const float* bias, const float* in_scale, const float* post,
                           const float* out_scale, int act_out, int64_t H, float* z_next, uint32_t* hmask,
                           void* workspace, size_t* workspace_bytes, void* stream);
+/* The same layer with dropout on h, applied in the epilogue (hub rows included): keep uint32 [N] = this layer's slice of
+ * mgcn_dropout_keep_bits, keep_scale = 1 / (1 - p):
+ *     h_i = bit c of keep[i] ? h_i * keep_scale : 0   (one rounded fp32 multiply, as torch's dropout);  hmask bit c = (h > 0)
+ * so the mask word carries kept * relu'(h) and the backward entry points need no change: the caller multiplies the
+ * `post` it passes to them by keep_scale.  keep == NULL: exactly mgcn_gcn_layer_fwd_tc. */
+int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int64_t n_in, const float* w, const float* res_w,
+                             const float* res_b, const float* bias, const float* in_scale, const float* post,
+                             const float* out_scale, const uint32_t* keep, float keep_scale, int act_out, int64_t H,
+                             float* z_next, uint32_t* hmask, void* workspace, size_t* workspace_bytes, void* stream);
 /* The same layer with the A operands of its products in TENSOR MEMORY (csrc/gcn_fwd_tm.cu): the gather lanes write
  * their sums with tcgen05.st.16x256b, the products are tcgen05.mma with A from TMEM — no operand image passes
  * through shared memory (the layer kernels are bound by the LSU data pipe).  Same contract, same results within
@@ -358,6 +375,24 @@ int mgcn_gcn_layer_bwd_fused(const mgcn_csr_t* gt, const float* gs, const float*
 /* gs[i,c] = post[i] * gy[i,c] * bit c of bits[i]   (H = 32; post may be NULL) */
 int mgcn_mask_bits_scale(const float* gy, const uint32_t* bits, const float* post, int64_t N,
                          int64_t H, float* gs, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Dropout keep masks of the residual stack — nn.Dropout(p) of gcn_model.py:92 on every layer's h, as bits.
+ * keep uint32 [L][N][W] (W words per row, W >= ceil(H/32)); bit b of keep[l][n][w] = column 32w + b of row n in layer l
+ * is kept.  A pure function of (seed, l, n, column), independent of the launch configuration:
+ *   key      (k0, k1) = (low 32 bits, high 32 bits) of seed[0] (ONE int64 in device memory: drawn on the device, so a
+ *            captured CUDA graph draws anew on every replay)
+ *   calls    for j = 0..3:  (r0, r1, r2, r3) = Philox4x32-10(counter = (n, l, 4w + j, 0), key)
+ *   draws    r_i & 0xffff is column 32w + 8j + 2i, r_i >> 16 is column 32w + 8j + 2i + 1
+ *   rule     kept iff draw >= t, t = nearest integer to p * 65536 (ties to even)
+ * The keep probability is 1 - t / 65536, within 2^-17 of 1 - p (exact for p = k / 65536, e.g. 0.5); 16-bit draws
+ * give 4 Philox calls per 32-column word instead of 8.  p outside [0, 1] or t = 65536 (nothing kept): MGCN_ERR_SHAPE.
+ * One launch for all L layers. */
+int mgcn_dropout_keep_bits(const int64_t* seed, int64_t L, int64_t N, int64_t W, float p, uint32_t* keep,
+                           void* stream);
+/* h[n,c] = bit (c % 32) of keep[n*W + c/32] ? h[n,c] * scale : 0, in place (H % 4 == 0, W >= ceil(H/32)): dropout on the
+ * saved h of the generic stack (widths 16..128); its ReLU mask is then h > 0. */
+int mgcn_dropout_apply(float* h, const uint32_t* keep, int64_t N, int64_t H, int64_t W, float scale, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Segment reductions — global_mean_pool / global_add_pool (kernel/gcn.py:29, gin.py:44,

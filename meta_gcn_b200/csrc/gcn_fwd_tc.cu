@@ -88,6 +88,8 @@ struct FwdTcArgs {
   const float* in_scale;    // [N] or NULL
   const float* post;        // [N] or NULL
   const float* out_scale;   // [N] or NULL
+  const uint32_t* keep;     // [N] dropout keep bits of this layer, or NULL (no dropout)
+  float keep_scale;         // 1 / (1 - p)
   float* z_next;            // [N, 32]
   uint32_t* hmask;          // [N]
   float* partial;           // [seg_cap, 32]
@@ -371,6 +373,7 @@ __global__ void __launch_bounds__(kFtThreads, 1) k_gcn_fwd_tc(const FwdTcArgs a)
       const float4 sc4 = scal[(tl % (2 * kFtStages)) * kFtRows + r];
       const float postv = sc4.x, inv = sc4.y, outs = sc4.z;
       const int row = __float_as_int(sc4.w);
+      const uint32_t kept = (a.keep && row >= 0) ? __ldg(a.keep + row) : 0xffffffffu;
       const uint32_t ta = tmem + stage * 128 + ((uint32_t)(32 * warp) << 16);
       uint32_t bits = 0;
 #pragma unroll
@@ -389,6 +392,9 @@ __global__ void __launch_bounds__(kFtThreads, 1) k_gcn_fwd_tc(const FwdTcArgs a)
           const float v2 = __uint_as_float(m2[t]) + __uint_as_float(c2[t]);
           float h = __fmul_rn(postv, v1) + vec[32 + c];
           h = h > 0.f ? h : 0.f;
+          // dropout: one rounded multiply (no contraction into the add below), as torch's dropout; a dropped entry is
+          // one more cleared bit of the ReLU mask word
+          if (a.keep) h = ((kept >> c) & 1u) ? __fmul_rn(h, a.keep_scale) : 0.f;
           bits |= (h > 0.f ? 1u : 0u) << c;
           float y = h + (__fmul_rn(inv, v2) + vec[c]);
           if (a.act_out == 1) y = y > 0.f ? y : 0.f;
@@ -429,6 +435,15 @@ extern "C" int mgcn_gcn_layer_fwd_tc(const mgcn_csr_t* g, const float* z, int64_
                                      const float* in_scale, const float* post, const float* out_scale, int act_out,
                                      int64_t H, float* z_next, uint32_t* hmask, void* workspace,
                                      size_t* workspace_bytes, void* stream) {
+  return mgcn_gcn_layer_fwd_tc_ex(g, z, n_in, w, res_w, res_b, bias, in_scale, post, out_scale, nullptr, 1.f, act_out,
+                                  H, z_next, hmask, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int64_t n_in, const float* w,
+                                        const float* res_w, const float* res_b, const float* bias,
+                                        const float* in_scale, const float* post, const float* out_scale,
+                                        const uint32_t* keep, float keep_scale, int act_out, int64_t H, float* z_next,
+                                        uint32_t* hmask, void* workspace, size_t* workspace_bytes, void* stream) {
   MGCN_REQUIRE(workspace_bytes != nullptr && g != nullptr, MGCN_ERR_NULL);
   MGCN_REQUIRE(H == kGH, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(act_out == 0 || act_out == 1, MGCN_ERR_SHAPE);
@@ -457,6 +472,7 @@ extern "C" int mgcn_gcn_layer_fwd_tc(const mgcn_csr_t* g, const float* z, int64_
   a.hub_threshold = g->hub_threshold;
   a.z = z; a.w = w; a.res_w = res_w; a.res_b = res_b; a.bias = bias;
   a.in_scale = in_scale; a.post = post; a.out_scale = out_scale;
+  a.keep = keep; a.keep_scale = keep_scale;
   a.z_next = z_next; a.hmask = hmask; a.partial = partial;
   a.n_rows = g->n_rows;
   a.seg_cap = hubs ? g->seg_cap : 0;

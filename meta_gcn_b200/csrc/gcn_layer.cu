@@ -91,6 +91,8 @@ struct LayerFwdArgs {
   const float* nw;          // [nhin][32] weight_node of the first layer (in, out)
   const float* npost;       // [N] per-target factor or NULL
   int nhin;
+  const uint32_t* keep;     // [N] dropout keep bits (streaming first layer only), or NULL
+  float keep_scale;         // 1 / (1 - p)
   float* x_next;            // [N, 32]
   float* m_next;            // [N, 32] (with w_next)
   uint32_t* hmask;          // [N]
@@ -516,6 +518,7 @@ __global__ void __launch_bounds__(256) k_first_layer_fwd_stream(const LayerFwdAr
     }
     const float ps = a.npost ? __ldg(a.npost + row) : 1.f;
     const float os = a.out_scale ? __ldg(a.out_scale + row) : 1.f;
+    const uint32_t kept = a.keep ? __ldg(a.keep + row) >> col : 0xffu;
     uint32_t bits = 0;
     float o[8];
 #pragma unroll
@@ -523,6 +526,7 @@ __global__ void __launch_bounds__(256) k_first_layer_fwd_stream(const LayerFwdAr
       float h = z.v[q] * ps;
       if (a.bias) h = __fadd_rn(h, __ldg(a.bias + col + q));
       h = h > 0.f ? h : 0.f;
+      if (a.keep) h = ((kept >> q) & 1u) ? __fmul_rn(h, a.keep_scale) : 0.f;   // dropout (see gcn_fwd_tc.cu)
       bits |= (h > 0.f ? 1u : 0u) << q;
       float v = h + (rs.v[q] + nws[256 + col + q]);
       if (a.act_out == 1) v = v > 0.f ? v : 0.f;
@@ -1069,7 +1073,17 @@ extern "C" int mgcn_gcn_first_layer_fwd(const float* s, const float* x, int64_t 
                                         const float* res_w, const float* res_b, const float* w_next,
                                         const float* pre, const float* post, const float* out_scale, int act_out,
                                         int64_t H, float* x_next, float* m_next, uint32_t* hmask, void* stream) {
+  return mgcn_gcn_first_layer_fwd_ex(s, x, N, Hin, w_in, res_w, res_b, w_next, pre, post, out_scale, nullptr, 1.f,
+                                     act_out, H, x_next, m_next, hmask, stream);
+}
+
+extern "C" int mgcn_gcn_first_layer_fwd_ex(const float* s, const float* x, int64_t N, int64_t Hin, const float* w_in,
+                                           const float* res_w, const float* res_b, const float* w_next,
+                                           const float* pre, const float* post, const float* out_scale,
+                                           const uint32_t* keep, float keep_scale, int act_out, int64_t H,
+                                           float* x_next, float* m_next, uint32_t* hmask, void* stream) {
   MGCN_REQUIRE(H == kH, MGCN_ERR_SHAPE);
+  MGCN_REQUIRE(!(keep && w_next), MGCN_ERR_SHAPE);   // dropout only in the streaming pass
   MGCN_REQUIRE(Hin >= 1 && Hin <= 4, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(act_out == 0 || act_out == 1, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(N >= 0 && N < (int64_t(1) << 31), MGCN_ERR_RANGE);
@@ -1080,6 +1094,7 @@ extern "C" int mgcn_gcn_first_layer_fwd(const float* s, const float* x, int64_t 
   MGCN_REQUIRE(aligned16(x_next) && (!m_next || aligned16(m_next)), MGCN_ERR_ALIGN);
   LayerFwdArgs a{};
   a.ns = s; a.nx = x; a.nw = w_in; a.npost = post; a.nhin = (int)Hin;
+  a.keep = keep; a.keep_scale = keep_scale;
   a.resid = x_next;   // row-local mode with a finished residual term: the tail reads it from the tile, never from here
   a.res_w = res_w; a.res_b = res_b; a.w_next = w_next; a.pre = pre; a.out_scale = out_scale;
   a.x_next = x_next; a.m_next = m_next; a.hmask = hmask;

@@ -29,19 +29,46 @@ FORWARD_AGGREGATE_FIRST = True
 BWD_FUSED = os.environ.get("MGCN_BWD_FUSED", "0") == "1"
 
 
+def dropout_seed(device):
+    """The seed of one forward's dropout masks: one int64 drawn on the device from torch's CUDA generator, so
+    torch.manual_seed / torch.cuda.set_rng_state reproduce it and every replay of a captured CUDA graph draws anew.
+    The only source of randomness of the stack (a test pins the masks by replacing this function)."""
+    return torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), device=device, dtype=torch.int64)
+
+
+def _dropout_masks(x, L, W, p):
+    """(keep int32 [L, N, W], scale 1 / (1 - p)) for 0 < p < 1, else (None, None): the masks of all L layers in one
+    launch (csrc/dropout.cu); dropped with the forward's locals — the backward reads only the saved ReLU masks"""
+    if not p:
+        return None, None
+    keep = ops.dropout_keep_bits_impl(dropout_seed(x.device), L, x.size(0), W, p)
+    return keep, 1.0 / (1.0 - p)
+
+
+def _scaled_post(post, scale, n, like):
+    """the per-target factor of the backward with the dropout scale folded in: kept * relu'(h) is in the mask, the scale
+    rides on the row vector the backward multiplies by anyway (exact at p = 0.5, one rounding otherwise)"""
+    if scale is None:
+        return post
+    return post * scale if post is not None else torch.full((n,), scale, dtype=torch.float32, device=like.device)
+
+
 class _ResidualGCNStack(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, graph, pre, post, has_bias, last_relu, *params):
+    def forward(ctx, x, graph, pre, post, has_bias, last_relu, p, *params):
         per = 4 if has_bias else 3
         L = len(params) // per
         layers = [params[i * per:(i + 1) * per] for i in range(L)]
         xs, hs = [x.contiguous()], []
         fwd = graph.fwd_plain
+        keep, scale = _dropout_masks(x, L, (max(lp[0].size(1) for lp in layers) + 31) // 32, p)
         xw = ops.linear_impl(xs[0], layers[0][0], False, row_scale=pre)
         for n, lp in enumerate(layers):
             w, b = lp[0], (lp[1] if has_bias else None)
             res_w, res_b = lp[-2], lp[-1]
             h = ops.aggregate_prescaled_impl(fwd, xw, post, 0, b, None, 1)
+            if keep is not None:
+                ops.dropout_apply_impl(h, keep[n], scale)      # saved as dropped: its ReLU mask is h > 0
             relu_out = last_relu or n < L - 1
             xn = ops.linear_impl(xs[n], res_w, True, res_b, h, 1 if relu_out else 0)
             hs.append(h)
@@ -50,6 +77,12 @@ class _ResidualGCNStack(torch.autograd.Function):
                 xw = ops.linear_impl(xn, layers[n + 1][0], False, row_scale=pre)
         ctx.graph, ctx.cfg = graph, (L, per, has_bias, last_relu)
         ctx.pre, ctx.post = pre, post
+        # dropout scale of the backward: on the node-model output before the bias gradient is taken, else with post
+        ctx.unit_scale = None
+        if scale is not None and has_bias:
+            ctx.unit_scale = torch.full((x.size(0),), scale, dtype=torch.float32, device=x.device)
+        elif scale is not None:
+            ctx.post = _scaled_post(post, scale, x.size(0), x)
         ctx.save_for_backward(*xs, *hs, *params)
         return xs[-1]
 
@@ -71,7 +104,7 @@ class _ResidualGCNStack(torch.autograd.Function):
             need_dx = n > 0 or need_x
             dxres = ops.linear_impl(g, res_w, False, xmask=omask) if need_dx else None
             if has_bias:
-                gsu = ops.masked_scale_impl(g, omask, hs[n], None)
+                gsu = ops.masked_scale_impl(g, omask, hs[n], ctx.unit_scale)
                 grads[n * per + 1] = gsu.sum(0)
                 gs = ops.masked_scale_impl(gsu, None, None, post) if post is not None else gsu
             else:
@@ -82,7 +115,7 @@ class _ResidualGCNStack(torch.autograd.Function):
             grads[n * per + per - 1] = d_res_b
             if need_dx:
                 g = ops.linear_impl(dxw, w, True, add=dxres)
-        return (g if need_x else None, None, None, None, None, None, *grads)
+        return (g if need_x else None, None, None, None, None, None, None, *grads)
 
 
 class _ResidualGCNStack32(torch.autograd.Function):
@@ -169,7 +202,7 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
     the masked gradient, then the row-local tcgen05 launch."""
 
     @staticmethod
-    def forward(ctx, x, graph, pre, post, last_relu, *params):
+    def forward(ctx, x, graph, pre, post, last_relu, p, *params):
         L = len(params) // 3
         layers = [params[i * 3:(i + 1) * 3] for i in range(L)]
         fwd = graph.fwd_plain
@@ -177,6 +210,9 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         sigma = None
         if pre is not None:
             sigma = torch.where(pre > 0, pre, torch.ones_like(pre))
+        # dropout: applied in the layer kernels' epilogues, the dropped entries cleared in the ReLU mask words
+        keep, scale = _dropout_masks(x0, L, 1, p)
+        drop = (lambda n: {"keep": keep[n], "keep_scale": scale}) if keep is not None else (lambda n: {})
         zs, hmasks = [], []
         agg_first = x0.size(1) <= 4
         s0 = None
@@ -185,7 +221,7 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             s0 = ops.spmm_impl(fwd, xs0)                                      # [N, H_in]
             z, _, hm = ops.gcn_first_layer_fwd_impl(
                 s0, x0, layers[0][0], layers[0][1], layers[0][2], None, None, post,
-                1 if (last_relu or L > 1) else 0, out_scale=sigma if L > 1 else None)
+                1 if (last_relu or L > 1) else 0, out_scale=sigma if L > 1 else None, **drop(0))
             zs.append(None)
             hmasks.append(hm)
             first = 1
@@ -196,11 +232,12 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             zs.append(z)
             z, hm = ops.gcn_layer_fwd_tc_impl(
                 fwd, z, layers[n][0], layers[n][1], layers[n][2], None, sigma, post,
-                sigma if n < L - 1 else None, 1 if (last_relu or n < L - 1) else 0)
+                sigma if n < L - 1 else None, 1 if (last_relu or n < L - 1) else 0, **drop(n))
             hmasks.append(hm)
         ctx.agg_first = agg_first
         ctx.graph, ctx.cfg = graph, (L, last_relu)
-        ctx.save_for_backward(x0, s0, pre, post, sigma, z if last_relu else None,
+        # the backward reads `post` only where it scales a gradient by the mask words: the dropout scale goes there
+        ctx.save_for_backward(x0, s0, pre, _scaled_post(post, scale, x0.size(0), x0), sigma, z if last_relu else None,
                               *[t for t in zs if t is not None], *hmasks, *params)
         return z
 
@@ -240,16 +277,24 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         if ctx.agg_first:
             grads[1], grads[2] = ops.linear_wgrad_impl(x0, gy, True, True)
             grads[0] = ops.linear_wgrad_impl(s0, gs, False, False)[0]    # dW0 = s0^T gs0
-        return (None, None, None, None, None, *grads)
+        return (None, None, None, None, None, None, *grads)
 
 
-def residual_gcn_stack(x, graph, pre, post, layer_params, has_bias, last_relu=False, aggregate_first=True):
+def residual_gcn_stack(x, graph, pre, post, layer_params, has_bias, last_relu=False, aggregate_first=True,
+                       dropout=0.0):
     """layer_params: per layer (weight_node [Hin,H], [bias [H]], residual.weight [H,Hin],
-    residual.bias [H]).  pre/post: per-source / per-target degree factors (either may be None)."""
+    residual.bias [H]).  pre/post: per-source / per-target degree factors (either may be None).
+    dropout: p of nn.Dropout on every layer's node-model output (0 <= p < 1; pass 0 outside training).
+    Returns None where the stack does not take dropout (the round-1 hidden-32 kernels, chosen for an x that requires
+    grad or a degree with zeros): the caller then composes the layers one by one."""
+    if not 0.0 <= dropout < 1.0:
+        raise ValueError(f"dropout must be in [0, 1), got {dropout}")
     flat = [p for lp in layer_params for p in lp]
     widths = {lp[0].size(1) for lp in layer_params} | {lp[0].size(0) for lp in layer_params[1:]}
     if not has_bias and widths == {32}:
         if FORWARD_AGGREGATE_FIRST and aggregate_first and not x.requires_grad and (x.size(1) <= 4 or x.size(1) == 32):
-            return _ResidualGCNStack32AT.apply(x, graph, pre, post, last_relu, *flat)
+            return _ResidualGCNStack32AT.apply(x, graph, pre, post, last_relu, dropout, *flat)
+        if dropout > 0:
+            return None
         return _ResidualGCNStack32.apply(x, graph, pre, post, last_relu, *flat)
-    return _ResidualGCNStack.apply(x, graph, pre, post, has_bias, last_relu, *flat)
+    return _ResidualGCNStack.apply(x, graph, pre, post, has_bias, last_relu, dropout, *flat)

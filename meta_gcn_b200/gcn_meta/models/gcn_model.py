@@ -108,12 +108,13 @@ class GCNModel(nn.Module):
 
     def _stack_eligible(self, edge_index_K, edge_attr_K, edge_weight_K):
         """the whole-stack path covers the botnet configuration family (train_botnet.py:200-212):
-        one edge set, additive node models, residual every layer, ReLU/ReLU, sum aggregation"""
+        one edge set, additive node models, residual every layer, ReLU/ReLU, sum aggregation, dropout p < 1
+        (p = 1 drops everything: torch's dropout returns zeros, the per-layer path keeps that)"""
         if self.residual_hop != 1 or getattr(self, "num_residuals", 0) != self.num_layers:
             return False
         if self.non_linear_layer_wise != "relu" or self._res_act != "relu":
             return False
-        if self.training and self.dropout.p > 0:
+        if self.training and self.dropout.p >= 1:
             return False
         if edge_attr_K is not None or edge_weight_K is not None:
             return False
@@ -145,7 +146,9 @@ class GCNModel(nn.Module):
             nm = layer.gcn.node_models[0]
             params.append((nm.weight_node, nm.bias, lin.weight, lin.bias) if has_bias
                           else (nm.weight_node, lin.weight, lin.bias))
-        return fused.residual_gcn_stack(x, graph, pre, post, params, has_bias, aggregate_first=aggregate_first)
+        # None: the stack chosen for these inputs does not take dropout (fused.residual_gcn_stack)
+        return fused.residual_gcn_stack(x, graph, pre, post, params, has_bias, aggregate_first=aggregate_first,
+                                        dropout=self.dropout.p if self.training else 0.0)
 
     def forward(self, x, edge_index_K, edge_attr_K=None, deg_K=None, edge_weight_K=None, **kwargs):
         hidden = kwargs.pop("_hidden", False)        # forward_loss: stop before the output layer
@@ -153,8 +156,9 @@ class GCNModel(nn.Module):
         if self._stack_eligible(edge_index_K, edge_attr_K, edge_weight_K) and not kwargs.get("_no_stack"):
             ei = edge_index_K if isinstance(edge_index_K, torch.Tensor) else edge_index_K[0]
             deg = deg_K if isinstance(deg_K, torch.Tensor) or deg_K is None else deg_K[0]
-            x = self._forward_stack(x, ei, dis, deg)
-            return x if hidden else self._head(x, kwargs)
+            out = self._forward_stack(x, ei, dis, deg)
+            if out is not None:
+                return out if hidden else self._head(out, kwargs)
         kwargs.pop("_no_stack", None)
         hop = self.residual_hop
         xr_src, add_xr_at, res_idx = None, -1, -1

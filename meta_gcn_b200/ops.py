@@ -477,10 +477,12 @@ def gcn_layer_fwd_impl(csr, m, x, resid, res_w, res_b, w_next, bias, pre, post, 
     return x_next, m_next, hmask
 
 
-def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_out, out_scale=None):
-    """first layer with a narrow input (mgcn_gcn_first_layer_fwd): s = aggregated input [N,Hin], x = layer input
-    [N,Hin]; returns (x_next [N,32], m_next | None, hmask int32[N]); out_scale [N]: x_next rows leave scaled"""
-    _need_cuda(s, x, w_in, res_w, res_b, w_next, pre, post, out_scale)
+def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_out, out_scale=None, keep=None,
+                             keep_scale=1.0):
+    """first layer with a narrow input (mgcn_gcn_first_layer_fwd_ex): s = aggregated input [N,Hin], x = layer input
+    [N,Hin]; returns (x_next [N,32], m_next | None, hmask int32[N]); out_scale [N]: x_next rows leave scaled;
+    keep int32 [N] (w_next None only): dropout keep bits of the layer, kept entries of h multiplied by keep_scale"""
+    _need_cuda(s, x, w_in, res_w, res_b, w_next, pre, post, out_scale, keep)
     out_scale = _f32c(out_scale, "out_scale")
     s = _f32c(s, "s")
     x = _f32c(x, "x")
@@ -498,10 +500,21 @@ def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_ou
     x_next = torch.empty(N, H, dtype=torch.float32, device=dev)
     m_next = torch.empty(N, H, dtype=torch.float32, device=dev) if w_next is not None else None
     hmask = torch.empty(N, dtype=torch.int32, device=dev)
-    _lib.check(_lib.load().mgcn_gcn_first_layer_fwd(
+    keep = _keep_rows(keep, N, 1)
+    _lib.check(_lib.load().mgcn_gcn_first_layer_fwd_ex(
         _ptr(s), _ptr(x), N, Hin, _ptr(w_in), _ptr(res_w), _ptr(res_b), _ptr(w_next), _ptr(pre), _ptr(post),
-        _ptr(out_scale), int(act_out), H, _ptr(x_next), _ptr(m_next), _ptr(hmask), _stream()))
+        _ptr(out_scale), _ptr(keep), float(keep_scale), int(act_out), H, _ptr(x_next), _ptr(m_next), _ptr(hmask),
+        _stream()))
     return x_next, m_next, hmask
+
+
+def _keep_rows(keep, N, W):
+    """keep bits of one layer as a contiguous int32 [N, W] (or [N] for W = 1)"""
+    if keep is None:
+        return None
+    if keep.dtype != torch.int32 or keep.numel() != N * W:
+        raise ValueError(f"keep must be int32 with {N} x {W} words, got {keep.dtype} {tuple(keep.shape)}")
+    return keep.contiguous()
 
 
 # forward layer of the hidden-32 stack: A operands through tensor memory (csrc/gcn_fwd_tm.cu) or as shared-memory
@@ -509,10 +522,16 @@ def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_ou
 FWD_TMEM_OPERANDS = False
 
 
-def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, tmem_operands=None):
-    """one aggregate-then-transform forward layer at hidden 32 on tcgen05 (mgcn_gcn_layer_fwd_tc): z = in_scale (.) x
-    [N,32]; returns (z_next = out_scale (.) x_next [N,32], hmask int32[N])"""
-    _need_cuda(z, w, res_w, res_b, bias, in_scale, post, out_scale)
+def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, tmem_operands=None,
+                          keep=None, keep_scale=1.0):
+    """one aggregate-then-transform forward layer at hidden 32 on tcgen05 (mgcn_gcn_layer_fwd_tc_ex): z = in_scale (.) x
+    [N,32]; returns (z_next = out_scale (.) x_next [N,32], hmask int32[N]).  keep int32 [N]: dropout keep bits of the
+    layer (kept entries of h multiplied by keep_scale, dropped ones cleared in hmask too)"""
+    _need_cuda(z, w, res_w, res_b, bias, in_scale, post, out_scale, keep)
+    tmem = FWD_TMEM_OPERANDS if tmem_operands is None else tmem_operands
+    if keep is not None and tmem:
+        raise ValueError("dropout keep bits need the shared-memory operand forward (mgcn_gcn_layer_fwd_tc_ex), "
+                         "not the TMEM-operand kernel")
     z = _f32c(z, "z")
     w = _f32c(w, "w")
     res_w = _f32c(res_w, "res_w")
@@ -528,10 +547,14 @@ def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_sca
     z_next = torch.empty(n_rows, H, dtype=torch.float32, device=dev)
     hmask = torch.empty(n_rows, dtype=torch.int32, device=dev)
     lib = _lib.load()
-    args = (ctypes.byref(csr.struct()), _ptr(z), z.size(0), _ptr(w), _ptr(res_w), _ptr(res_b), _ptr(bias),
-            _ptr(in_scale), _ptr(post), _ptr(out_scale), int(act_out), H, _ptr(z_next), _ptr(hmask))
-    fn = lib.mgcn_gcn_layer_fwd_tm if (FWD_TMEM_OPERANDS if tmem_operands is None else tmem_operands) \
-        else lib.mgcn_gcn_layer_fwd_tc
+    lead = (ctypes.byref(csr.struct()), _ptr(z), z.size(0), _ptr(w), _ptr(res_w), _ptr(res_b), _ptr(bias),
+            _ptr(in_scale), _ptr(post), _ptr(out_scale))
+    tail = (int(act_out), H, _ptr(z_next), _ptr(hmask))
+    if tmem:
+        fn, args = lib.mgcn_gcn_layer_fwd_tm, lead + tail
+    else:
+        keep = _keep_rows(keep, n_rows, 1)
+        fn, args = lib.mgcn_gcn_layer_fwd_tc_ex, lead + (_ptr(keep), float(keep_scale)) + tail
     ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
     _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
     return z_next, hmask
@@ -608,6 +631,30 @@ def mask_bits_scale_impl(gy, bits, post):
     _lib.check(_lib.load().mgcn_mask_bits_scale(_ptr(gy), _ptr(bits), _ptr(post), gy.size(0), gy.size(1),
                                                 _ptr(out), _stream()))
     return out
+
+
+def dropout_keep_bits_impl(seed, L, N, W, p):
+    """dropout keep masks of L layers as bits (mgcn_dropout_keep_bits): int32 [L, N, W], bit b of word w = column
+    32 w + b kept; a pure function of (seed[0], layer, row, column) — include/mgcn.h states the generator exactly"""
+    _need_cuda(seed)
+    if seed.dtype != torch.int64 or seed.numel() != 1:
+        raise TypeError("seed must be one int64 on the device")
+    keep = torch.empty(L, N, W, dtype=torch.int32, device=seed.device)
+    _lib.check(_lib.load().mgcn_dropout_keep_bits(_ptr(seed.contiguous()), int(L), int(N), int(W), float(p),
+                                                  _ptr(keep), _stream()))
+    return keep
+
+
+def dropout_apply_impl(h, keep, scale):
+    """h[n,c] = keep bit ? h[n,c] * scale : 0 IN PLACE (mgcn_dropout_apply); keep int32 [N, W] (one layer's bits)"""
+    _need_cuda(h, keep)
+    if h.dtype != torch.float32 or not h.is_contiguous():
+        raise TypeError("h must be a contiguous float32 tensor (updated in place)")
+    N, H = h.shape
+    W = keep.size(-1) if keep.dim() > 1 else 1
+    keep = _keep_rows(keep, N, W)
+    _lib.check(_lib.load().mgcn_dropout_apply(_ptr(h), _ptr(keep), N, H, W, float(scale), _stream()))
+    return h
 
 
 def cross_entropy_fwd_impl(logits, target, mean):
@@ -946,6 +993,7 @@ _LIBDEF.define("gcn_first_layer_fwd(Tensor s, Tensor x, Tensor w_in, Tensor res_
 _LIBDEF.define("gcn_layer_bwd(Tensor dxw, Tensor gy, Tensor x, Tensor w, Tensor res_w, Tensor? hmask_prev, Tensor? post, "
                "bool want_prev, bool tensor_memory, Tensor? x_scale) -> (Tensor, Tensor, Tensor, Tensor, Tensor)")
 _LIBDEF.define("mask_bits_scale(Tensor gy, Tensor bits, Tensor? post) -> Tensor")
+_LIBDEF.define("dropout_keep_bits(Tensor seed, int L, int N, int W, float p) -> Tensor")
 _LIBDEF.define("segment_max(Tensor[] csr, int hub_threshold, Tensor x, bool gather_perm, Tensor? edge_val) -> (Tensor, Tensor)")
 _LIBDEF.define("segment_max_bwd(Tensor[] csr_t, int hub_threshold, Tensor grad, Tensor arg, Tensor? edge_val) -> Tensor")
 _LIBDEF.define("scatter_max_bwd(Tensor arg, Tensor grad, int n_src) -> Tensor")
@@ -996,6 +1044,7 @@ _IMPLS2 = {
     "gcn_first_layer_fwd": _op_first_layer_fwd,
     "gcn_layer_bwd": _op_layer_bwd,
     "mask_bits_scale": mask_bits_scale_impl,
+    "dropout_keep_bits": dropout_keep_bits_impl,
     "segment_max": lambda csr, ht, x, gp, ev: segment_max_impl(_as_csr(csr, ht), x, gp, ev),
     "segment_max_bwd": lambda csr_t, ht, grad, arg, ev: segment_max_bwd_impl(_as_csr(csr_t, ht), grad, arg, ev),
     "scatter_max_bwd": scatter_max_bwd_impl,
@@ -1041,6 +1090,11 @@ def _(dxw, gy, x, w, res_w, hmask_prev, post, want_prev, tensor_memory, x_scale)
 @torch.library.register_fake("mgcn::mask_bits_scale")
 def _(gy, bits, post):
     return torch.empty_like(gy)
+
+
+@torch.library.register_fake("mgcn::dropout_keep_bits")
+def _(seed, L, N, W, p):
+    return torch.empty(L, N, W, dtype=torch.int32, device=seed.device)
 
 
 @torch.library.register_fake("mgcn::segment_max")
