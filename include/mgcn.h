@@ -457,9 +457,16 @@ int mgcn_head_cross_entropy_bwd(const float* x, const float* logits, int64_t N, 
  * torch_scatter's gradient rule (the first entry that attains the maximum receives the gradient).
  * out[i,c] = max over the row's entries, in row order, of edge_val[k] * x[idx_k, c] (idx = perm when gather_perm:
  * primitive seam, else nbr: layer seam; edge_val in row order or NULL); arg[i,c] = edge id (perm) of the first
- * maximal entry, -1 (and out = 0) for a row without entries.  Deterministic, no atomics. */
+ * maximal entry, -1 (and out = 0) for a row without entries.  Deterministic, no atomics.
+ * mgcn_segment_max: the row's first entry always wins, whatever its value.
+ * mgcn_segment_max_ex: torch_scatter's fill rule — the running maximum starts at `fill` and an entry wins only if it
+ * is strictly greater, so an entry <= fill never wins; a (row, column) without a winner gives out = 0, arg = -1.
+ * Callers pass the fill of the call they stand for (-1e38 for common.py's scatter_('max'), -1e9 for PyG 1.3's
+ * scatter_('max'), fill_value for scatter_max).  The two agree wherever some entry of the row is > fill. */
 int mgcn_segment_max(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
                      const float* edge_val, float* out, int32_t* arg, void* stream);
+int mgcn_segment_max_ex(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
+                        const float* edge_val, float fill, float* out, int32_t* arg, void* stream);
 /* layer seam, gt = the structure grouped by the OTHER endpoint (by source):
  * dx[j,c] = sum over row j's entries k of [arg[nbr_k, c] == perm_k] * edge_val[k] * grad[nbr_k, c] */
 int mgcn_segment_max_bwd(const mgcn_csr_t* gt, const float* grad, const int32_t* arg, const float* edge_val,
@@ -470,9 +477,12 @@ int mgcn_scatter_max_bwd(const int32_t* arg, const float* grad, int64_t N, int64
 
 /* out[e] = scale_src[row_e] * scale_tgt[col_e] * sum_c a[col_e,c] * b[row_e,c]   (row = edge_index[0], col =
  * edge_index[1]; scales may be NULL): the gradient of an aggregation w.r.t. a per-edge weight, used by the edge gates
- * (gcn_base_models.py:230-232, 322-369: x_j = sigmoid(...)_e * x_j before scatter_).  Deterministic. */
+ * (gcn_base_models.py:230-232, 322-369: x_j = sigmoid(...)_e * x_j before scatter_).  Deterministic.
+ * _i32: the same for an int32 edge_index (bit-identical output). */
 int mgcn_edge_dot(const int64_t* edge_index, int64_t E, const float* a, const float* b, int64_t H,
                   const float* scale_src, const float* scale_tgt, float* out, void* stream);
+int mgcn_edge_dot_i32(const int32_t* edge_index, int64_t E, const float* a, const float* b, int64_t H,
+                      const float* scale_src, const float* scale_tgt, float* out, void* stream);
 
 /* Binary-classification counters of src/gcn_meta/optim/metrics.py:8-24 as used at train_botnet.py:296-305:
  * counts5 = {TP, FP, TN, FN, correct} (int64) with pred = argmax(logits[n,:]) (first maximal class; logits

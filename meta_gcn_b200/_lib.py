@@ -76,9 +76,11 @@ SIGNATURES = {
     "mgcn_gcn_layer_fwd_tm": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int,
                                       c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_segment_max": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "mgcn_segment_max_ex": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_int, c_ptr, c_f32, c_ptr, c_ptr, c_ptr]),
     "mgcn_segment_max_bwd": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
     "mgcn_scatter_max_bwd": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_i64, c_ptr, c_ptr]),
     "mgcn_edge_dot": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "mgcn_edge_dot_i32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
     "mgcn_edge_fingerprint": (c_int, [c_ptr, c_i64, c_ptr, c_ptr]),
     "mgcn_binary_confusion": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_ptr, c_ptr]),
     "mgcn_permute_edge_values": (c_int, [CSR_P, c_ptr, c_i64, c_f32, c_ptr, c_ptr]),

@@ -6,11 +6,11 @@ from ....graph import structure_of_index
 
 
 def scatter_(name, src, index, dim_size=None):
-    """PyG 1.3 utils.scatter_: 'add' | 'mean' | 'max' along dim 0; for 'max' the fill value (-1e9) of rows without
-    entries is replaced by 0, which is what the first-maximum kernel writes there"""
+    """PyG 1.3 utils.scatter_: 'add' | 'mean' | 'max' along dim 0; 'max' is torch_scatter's scatter_max from the fill
+    value -1e9, whose untouched entries are then replaced by 0 — what the first-maximum kernel with that fill writes"""
     assert name in ["add", "mean", "max"]
     if name == "max":
-        return F_mgcn.scatter_rows_max(src, index, dim_size)[0]
+        return F_mgcn.scatter_rows_max(src, index, dim_size, fill=-1e9)[0]
     return F_mgcn.scatter_rows(src, index, dim_size, name)
 
 

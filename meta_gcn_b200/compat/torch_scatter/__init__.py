@@ -28,7 +28,8 @@ def scatter_mean(src, index, dim=-1, out=None, dim_size=None, fill_value=0):
 
 
 def scatter_max(src, index, dim=-1, out=None, dim_size=None, fill_value=None):
-    """torch_scatter 1.x scatter_max along dim 0 -> (out, argmax): rows without entries hold fill_value / -1
+    """torch_scatter 1.x scatter_max along dim 0 -> (out, argmax): out = max(fill_value, entries), argmax = the first
+    entry strictly greater than fill_value that attains it, -1 (and out = fill_value) where no entry exceeds fill_value
     (common.py:56-57 passes -1e38 and zeroes those rows afterwards)"""
     import torch
     if src.dim() == 1 and dim == -1:
@@ -39,5 +40,5 @@ def scatter_max(src, index, dim=-1, out=None, dim_size=None, fill_value=None):
         raise NotImplementedError("scatter_max(out=...) is not used by the reference")
     if fill_value is None:
         fill_value = torch.finfo(src.dtype).min
-    res, arg = F_mgcn.scatter_rows_max(src, index, dim_size)
+    res, arg = F_mgcn.scatter_rows_max(src, index, dim_size, fill=fill_value)
     return torch.where(arg < 0, torch.full_like(res, fill_value), res), arg

@@ -3,7 +3,9 @@
 // (gcn_base_models.py:223-237: max over the edges of (x W)[row] * norm), with the autograd of torch_scatter's
 // scatter_max (the gradient of out[i,c] goes to the FIRST entry that attains the maximum).
 //   forward   out[i,c] = max_k v_k * x[idx_k, c] over the row's entries in row order (= edge_index order: the
-//             structure is a stable sort), arg[i,c] = edge id (perm) of the first maximal entry, -1 / 0 for an empty row
+//             structure is a stable sort), arg[i,c] = edge id (perm) of the first maximal entry, -1 / 0 for an empty row;
+//             with a fill value (torch_scatter's running maximum starts at fill_value and only a strictly greater entry
+//             replaces it) an entry <= fill never wins, and a (row, column) without a winner is 0 / -1 as well
 //   backward  primitive seam: dsrc[arg[i,c], c] = g[i,c] (an edge belongs to one row: no conflicts)
 //             layer seam: a row-owned pass over the structure grouped by source,
 //             dx[j,c] = sum_{k in row j} [arg[target_k, c] == edge_k] * v_k * g[target_k, c]
@@ -12,26 +14,29 @@
 
 namespace mgcn {
 
+// kFill: the running maximum starts at `fill` and an entry must be strictly greater to win; otherwise the row's first
+// entry always wins
+template <bool kFill>
 __global__ void __launch_bounds__(256)
     k_segment_max(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ idx, const int32_t* __restrict__ perm,
-                  const float* __restrict__ x, const float* __restrict__ edge_val, int64_t n_rows, int H,
+                  const float* __restrict__ x, const float* __restrict__ edge_val, int64_t n_rows, int H, float fill,
                   float* __restrict__ out, int32_t* __restrict__ arg) {
   const int64_t total = n_rows * H;
   for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
     const int64_t i = t / H;
     const int c = (int)(t - i * H);
     const int beg = __ldg(rowptr + i), end = __ldg(rowptr + i + 1);
-    float best = 0.f;
+    float best = kFill ? fill : 0.f;
     int32_t who = -1;
     for (int k = beg; k < end; ++k) {
       float v = __ldg(x + (int64_t)__ldg(idx + k) * H + c);
       if (edge_val) v = __fmul_rn(v, __ldg(edge_val + k));
-      if (who < 0 || v > best) {
+      if ((!kFill && who < 0) || v > best) {
         best = v;
         who = __ldg(perm + k);
       }
     }
-    out[t] = best;
+    out[t] = who < 0 ? 0.f : best;
     arg[t] = who;
   }
 }
@@ -77,16 +82,32 @@ static unsigned grid_for(int64_t total) {
 
 using namespace mgcn;
 
-extern "C" int mgcn_segment_max(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
-                                const float* edge_val, float* out, int32_t* arg, void* stream) {
+static int segment_max(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
+                       const float* edge_val, bool with_fill, float fill, float* out, int32_t* arg, void* stream) {
   MGCN_REQUIRE(g != nullptr, MGCN_ERR_NULL);
   MGCN_REQUIRE(H >= 1 && H <= 65536 && n_in >= 0 && g->n_rows >= 0, MGCN_ERR_SHAPE);
   if (g->n_rows == 0) return MGCN_OK;
   MGCN_REQUIRE(g->rowptr && out && arg, MGCN_ERR_NULL);
   MGCN_REQUIRE(g->nnz_cap == 0 || (g->nbr && g->perm && x), MGCN_ERR_NULL);
-  MGCN_LAUNCH(k_segment_max, grid_for(g->n_rows * H), 256, 0, stream, g->rowptr, gather_perm ? g->perm : g->nbr,
-              g->perm, x, edge_val, g->n_rows, (int)H, out, arg);
+  const int32_t* idx = gather_perm ? g->perm : g->nbr;
+  if (with_fill) {
+    MGCN_LAUNCH(k_segment_max<true>, grid_for(g->n_rows * H), 256, 0, stream, g->rowptr, idx, g->perm, x, edge_val,
+                g->n_rows, (int)H, fill, out, arg);
+  } else {
+    MGCN_LAUNCH(k_segment_max<false>, grid_for(g->n_rows * H), 256, 0, stream, g->rowptr, idx, g->perm, x, edge_val,
+                g->n_rows, (int)H, 0.f, out, arg);
+  }
   return MGCN_OK;
+}
+
+extern "C" int mgcn_segment_max(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
+                                const float* edge_val, float* out, int32_t* arg, void* stream) {
+  return segment_max(g, x, n_in, H, gather_perm, edge_val, false, 0.f, out, arg, stream);
+}
+
+extern "C" int mgcn_segment_max_ex(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int gather_perm,
+                                   const float* edge_val, float fill, float* out, int32_t* arg, void* stream) {
+  return segment_max(g, x, n_in, H, gather_perm, edge_val, true, fill, out, arg, stream);
 }
 
 extern "C" int mgcn_segment_max_bwd(const mgcn_csr_t* gt, const float* grad, const int32_t* arg, const float* edge_val,
@@ -121,8 +142,9 @@ extern "C" int mgcn_scatter_max_bwd(const int32_t* arg, const float* grad, int64
 // 8 lanes per edge, fixed butterfly over the lanes: deterministic.
 // -------------------------------------------------------------------------------------------------
 namespace mgcn {
+template <typename Index>
 __global__ void __launch_bounds__(256)
-    k_edge_dot(const int64_t* __restrict__ ei, int64_t E, const float* __restrict__ a, const float* __restrict__ b, int H,
+    k_edge_dot(const Index* __restrict__ ei, int64_t E, const float* __restrict__ a, const float* __restrict__ b, int H,
                const float* __restrict__ s_src, const float* __restrict__ s_tgt, float* __restrict__ out) {
   const int sub = threadIdx.x & 7;
   const int64_t per_iter = (int64_t)gridDim.x * (blockDim.x >> 3);
@@ -132,8 +154,8 @@ __global__ void __launch_bounds__(256)
     float s = 0.f;
     int64_t r = 0, c = 0;
     if (e < E) {
-      r = ei[e];
-      c = ei[E + e];
+      r = (int64_t)ei[e];
+      c = (int64_t)ei[E + e];
       for (int k = sub; k < H; k += 8) s = fmaf(__ldg(a + c * H + k), __ldg(b + r * H + k), s);
     }
     s += __shfl_xor_sync(0xffffffffu, s, 4);
@@ -148,13 +170,25 @@ __global__ void __launch_bounds__(256)
 }
 }  // namespace mgcn
 
-extern "C" int mgcn_edge_dot(const int64_t* edge_index, int64_t E, const float* a, const float* b, int64_t H,
-                             const float* scale_src, const float* scale_tgt, float* out, void* stream) {
+template <typename Index>
+static int edge_dot(const Index* edge_index, int64_t E, const float* a, const float* b, int64_t H,
+                    const float* scale_src, const float* scale_tgt, float* out, void* stream) {
   MGCN_REQUIRE(E >= 0 && H >= 1 && H <= 65536, MGCN_ERR_SHAPE);
   if (E == 0) return MGCN_OK;
   MGCN_REQUIRE(edge_index && a && b && out, MGCN_ERR_NULL);
   int64_t blocks = ceil_div(E, 32);
   if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
-  MGCN_LAUNCH(k_edge_dot, (unsigned)blocks, 256, 0, stream, edge_index, E, a, b, (int)H, scale_src, scale_tgt, out);
+  MGCN_LAUNCH(k_edge_dot<Index>, (unsigned)blocks, 256, 0, stream, edge_index, E, a, b, (int)H, scale_src, scale_tgt,
+              out);
   return MGCN_OK;
+}
+
+extern "C" int mgcn_edge_dot(const int64_t* edge_index, int64_t E, const float* a, const float* b, int64_t H,
+                             const float* scale_src, const float* scale_tgt, float* out, void* stream) {
+  return edge_dot(edge_index, E, a, b, H, scale_src, scale_tgt, out, stream);
+}
+
+extern "C" int mgcn_edge_dot_i32(const int32_t* edge_index, int64_t E, const float* a, const float* b, int64_t H,
+                                 const float* scale_src, const float* scale_tgt, float* out, void* stream) {
+  return edge_dot(edge_index, E, a, b, H, scale_src, scale_tgt, out, stream);
 }

@@ -72,8 +72,8 @@ class _AggregateMax(torch.autograd.Function):
     structure"""
 
     @staticmethod
-    def forward(ctx, x, graph, ev_fwd, ev_bwd):
-        out, arg = ops.segment_max_impl(graph.fwd, x, False, ev_fwd)
+    def forward(ctx, x, graph, ev_fwd, ev_bwd, fill):
+        out, arg = ops.segment_max_impl(graph.fwd, x, False, ev_fwd, fill)
         ctx.graph = graph
         ctx.save_for_backward(arg, ev_bwd)
         ctx.mark_non_differentiable(arg)
@@ -83,16 +83,17 @@ class _AggregateMax(torch.autograd.Function):
     def backward(ctx, g, _garg):
         arg, ev_bwd = ctx.saved_tensors
         dx = ops.segment_max_bwd_impl(ctx.graph.bwd, g.contiguous(), arg, ev_bwd) if ctx.needs_input_grad[0] else None
-        return dx, None, None, None
+        return dx, None, None, None, None
 
 
-def aggregate_max(x, graph, edge_weight=None, loop_value=1.0):
+def aggregate_max(x, graph, edge_weight=None, loop_value=1.0, fill=-1e38):
     """NodeModelAdditive(aggr='max') (gcn_base_models.py:223-237): max over incoming edges of x[row] * norm_e;
-    edge_weight = the per-edge factor norm[E] in edge_index order (or None)"""
+    edge_weight = the per-edge factor norm[E] in edge_index order (or None).  As scatter_('max') of common.py:54-64,
+    an entry <= fill (-1e38) never wins, and a (node, column) without a winner is 0 and receives no gradient."""
     ev_fwd = ev_bwd = None
     if edge_weight is not None:
         ev_fwd, ev_bwd = graph.edge_values(edge_weight, loop_value)
-    return _AggregateMax.apply(x, graph, ev_fwd, ev_bwd)[0]
+    return _AggregateMax.apply(x, graph, ev_fwd, ev_bwd, fill)[0]
 
 
 class _Linear(torch.autograd.Function):
@@ -238,8 +239,8 @@ class _ScatterRows(torch.autograd.Function):
 
 class _ScatterRowsMax(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, src, graph):
-        out, arg = ops.segment_max_impl(graph.fwd, src, True, None)
+    def forward(ctx, src, graph, fill):
+        out, arg = ops.segment_max_impl(graph.fwd, src, True, None, fill)
         ctx.n_src = src.size(0)
         ctx.save_for_backward(arg)
         ctx.mark_non_differentiable(arg)
@@ -248,17 +249,19 @@ class _ScatterRowsMax(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g, _garg):
         (arg,) = ctx.saved_tensors
-        return ops.scatter_max_bwd_impl(arg, g.contiguous(), ctx.n_src), None
+        return ops.scatter_max_bwd_impl(arg, g.contiguous(), ctx.n_src), None, None
 
 
-def scatter_rows_max(src, index, dim_size=None):
-    """scatter_('max', src, index, dim_size) (common.py:54-64) -> (out, argmax); rows without entries are 0 / -1"""
+def scatter_rows_max(src, index, dim_size=None, fill=-1e38):
+    """scatter_('max', src, index, dim_size) (common.py:54-64) -> (out, argmax) with torch_scatter's fill rule: an
+    entry <= fill never wins; a (row, column) without a winner (no entries, or all <= fill) is 0 / -1.  The default is
+    common.py's fill; other callers pass the fill of the call they stand for."""
     squeeze = src.dim() == 1
     src2 = src.unsqueeze(1) if squeeze else src.reshape(src.size(0), -1)
     if dim_size is None:
         dim_size = int(index.max().item()) + 1 if index.numel() else 0
     graph = structure_of_index(index, dim_size)
-    out, arg = _ScatterRowsMax.apply(src2, graph)
+    out, arg = _ScatterRowsMax.apply(src2, graph, fill)
     if squeeze:
         return out.squeeze(1), arg.squeeze(1).long()
     return out.reshape(dim_size, *src.shape[1:]), arg.reshape(dim_size, *src.shape[1:]).long()
@@ -278,6 +281,27 @@ def scatter_rows(src, index, dim_size=None, reduce="add"):
     if squeeze:
         return out.squeeze(1)
     return out.reshape(dim_size, *src.shape[1:])
+
+
+class _GatherRows(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, src, index):
+        ctx.n_src = src.size(0)
+        ctx.save_for_backward(index)
+        return src.index_select(0, index)
+
+    @staticmethod
+    def backward(ctx, g):
+        (index,) = ctx.saved_tensors
+        return scatter_rows(g.contiguous(), index, ctx.n_src, "add") if ctx.needs_input_grad[0] else None, None
+
+
+def gather_rows(src, index):
+    """src.index_select(0, index) whose gradient is summed per source row by the row-owned scatter kernel
+    (scatter_rows) instead of index_select's atomicAdd backward: deterministic, and the same for int32 and int64
+    indices.  Used for per-edge gathers of node tensors that require grad (edge-gate scores, attention scores,
+    the messages of the 'max' aggregation with gates or edge features)."""
+    return _GatherRows.apply(src, index)
 
 
 class _CrossEntropy(torch.autograd.Function):

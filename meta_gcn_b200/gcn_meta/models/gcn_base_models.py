@@ -135,7 +135,7 @@ class NodeModelAdditive(NodeModelBase):
                 # the maximum is taken over gate_e * (x W [row_e] * norm_e + edge_attr_e W_e): not separable into a
                 # per-node and a per-edge part, so the [E,H] messages are formed as the reference does
                 # (gcn_base_models.py:223-232) and reduced by the primitive seam's first-maximum kernel
-                msg = xw.index_select(0, edge_index[0])
+                msg = F_mgcn.gather_rows(xw, edge_index[0])
                 if norm_e is not None:
                     msg = msg * norm_e.view(-1, 1)
                 if edge_attr is not None:
@@ -187,7 +187,8 @@ class EdgeGateProj(nn.Module):
 
     def forward(self, x, edge_index, edge_attr=None, edge_weight=None):
         score = lambda lin, t: F_mgcn.linear(t, lin.weight, weight_layout="out_in")   # noqa: E731  [*, 1]
-        gate = score(self.linsrc, x).index_select(0, edge_index[0]) + score(self.lintgt, x).index_select(0, edge_index[1])
+        gate = (F_mgcn.gather_rows(score(self.linsrc, x), edge_index[0])
+                + F_mgcn.gather_rows(score(self.lintgt, x), edge_index[1]))
         if edge_attr is not None:
             gate = gate + score(self.linedge, edge_attr)
         if self.bias is not None:

@@ -60,7 +60,7 @@ class NodeModelAttention(NodeModelBase):
         s_src = (xv * a[:, :c1]).sum(-1)                                             # <x_j, a_src>   [N, heads]
         s_tgt = (xv * a[:, c1:]).sum(-1)                                             # <x_i, a_tgt>
         row, col = edge_index[0], edge_index[1]
-        alpha = self.att_act(s_src.index_select(0, row) + s_tgt.index_select(0, col))   # :71   [E, heads]
+        alpha = self.att_act(F_mgcn.gather_rows(s_src, row) + F_mgcn.gather_rows(s_tgt, col))   # :71   [E, heads]
         alpha = softmax(alpha, row if self.att_dir == "out" else col, num_nodes=n)      # :74-79
         alpha = self.att_dropout(alpha)                                              # :82
         heads = [F_mgcn.aggregate(xv[:, h, :].contiguous(), graph, None, None, alpha[:, h].contiguous(), self.aggr)

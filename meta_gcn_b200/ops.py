@@ -312,8 +312,10 @@ def spmm_impl(csr, x, gather_perm=False, edge_val=None, nbr_scale=None, row_scal
 
 
 def edge_dot_impl(edge_index, a, b, scale_src=None, scale_tgt=None):
-    """out[e] = scale_src[row_e] * scale_tgt[col_e] * <a[col_e], b[row_e]>   (mgcn_edge_dot)"""
+    """out[e] = scale_src[row_e] * scale_tgt[col_e] * <a[col_e], b[row_e]>   (mgcn_edge_dot / _i32)"""
     _need_cuda(edge_index, a, b, scale_src, scale_tgt)
+    if edge_index.dtype not in (torch.int64, torch.int32) or edge_index.dim() != 2 or edge_index.size(0) != 2:
+        raise TypeError("edge_index must be int64 or int32, shape [2, E]")
     a = _f32c(a, "a")
     b = _f32c(b, "b")
     scale_src = _f32c(scale_src, "scale_src")
@@ -321,13 +323,15 @@ def edge_dot_impl(edge_index, a, b, scale_src=None, scale_tgt=None):
     ei = edge_index.contiguous()
     E = ei.size(1)
     out = torch.empty(E, dtype=torch.float32, device=a.device)
-    _lib.check(_lib.load().mgcn_edge_dot(_ptr(ei), E, _ptr(a), _ptr(b), a.size(1), _ptr(scale_src), _ptr(scale_tgt),
-                                         _ptr(out), _stream()))
+    lib = _lib.load()
+    fn = lib.mgcn_edge_dot if ei.dtype == torch.int64 else lib.mgcn_edge_dot_i32
+    _lib.check(fn(_ptr(ei), E, _ptr(a), _ptr(b), a.size(1), _ptr(scale_src), _ptr(scale_tgt), _ptr(out), _stream()))
     return out
 
 
-def segment_max_impl(csr, x, gather_perm=False, edge_val=None):
-    """(out [n_rows,H], arg int32 [n_rows,H]) of mgcn_segment_max"""
+def segment_max_impl(csr, x, gather_perm=False, edge_val=None, fill=None):
+    """(out [n_rows,H], arg int32 [n_rows,H]) of mgcn_segment_max, or of mgcn_segment_max_ex with a fill value
+    (torch_scatter's rule: only an entry strictly greater than fill can win; no winner -> 0 / -1)"""
     _need_cuda(csr.rowptr, x, edge_val)
     x = _f32c(x, "x")
     edge_val = _f32c(edge_val, "edge_val")
@@ -336,8 +340,12 @@ def segment_max_impl(csr, x, gather_perm=False, edge_val=None):
     H = x.size(1)
     out = torch.empty(csr.n_rows, H, dtype=torch.float32, device=x.device)
     arg = torch.empty(csr.n_rows, H, dtype=torch.int32, device=x.device)
-    _lib.check(_lib.load().mgcn_segment_max(ctypes.byref(csr.struct()), _ptr(x), x.size(0), H, int(bool(gather_perm)),
-                                            _ptr(edge_val), _ptr(out), _ptr(arg), _stream()))
+    lib = _lib.load()
+    head = (ctypes.byref(csr.struct()), _ptr(x), x.size(0), H, int(bool(gather_perm)), _ptr(edge_val))
+    if fill is None:
+        _lib.check(lib.mgcn_segment_max(*head, _ptr(out), _ptr(arg), _stream()))
+    else:
+        _lib.check(lib.mgcn_segment_max_ex(*head, float(fill), _ptr(out), _ptr(arg), _stream()))
     return out, arg
 
 

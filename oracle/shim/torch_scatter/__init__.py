@@ -44,9 +44,12 @@ class _ScatterMax(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, out, src, index, dim):
+        init = out
         out = out.scatter_reduce(dim, index, src, reduce="amax", include_self=True)
-        # argmax: first position attaining the max, -1 for untouched rows (torch_scatter 1.x)
-        hit = src == out.gather(dim, index)
+        # argmax: first position attaining the max, -1 for untouched rows (torch_scatter 1.x); the running maximum
+        # starts at the initial value and only a strictly greater entry replaces it, so an entry equal to the
+        # initial value (fill_value) is never the argmax
+        hit = (src == out.gather(dim, index)) & (src > init.gather(dim, index))
         pos_shape = [1] * src.dim()
         pos_shape[dim] = src.size(dim)
         pos = torch.arange(src.size(dim), device=src.device).view(pos_shape).expand_as(src)
