@@ -716,7 +716,8 @@ __device__ __forceinline__ uint64_t mix64(uint64_t z) {
 // out[0..3]: the multiset fingerprints (as k_edge_fingerprint; accumulated here in the same pass over the list — one
 // read of edge_index instead of two); out[4] entries e with (src,dst)[e] > (src,dst)[e+1]
 // over the whole list, out[5] the same over the first E-N entries, out[6] entries of the last N that are not the
-// loop (e-(E-N), e-(E-N)), out[7] adjacent equal entries (whole list).
+// loop (e-(E-N), e-(E-N)), out[7] adjacent equal entries (whole list).  An entry with an endpoint outside [0, N) (in a
+// batch: outside its graph's node range) counts once more in out[4] and out[5].
 template <typename IndexT>
 __global__ void __launch_bounds__(256) k_edge_order_check(const IndexT* __restrict__ ei, int64_t E, int64_t N, int G,
                                                           const int32_t* __restrict__ node_off,
@@ -742,11 +743,12 @@ __global__ void __launch_bounds__(256) k_edge_order_check(const IndexT* __restri
       e0 = edge_off[g];
       ng = node_off[g + 1] - n0;
       eg = edge_off[g + 1] - e0;
-      // every endpoint of a graph's entries lies in the graph's own node range
-      if (s < n0 || s >= n0 + ng || d < n0 || d >= n0 + ng) {
-        f[0] += 1u;
-        f[1] += 1u;
-      }
+    }
+    // every endpoint of a graph's entries lies in the graph's own node range: a list with an id outside it takes the
+    // sorting build, which drops that entry (the sort-free placement k = e (+ s) would shift every later entry)
+    if (s < n0 || s >= n0 + ng || d < n0 || d >= n0 + ng) {
+      f[0] += 1u;
+      f[1] += 1u;
     }
     const int64_t Ep = eg >= ng ? e0 + eg - ng : -1;   // end of the sorted prefix under the "+ loops" reading
     if (e + 1 < e0 + eg) {

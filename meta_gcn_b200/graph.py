@@ -72,9 +72,11 @@ class GraphStructure:
             # (a batch described graph by graph: by source only — the mirror search of the by-target build is per list)
             if f["layout"] and (by == 0 or (f["symmetric"] and self.segments is None)):
                 layout = f["layout"]
+        # only the "+ loops" layouts need the graph boundaries: a batch whose graphs are each sorted, with their ids in
+        # their own node ranges, is sorted as one list (node ids ascend from graph to graph)
+        segments = self.segments if layout & 3 == 2 else None
         return ops.csr_build_impl(self.edge_index, self.num_nodes, by, self.loop_mode,
-                                  self.hub_threshold, layout, self.segments if layout else None,
-                                  reuse=self._recycle.pop(by, None))
+                                  self.hub_threshold, layout, segments, reuse=self._recycle.pop(by, None))
 
     def built(self):
         """the structures built so far (Csr objects)"""

@@ -7,90 +7,19 @@ import torch
 from meta_gcn_b200 import ops
 from meta_gcn_b200.data import synth_botnet_graph
 from oracle import port
-from util import assert_bitexact
+from util import assert_bitexact, check_structure, csr_numpy
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 
 
-class _Built:
-    pass
-
-
 def build(ei_np, n, by, mode, hub_t=256):
     ei = torch.from_numpy(np.ascontiguousarray(ei_np)).long().to(DEV)
-    csr = ops.csr_build_impl(ei, n, by, mode, hub_t)
-    torch.cuda.synchronize()
-    b = _Built()
-    for name in ops.CSR_FIELDS:
-        setattr(b, name, getattr(csr, name).cpu().numpy())
-    b.bad = csr.bad.cpu().numpy()
-    return b
+    return csr_numpy(ops.csr_build_impl(ei, n, by, mode, hub_t))
 
 
 def check_against_oracle(ei_np, n, by, mode, hub_t=256):
-    b = build(ei_np, n, by, mode, hub_t)
-    o_rowptr, o_nbr, o_perm = port.csr_oracle(ei_np, n, by, mode)
-    assert b.bad[0] == 0
-    assert_bitexact(b.rowptr, o_rowptr, "rowptr")
-    nnz = int(o_rowptr[-1])
-    assert_bitexact(b.nbr[:nnz], o_nbr, "nbr")
-    assert_bitexact(b.perm[:nnz], o_perm, "perm")
-    assert (b.perm[nnz:] == -1).all()
-    deg = np.diff(o_rowptr)
-    # hubs and their segments: every hub once, segments contiguous, covering the row in order
-    want_hubs = np.nonzero(deg > hub_t)[0]
-    nh = int(b.hub_count[0])
-    assert nh == len(want_hubs)
-    assert sorted(b.hub_rows[:nh].tolist()) == want_hubs.tolist()
-    total_segs = 0
-    for k in range(nh):
-        row, s0 = int(b.hub_rows[k]), int(b.hub_seg0[k])
-        nseg = -(-int(deg[row]) // hub_t)
-        total_segs += nseg
-        assert (b.seg_row[s0:s0 + nseg] == row).all()
-        assert b.seg_beg[s0:s0 + nseg].tolist() == [int(o_rowptr[row]) + q * hub_t for q in range(nseg)]
-    assert int(b.seg_count[0]) == total_segs
-    # work order: a permutation of the rows, sorted by (row // 16384, min(len, 1023)), stable
-    assert sorted(b.order.tolist()) == list(range(n))
-    key = (b.order.astype(np.int64) >> 14) * 1024 + np.minimum(deg[b.order], 1023)
-    assert (np.diff(key) >= 0).all()
-    same = np.diff(key) == 0
-    assert (np.diff(b.order)[same] > 0).all()
-    # work descriptors {row, beg, end, partial_slot}: n + total_segs tasks sorted (stably, by task id)
-    # by (window, length; segments behind the rows of their window); positions contiguous in nbr_w
-    t = b.tasks.reshape(-1, 4)
-    nt = n + total_segs
-    tid_len = np.concatenate([np.minimum(deg, 1023), np.full(total_segs, 1024)]).astype(np.int64)
-    tid_win = np.concatenate([np.arange(n) >> 14, b.seg_row[:total_segs] >> 14]).astype(np.int64)
-    want = np.argsort(tid_win * 2048 + tid_len, kind="stable")
-    pos = 0
-    rows_seen, segs_seen = [], []
-    for p in range(nt):
-        s_id = int(want[p])
-        row, beg, end, slot = (int(v) for v in t[p])
-        assert beg == pos, (p, beg, pos)
-        if s_id < n:
-            assert slot == 0
-            if deg[s_id] > hub_t:
-                assert row == -1 and end == beg
-            else:
-                assert row == s_id and end - beg == deg[s_id]
-                assert (b.nbr_w[beg:end] == o_nbr[o_rowptr[s_id]:o_rowptr[s_id + 1]]).all()
-                rows_seen.append(s_id)
-        else:
-            q = s_id - n
-            assert slot == q + 1 and row == b.seg_row[q]
-            sb = int(b.seg_beg[q])
-            se = min(sb + hub_t, int(o_rowptr[row + 1]))
-            assert end - beg == se - sb
-            assert (b.nbr_w[beg:end] == o_nbr[sb:se]).all()
-            segs_seen.append(q)
-        pos = end
-    assert pos == nnz
-    assert sorted(segs_seen) == list(range(total_segs))
-    pad = t[nt:]
-    assert (pad[:, 0] == -1).all() and (pad[:, 1] == nnz).all() and (pad[:, 2] == nnz).all()
+    check_structure(build(ei_np, n, by, mode, hub_t), *port.csr_oracle(ei_np, n, by, mode), hub_t)
 
 
 @pytest.mark.parametrize("n,e", [(1, 1), (5, 0), (7, 3), (100, 4095), (100, 4096), (100, 4097), (300, 8193),
