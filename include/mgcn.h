@@ -433,8 +433,16 @@ int mgcn_batchnorm_bwd(const float* x, const float* g, int64_t N, int64_t H, con
 /* ---------------------------------------------------------------------------------------------
  * Node-level cross entropy — nn.CrossEntropyLoss()(x, batch.y.long()) (train_botnet.py:225,287).
  * loss[0] = sum_n ( logsumexp(logits[n,:]) - logits[n, target[n]] ) (* 1/N if mean), fixed-order
- * two-stage sum.  bad_target int32[1] is set if a label is outside [0,C).
- * bwd: dlogits = (softmax - onehot) * (1/N if mean) * upstream[0]   (upstream: device scalar or NULL)
+ * two-stage sum.  A row's NLL is log1p(t) - (z_y - m), m = max_c z_c, t = sum of exp(z_c - m) over the classes
+ * other than the first maximal one, so a confidently classified row keeps its small loss.
+ * bwd: dlogits = (softmax - onehot) * (1/N if mean) * upstream[0]   (upstream: device scalar or NULL); the label's
+ * entry is computed as -(sum over c != y of exp(z_c - m)) / s, not p_y - 1.
+ *
+ * Labels (both cross-entropy contracts, this one and the fused head below): a label outside [0, C) — -100
+ * included, which is not an "ignore" value here — makes loss[0] NaN in both reductions, makes that row's
+ * gradient NaN (its dlogits row; in the fused head its dx row and so dw and db), and is skipped by the counters.
+ * bad_target int32[1] is set when such a label occurs.  No host synchronisation is involved.
+ * No rows (N = 0): the sum is 0, the mean NaN (as torch); gradients over no rows are 0.
  */
 int mgcn_cross_entropy_fwd(const float* logits, const int64_t* target, int64_t N, int64_t C, int mean,
                            float* loss, int32_t* bad_target, void* workspace, size_t* workspace_bytes,
@@ -449,7 +457,8 @@ int mgcn_cross_entropy_bwd(const float* logits, const int64_t* target, int64_t N
  * correct} (int64, may be NULL) — and ONE backward launch that reads x and the logits once:
  *   dl = (softmax(logits) - onehot(target)) * (1/N if mean) * upstream[0]
  *   dx = dl w  (may be NULL);   dw = dl^T x;   db = colsum(dl)      (fixed-order partials: deterministic)
- * H in {16, 32, 64, 128}, C <= 8, w [C,H] (nn.Linear.weight), b [C] or NULL. */
+ * H in {16, 32, 64, 128}, C <= 8, w [C,H] (nn.Linear.weight), b [C] or NULL.  The row NLL, the label's gradient
+ * entry, labels outside [0, C) and N = 0 follow the node-level cross entropy above. */
 int mgcn_head_cross_entropy_fwd(const float* x, int64_t N, int64_t H, const float* w, const float* b, int64_t C,
                                 const int64_t* target, int mean, float* logits, float* loss, int64_t* counts5,
                                 int32_t* bad_target, void* workspace, size_t* workspace_bytes, void* stream);

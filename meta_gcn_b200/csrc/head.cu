@@ -10,6 +10,8 @@
 // counters integer sums (exact): deterministic, no floating-point atomics.
 //
 // Thread mapping: L = H / 4 lanes own a row (one float4 each), 32 / L rows per warp; C <= kHeadMaxC classes.
+#include <limits>
+
 #include "common.cuh"
 
 namespace mgcn {
@@ -88,21 +90,24 @@ __global__ void __launch_bounds__(kHeadThreads) k_head_ce_fwd(const HeadArgs a) 
           m = z[c];
           am = c;
         }
-      float s = 0.f;
+      // t = sum over the classes other than the argmax of exp(z_c - m); exp(z_am - m) = 1 is left out so that the
+      // NLL of a confidently classified row, log1p(t) - (z_y - m), does not vanish into m + log(1 + t) - z_y
+      float t = 0.f;
 #pragma unroll
       for (int c = 0; c < CM; ++c)
         if (c < a.C) {
-          s += expf(z[c] - m);
+          if (c != am) t += expf(z[c] - m);
           a.logits[n * a.C + c] = z[c];
         }
-      if (y < 0 || y >= a.C) {
+      if (y < 0 || y >= a.C) {   // the row's loss is NaN, so is the sum; the counters skip it
         *a.bad = 1;
+        loss += __int_as_float(0x7fc00000);
       } else {
         float zy = z[0];
 #pragma unroll
         for (int c = 1; c < CM; ++c)
           if (c == (int)y) zy = z[c];
-        loss += (m + logf(s)) - zy;
+        loss += log1pf(t) - (zy - m);
         if (a.counts) {   // optim/metrics.py:8-24: positives are class 1
           cnt[0] += (am == 1 && y == 1) ? 1u : 0u;
           cnt[1] += (am == 1 && y == 0) ? 1u : 0u;
@@ -214,16 +219,23 @@ __global__ void __launch_bounds__(kHeadThreads) k_head_ce_bwd(const HeadArgs a) 
 #pragma unroll
     for (int c = 0; c < CM; ++c)
       if (c < a.C) m = fmaxf(m, r.z[c]);
-    float s = 0.f;
+    float e[CM];
+    float s = 0.f, t = 0.f;   // t = sum of e_c over c != y
 #pragma unroll
     for (int c = 0; c < CM; ++c)
-      if (c < a.C) s += expf(r.z[c] - m);
-    const float inv = 1.f / s;
+      if (c < a.C) {
+        e[c] = expf(r.z[c] - m);
+        s += e[c];
+        if (c != r.y) t += e[c];
+      }
+    // a label outside [0, C) makes the whole row NaN (and with it dw and db)
+    const float inv = (r.y < 0 || r.y >= a.C) ? __int_as_float(0x7fc00000) : 1.f / s;
     float4 dxv = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int c = 0; c < CM; ++c)
       if (c < a.C) {
-        const float dl = (expf(r.z[c] - m) * inv - (c == (int)r.y ? 1.f : 0.f)) * g;
+        // the label's class as -(sum of the others) / s: 1 - e_y / s cancels for a confident row
+        const float dl = (c == r.y ? -t : e[c]) * inv * g;
         const float4 wv = *reinterpret_cast<const float4*>(&ws[c][4 * sub]);
         dxv.x = fmaf(dl, wv.x, dxv.x);
         dxv.y = fmaf(dl, wv.y, dxv.y);
@@ -327,7 +339,8 @@ extern "C" int mgcn_head_cross_entropy_fwd(const float* x, int64_t N, int64_t H,
       default: MGCN_LAUNCH((k_head_ce_fwd<32, kHeadMaxC>), P, kHeadThreads, 0, stream, a); break;
     }
   }
-  const float scale = mean ? (N > 0 ? 1.0f / (float)N : 0.f) : 1.f;
+  // the mean over no rows is NaN, as torch's
+  const float scale = mean ? (N > 0 ? 1.0f / (float)N : std::numeric_limits<float>::quiet_NaN()) : 1.f;
   MGCN_LAUNCH(k_head_loss_finish, 1, 256, 0, stream, part, P, scale, loss);
   return MGCN_OK;
 }

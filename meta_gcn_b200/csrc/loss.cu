@@ -1,18 +1,28 @@
 // Cross-entropy over node logits — nn.CrossEntropyLoss()(x, batch.y.long()) of
 // train_botnet.py:225,287 — as two small deterministic kernels (fixed-order two-stage sum), so
 // the step has no single-block torch reduction over 3.6 M rows on its critical path.
+#include <limits>
+
 #include "common.cuh"
 
 namespace mgcn {
 
 constexpr int kCeThreads = 256;
 
+// log1p(t) - (z_y - m) with t = sum over the classes other than the (first) argmax of exp(z_c - m): the term
+// exp(z_argmax - m) = 1 is left out, so the small NLL of a confidently classified row is not lost in m + log(s) - z_y
 __device__ __forceinline__ float row_nll(const float* __restrict__ z, int C, int64_t y) {
   float m = z[0];
-  for (int c = 1; c < C; ++c) m = fmaxf(m, z[c]);
-  float s = 0.f;
-  for (int c = 0; c < C; ++c) s += expf(z[c] - m);
-  return (m + logf(s)) - z[y];
+  int am = 0;
+  for (int c = 1; c < C; ++c)
+    if (z[c] > m) {
+      m = z[c];
+      am = c;
+    }
+  float t = 0.f;
+  for (int c = 0; c < C; ++c)
+    if (c != am) t += expf(z[c] - m);
+  return log1pf(t) - (z[y] - m);
 }
 
 // partial[b] = sum of the NLL of the rows of slab b (rows strided by thread inside a slab,
@@ -26,8 +36,9 @@ __global__ void __launch_bounds__(kCeThreads)
   float s = 0.f;
   for (int64_t n = n0 + threadIdx.x; n < n1; n += kCeThreads) {
     const int64_t y = target[n];
-    if (y < 0 || y >= C) {
+    if (y < 0 || y >= C) {   // the row's loss is NaN, so is the sum
       *bad = 1;
+      s += __int_as_float(0x7fc00000);
       continue;
     }
     s += row_nll(logits + n * C, C, y);
@@ -55,7 +66,8 @@ __global__ void __launch_bounds__(kCeThreads)
   if (threadIdx.x == 0) out[0] = red[0] * scale;
 }
 
-// dlogits[n,c] = (softmax(z_n)[c] - [c == y_n]) * scale * upstream[0]
+// dlogits[n,c] = (softmax(z_n)[c] - [c == y_n]) * scale * upstream[0], the label's class as -(sum of the other
+// classes' exp(z_c - m)) / s (1 - p_y cancels for a confident row); a row with a label outside [0, C) is NaN
 __global__ void __launch_bounds__(kCeThreads)
     k_ce_bwd(const float* __restrict__ logits, const int64_t* __restrict__ target, int64_t N, int C,
              float scale, const float* __restrict__ upstream, float* __restrict__ dlogits) {
@@ -65,14 +77,15 @@ __global__ void __launch_bounds__(kCeThreads)
     const float* z = logits + n * C;
     float m = z[0];
     for (int c = 1; c < C; ++c) m = fmaxf(m, z[c]);
-    float s = 0.f;
-    for (int c = 0; c < C; ++c) s += expf(z[c] - m);
-    const float inv = 1.f / s;
     const int64_t y = target[n];
+    float s = 0.f, t = 0.f;
     for (int c = 0; c < C; ++c) {
-      const float p = expf(z[c] - m) * inv;
-      dlogits[n * C + c] = (p - (c == y ? 1.f : 0.f)) * g;
+      const float e = expf(z[c] - m);
+      s += e;
+      if (c != y) t += e;
     }
+    const float inv = (y < 0 || y >= C) ? __int_as_float(0x7fc00000) : 1.f / s;
+    for (int c = 0; c < C; ++c) dlogits[n * C + c] = (c == y ? -t : expf(z[c] - m)) * inv * g;
   }
 }
 
@@ -105,7 +118,8 @@ extern "C" int mgcn_cross_entropy_fwd(const float* logits, const int64_t* target
   const int64_t rows_per_block = ceil_div(N > 0 ? N : 1, P);
   MGCN_LAUNCH(k_ce_fwd, P, kCeThreads, 0, stream, logits, target, N, (int)C, rows_per_block, partial,
               bad_target);
-  const float scale = mean ? (N > 0 ? 1.0f / (float)N : 0.f) : 1.f;
+  // the mean over no rows is NaN, as torch's
+  const float scale = mean ? (N > 0 ? 1.0f / (float)N : std::numeric_limits<float>::quiet_NaN()) : 1.f;
   MGCN_LAUNCH(k_ce_finish, 1, kCeThreads, 0, stream, partial, P, scale, loss);
   return MGCN_OK;
 }

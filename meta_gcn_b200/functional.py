@@ -131,10 +131,11 @@ class _HeadCrossEntropy(torch.autograd.Function):
         ctx.mean = bool(mean)
         ctx.has_bias = bias is not None
         ctx.save_for_backward(x, logits, weight, target)
-        ctx.mark_non_differentiable(logits)
+        # one call: each call replaces the set of non-differentiable outputs
         if counts is not None:
-            ctx.mark_non_differentiable(counts)
+            ctx.mark_non_differentiable(logits, counts)
             return loss.view(()), logits, counts
+        ctx.mark_non_differentiable(logits)
         return loss.view(()), logits
 
     @staticmethod
@@ -150,7 +151,8 @@ def head_cross_entropy(x, linear, target, reduction="mean", confusion=False):
     counters TP / FP / TN / FN / correct of optim/metrics.py:8-24 in one forward and one backward launch
     (csrc/head.cu; gcn_model.py:73,108 + train_botnet.py:287,296-305).  ``linear``: an nn.Linear(H, C), H in
     {16,32,64,128}, C <= 8.  Returns (loss, logits[, counts int64[5]]); the logits are detached (the loss carries the
-    gradient to x and to the layer's parameters)."""
+    gradient to x and to the layer's parameters).  A label outside [0, C) (-100 included) makes the loss NaN and that
+    row's gradient NaN, and the counters skip the row; the mean over no rows is NaN (include/mgcn.h)."""
     if reduction not in ("mean", "sum"):
         raise ValueError("reduction must be 'mean' or 'sum'")
     return _HeadCrossEntropy.apply(x, linear.weight, linear.bias, target, reduction == "mean", bool(confusion))
@@ -320,7 +322,9 @@ class _CrossEntropy(torch.autograd.Function):
 
 def cross_entropy(logits, target, reduction="mean"):
     """nn.CrossEntropyLoss(reduction=...)(logits, target) over node logits (train_botnet.py:225,287)
-    as two deterministic kernels; target is int64 class ids."""
+    as two deterministic kernels; target is int64 class ids.  A label outside [0, C) (-100 included: there is no
+    ignore_index) makes the loss NaN and that row's gradient NaN, without a host synchronisation; the mean over no
+    rows is NaN, as torch's."""
     if reduction not in ("mean", "sum"):
         raise ValueError("reduction must be 'mean' or 'sum'")
     return _CrossEntropy.apply(logits, target, reduction == "mean")
