@@ -308,6 +308,14 @@ int mgcn_gcn_first_layer_fwd_ex(const float* s, const float* x, int64_t N, int64
                                 const float* res_w, const float* res_b, const float* w_next, const float* pre,
                                 const float* post, const float* out_scale, const uint32_t* keep, float keep_scale,
                                 int act_out, int64_t H, float* x_next, float* m_next, uint32_t* hmask, void* stream);
+/* The same with the node-model bias (NodeModelAdditive's default bias=True; gcn_base_models.py:241), bias [32]:
+ *     h = relu(post * (s W_in) + bias)   (one rounded fp32 add after the post multiply, then the ReLU, then dropout)
+ * bias == NULL: exactly mgcn_gcn_first_layer_fwd_ex.  Both the streaming pass and the tile kernel take it. */
+int mgcn_gcn_first_layer_fwd_bias(const float* s, const float* x, int64_t N, int64_t Hin, const float* w_in,
+                                  const float* res_w, const float* res_b, const float* bias, const float* w_next,
+                                  const float* pre, const float* post, const float* out_scale, const uint32_t* keep,
+                                  float keep_scale, int act_out, int64_t H, float* x_next, float* m_next,
+                                  uint32_t* hmask, void* stream);
 
 /* One residual GCN layer forward at hidden 32, AGGREGATE-THEN-TRANSFORM, on tcgen05.mma / tensor memory
  * (csrc/gcn_fwd_tc.cu) — the default of the hidden-32 stack.  Same reference lines as mgcn_gcn_layer_fwd
@@ -364,6 +372,21 @@ int mgcn_gcn_layer_bwd_tc(const float* dxw, const float* gy, const float* x, con
                           const float* res_w, const uint32_t* hmask_prev, const float* post, int64_t N,
                           int64_t H, float* gy_prev, float* gs_prev, float* dw, float* d_res_w,
                           float* d_res_b, void* workspace, size_t* workspace_bytes, void* stream);
+/* The same with the gradient of the node-model bias of the layer.  With gy = the gradient of the layer's output
+ * before its activation (the gy above), hmask_cur = this layer's mask words (bit c = relu'(h) & kept) and
+ * bias_scale = the dropout scale 1 / (1 - p) (1 without dropout):
+ *     d_bias[c] = bias_scale * sum_i (bit c of hmask_cur[i]) * gy[i,c]
+ * The per-target factor post does not enter it (d_bias is not a column sum of gs: post may be 0).  Computed after the
+ * row-local launch by the pass of mgcn_mask_bits_colsum (two more launches, one more read of gy: summed inside the
+ * row-local kernel it spills), in a fixed order, so it is identical from run to run; every other output is
+ * bit-identical to mgcn_gcn_layer_bwd_tc.  d_bias == NULL: exactly mgcn_gcn_layer_bwd_tc (hmask_cur and bias_scale
+ * unused); d_bias needs hmask_cur (else MGCN_ERR_NULL).  The workspace is larger with d_bias (query with the same
+ * arguments). */
+int mgcn_gcn_layer_bwd_tc_ex(const float* dxw, const float* gy, const float* x, const float* x_scale, const float* w,
+                             const float* res_w, const uint32_t* hmask_prev, const uint32_t* hmask_cur,
+                             const float* post, float bias_scale, int64_t N, int64_t H, float* gy_prev,
+                             float* gs_prev, float* dw, float* d_res_w, float* d_res_b, float* d_bias,
+                             void* workspace, size_t* workspace_bytes, void* stream);
 
 /* The backward of one hidden-32 layer as ONE launch (csrc/gcn_bwd_fused.cu): mgcn_aggregate_prescaled over the
  * by-source structure `gt` followed by mgcn_gcn_layer_bwd_tc, without the [N,32] array between them —
@@ -381,6 +404,13 @@ int mgcn_gcn_layer_bwd_fused(const mgcn_csr_t* gt, const float* gs, const float*
 /* gs[i,c] = post[i] * gy[i,c] * bit c of bits[i]   (H = 32; post may be NULL) */
 int mgcn_mask_bits_scale(const float* gy, const uint32_t* bits, const float* post, int64_t N,
                          int64_t H, float* gs, void* stream);
+
+/* d_bias[c] = scale * sum_i (bit c of bits[i]) * gy[i,c]   (H = 32): the node-model bias gradient of a layer without a
+ * row-local backward launch (the narrow-input first layer), the formula of mgcn_gcn_layer_bwd_tc_ex.  Per-block partial
+ * sums over a grid that depends on N only, then one block adds them in a fixed order: identical from run to run.
+ * N == 0 writes zeros.  Two launches; workspace query as elsewhere (workspace == NULL). */
+int mgcn_mask_bits_colsum(const float* gy, const uint32_t* bits, float scale, int64_t N, int64_t H, float* d_bias,
+                          void* workspace, size_t* workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Dropout keep masks of the residual stack — nn.Dropout(p) of gcn_model.py:92 on every layer's h, as bits.

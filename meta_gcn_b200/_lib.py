@@ -69,6 +69,8 @@ SIGNATURES = {
                                          c_int, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
     "mgcn_gcn_first_layer_fwd_ex": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                             c_ptr, c_ptr, c_f32, c_int, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "mgcn_gcn_first_layer_fwd_bias": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                              c_ptr, c_ptr, c_ptr, c_f32, c_int, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
     "mgcn_gcn_layer_fwd_tc": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int,
                                       c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_fwd_tc_ex": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
@@ -105,9 +107,12 @@ SIGNATURES = {
                                    c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_bwd_tc": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr,
                                       c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
+    "mgcn_gcn_layer_bwd_tc_ex": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_f32, c_i64,
+                                         c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_bwd_fused": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64,
                                          c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_mask_bits_scale": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_ptr]),
+    "mgcn_mask_bits_colsum": (c_int, [c_ptr, c_ptr, c_f32, c_i64, c_i64, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_dropout_keep_bits": (c_int, [c_ptr, c_i64, c_i64, c_i64, c_f32, c_ptr, c_ptr]),
     "mgcn_dropout_apply": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_i64, c_f32, c_ptr]),
     "mgcn_cross_entropy_fwd": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_int, c_ptr, c_ptr, c_ptr, c_size_p,

@@ -99,10 +99,17 @@ int launch_agg_flat32(const mgcn_csr_t* g, const float* x, const float* post, in
 size_t bwd_tc_workspace_floats(int64_t N);
 int launch_layer_bwd_tc(const float* dxw, const float* gy, const float* x, const float* x_scale, const float* w, const float* res_w,
                         const uint32_t* hmask_prev, const float* post, int64_t N, float* gy_prev, float* gs_prev,
-                        float* dw, float* d_res_w, float* d_res_b, float* ws, void* stream);
+                        float* dw, float* d_res_w, float* d_res_b, float* ws, void* stream,
+                        const uint32_t* hmask_cur = nullptr, float bias_scale = 1.f, float* d_bias = nullptr);
+// floats the launch above needs beyond bwd_tc_workspace_floats when d_bias is given (the masked column sum's partials)
+size_t bwd_tc_bias_workspace_floats(int64_t N);
 // dW / dR from per-CTA partials [P][128][32] of the transposed tcgen05 products, fixed order (gcn_layer_tc.cu)
 int launch_bwd_tc_reduce(const float* part, int P, float* dw, float* d_res_w, const float* part_b, int Pb,
                          float* d_res_b, void* stream);
+// d_bias[c] = scale * sum_i bit c of bits[i] * gy[i][c] over [N][32], two fixed-order levels (gcn_layer_tc.cu)
+size_t mask_bits_colsum_workspace_floats(int64_t N);
+int launch_mask_bits_colsum(const float* gy, const uint32_t* bits, float scale, int64_t N, float* d_bias, float* ws,
+                            void* stream);
 // narrow-side dense transforms (dense_narrow.cu)
 bool narrow_linear_applies(int64_t Hi, int64_t Ho, const float* x, const float* xmask, const float* add,
                            const float* y);

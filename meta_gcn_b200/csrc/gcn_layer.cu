@@ -1082,6 +1082,18 @@ extern "C" int mgcn_gcn_first_layer_fwd_ex(const float* s, const float* x, int64
                                            const float* pre, const float* post, const float* out_scale,
                                            const uint32_t* keep, float keep_scale, int act_out, int64_t H,
                                            float* x_next, float* m_next, uint32_t* hmask, void* stream) {
+  return mgcn_gcn_first_layer_fwd_bias(s, x, N, Hin, w_in, res_w, res_b, nullptr, w_next, pre, post, out_scale, keep,
+                                       keep_scale, act_out, H, x_next, m_next, hmask, stream);
+}
+
+// The same with the node-model bias b [32] (NodeModelAdditive's default bias=True), added where the reference adds it:
+// h = relu(post * (s W_in) + b), before the dropout (both kernels: finish_h / the streaming epilogue).
+extern "C" int mgcn_gcn_first_layer_fwd_bias(const float* s, const float* x, int64_t N, int64_t Hin, const float* w_in,
+                                             const float* res_w, const float* res_b, const float* bias,
+                                             const float* w_next, const float* pre, const float* post,
+                                             const float* out_scale, const uint32_t* keep, float keep_scale,
+                                             int act_out, int64_t H, float* x_next, float* m_next, uint32_t* hmask,
+                                             void* stream) {
   MGCN_REQUIRE(H == kH, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(!(keep && w_next), MGCN_ERR_SHAPE);   // dropout only in the streaming pass
   MGCN_REQUIRE(Hin >= 1 && Hin <= 4, MGCN_ERR_SHAPE);
@@ -1097,6 +1109,7 @@ extern "C" int mgcn_gcn_first_layer_fwd_ex(const float* s, const float* x, int64
   a.keep = keep; a.keep_scale = keep_scale;
   a.resid = x_next;   // row-local mode with a finished residual term: the tail reads it from the tile, never from here
   a.res_w = res_w; a.res_b = res_b; a.w_next = w_next; a.pre = pre; a.out_scale = out_scale;
+  a.bias = bias;
   a.x_next = x_next; a.m_next = m_next; a.hmask = hmask;
   a.n_rows = N;
   a.act_out = act_out;
@@ -1172,17 +1185,30 @@ extern "C" int mgcn_gcn_layer_bwd_tc(const float* dxw, const float* gy, const fl
                                      int64_t N, int64_t H, float* gy_prev, float* gs_prev, float* dw,
                                      float* d_res_w, float* d_res_b, void* workspace,
                                      size_t* workspace_bytes, void* stream) {
+  return mgcn_gcn_layer_bwd_tc_ex(dxw, gy, x, x_scale, w, res_w, hmask_prev, nullptr, post, 1.f, N, H, gy_prev, gs_prev,
+                                  dw, d_res_w, d_res_b, nullptr, workspace, workspace_bytes, stream);
+}
+
+// + the node-model bias gradient d_bias = bias_scale * colsum(gy * bits(hmask_cur)), summed by the producer warps next
+// to dr and reduced in the same launch (k_layer_bwd_tc<true>); d_bias == NULL: the kernel without it.
+extern "C" int mgcn_gcn_layer_bwd_tc_ex(const float* dxw, const float* gy, const float* x, const float* x_scale,
+                                        const float* w, const float* res_w, const uint32_t* hmask_prev,
+                                        const uint32_t* hmask_cur, const float* post, float bias_scale, int64_t N,
+                                        int64_t H, float* gy_prev, float* gs_prev, float* dw, float* d_res_w,
+                                        float* d_res_b, float* d_bias, void* workspace, size_t* workspace_bytes,
+                                        void* stream) {
   MGCN_REQUIRE(workspace_bytes != nullptr, MGCN_ERR_NULL);
   MGCN_REQUIRE(H == kH, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(N >= 0 && N < (int64_t(1) << 31), MGCN_ERR_RANGE);
   WorkspaceCarver ws(workspace);
-  float* tc_ws = ws.take<float>(bwd_tc_workspace_floats(N));
+  float* tc_ws = ws.take<float>(bwd_tc_workspace_floats(N) + (d_bias ? bwd_tc_bias_workspace_floats(N) : 0));
   if (workspace == nullptr) {
     *workspace_bytes = ws.bytes();
     return MGCN_OK;
   }
   MGCN_REQUIRE(*workspace_bytes >= ws.bytes(), MGCN_ERR_WORKSPACE);
   MGCN_REQUIRE(dxw && gy && x && w && res_w && dw && d_res_w && d_res_b, MGCN_ERR_NULL);
+  MGCN_REQUIRE(!d_bias || hmask_cur, MGCN_ERR_NULL);
   MGCN_REQUIRE((gy_prev == nullptr) == (gs_prev == nullptr), MGCN_ERR_NULL);
   MGCN_REQUIRE(!gy_prev || hmask_prev, MGCN_ERR_NULL);
   MGCN_REQUIRE(aligned16(dxw) && aligned16(gy) && aligned16(x) && (!gy_prev || aligned16(gy_prev)) &&
@@ -1190,7 +1216,7 @@ extern "C" int mgcn_gcn_layer_bwd_tc(const float* dxw, const float* gy, const fl
                MGCN_ERR_ALIGN);
   if (N == 0) return MGCN_OK;
   return launch_layer_bwd_tc(dxw, gy, x, x_scale, w, res_w, hmask_prev, post, N, gy_prev, gs_prev, dw, d_res_w,
-                             d_res_b, tc_ws, stream);
+                             d_res_b, tc_ws, stream, hmask_cur, bias_scale, d_bias);
 }
 
 extern "C" int mgcn_mask_bits_scale(const float* gy, const uint32_t* bits, const float* post,
@@ -1204,4 +1230,22 @@ extern "C" int mgcn_mask_bits_scale(const float* gy, const uint32_t* bits, const
   if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
   MGCN_LAUNCH(k_mask_bits_scale, (unsigned)blocks, 256, 0, stream, gy, bits, post, N, gs);
   return MGCN_OK;
+}
+
+// d_bias[c] = scale * sum_i bit c of bits[i] * gy[i][c]: the bias gradient of a layer without a row-local launch
+extern "C" int mgcn_mask_bits_colsum(const float* gy, const uint32_t* bits, float scale, int64_t N, int64_t H,
+                                     float* d_bias, void* workspace, size_t* workspace_bytes, void* stream) {
+  MGCN_REQUIRE(workspace_bytes != nullptr, MGCN_ERR_NULL);
+  MGCN_REQUIRE(H == kH, MGCN_ERR_SHAPE);
+  MGCN_REQUIRE(N >= 0 && N < (int64_t(1) << 31), MGCN_ERR_RANGE);
+  WorkspaceCarver ws(workspace);
+  float* part = ws.take<float>(mask_bits_colsum_workspace_floats(N));
+  if (workspace == nullptr) {
+    *workspace_bytes = ws.bytes();
+    return MGCN_OK;
+  }
+  MGCN_REQUIRE(*workspace_bytes >= ws.bytes(), MGCN_ERR_WORKSPACE);
+  MGCN_REQUIRE(d_bias && (N == 0 || (gy && bits)), MGCN_ERR_NULL);
+  MGCN_REQUIRE(aligned16(gy), MGCN_ERR_ALIGN);
+  return launch_mask_bits_colsum(gy, bits, scale, N, d_bias, part, stream);   // N == 0: zeros
 }

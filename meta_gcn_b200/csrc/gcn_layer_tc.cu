@@ -507,10 +507,12 @@ int bwd_tc_grid(int64_t N) {
 }
 
 size_t bwd_tc_workspace_floats(int64_t N) { return (size_t)bwd_tc_grid(N) * (128 * 32 + 32); }
+size_t bwd_tc_bias_workspace_floats(int64_t N) { return mask_bits_colsum_workspace_floats(N); }
 
 int launch_layer_bwd_tc(const float* dxw, const float* gy, const float* x, const float* x_scale, const float* w, const float* res_w,
                         const uint32_t* hmask_prev, const float* post, int64_t N, float* gy_prev, float* gs_prev,
-                        float* dw, float* d_res_w, float* d_res_b, float* ws, void* stream) {
+                        float* dw, float* d_res_w, float* d_res_b, float* ws, void* stream,
+                        const uint32_t* hmask_cur, float bias_scale, float* d_bias) {
   const int P = bwd_tc_grid(N);
   BwdTcArgs a{};
   a.dxw = dxw; a.gy = gy; a.x = x; a.x_scale = x_scale; a.w = w; a.res_w = res_w; a.hmask_prev = hmask_prev; a.post = post;
@@ -526,7 +528,83 @@ int launch_layer_bwd_tc(const float* dxw, const float* gy, const float* x, const
   }
   MGCN_CHECK_CUDA(attr_err);
   MGCN_LAUNCH(k_layer_bwd_tc, P, kBwdTcThreads, kBwdTcSmem, stream, a);
-  return launch_bwd_tc_reduce(a.part_t, P, dw, d_res_w, a.part_b, P, d_res_b, stream);   // dW, dR and dr: one launch
+  const int rc = launch_bwd_tc_reduce(a.part_t, P, dw, d_res_w, a.part_b, P, d_res_b, stream);   // dW, dR and dr: one launch
+  if (rc != MGCN_OK || !d_bias) return rc;
+  // the node-model bias gradient as its own pass over gy: summed by the producer warps above, next to dr, the kernel
+  // needs 8 more live registers than its 80 and spills (profiles/bias_ptxas.log)
+  return launch_mask_bits_colsum(gy, hmask_cur, bias_scale, N, d_bias, ws + bwd_tc_workspace_floats(N), stream);
+}
+
+// ---- masked column sum: the node-model bias gradient,  d_bias[c] = scale * sum_i bit c of bits[i] * gy[i][c] ----
+// Lane 8 q + k of a warp reads columns 4k .. 4k + 3 of row 4 w + q of the block's 32-row step: one float4 per lane, 512
+// contiguous bytes per warp.  The 4 rows of a warp are added by a fixed butterfly, the 8 warps of a block in order,
+// the per-block partials by one block (8 contiguous runs, then the runs in order).  The grid depends on N (and the
+// SM count) only, so the result is the same from run to run.
+constexpr int kColsumRows = 32;   // rows per block and step: 8 warps x 4 rows
+__global__ void __launch_bounds__(256) k_mask_bits_colsum(const float* __restrict__ gy, const uint32_t* __restrict__ bits,
+                                                          int64_t n_rows, float* __restrict__ part) {
+  __shared__ float red[8][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int q = lane >> 3, k = lane & 7;
+  float acc[4] = {0.f, 0.f, 0.f, 0.f};
+  const int64_t stride = (int64_t)gridDim.x * kColsumRows;
+  const uint64_t pol = policy_evict_first();
+#pragma unroll 4
+  for (int64_t r = (int64_t)blockIdx.x * kColsumRows + 4 * warp + q; r < n_rows; r += stride) {
+    const float4 g = ld_f4_hint(gy + r * kTH + 4 * k, pol);
+    const uint32_t m = __ldg(bits + r) >> (4 * k);
+    acc[0] += (m & 1u) ? g.x : 0.f;
+    acc[1] += (m & 2u) ? g.y : 0.f;
+    acc[2] += (m & 4u) ? g.z : 0.f;
+    acc[3] += (m & 8u) ? g.w : 0.f;
+  }
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    float v = acc[t];
+    v += __shfl_xor_sync(0xffffffffu, v, 8);
+    v += __shfl_xor_sync(0xffffffffu, v, 16);
+    if (q == 0) red[warp][4 * k + t] = v;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    float s = red[0][lane];
+#pragma unroll
+    for (int w = 1; w < 8; ++w) s += red[w][lane];
+    part[(int64_t)blockIdx.x * 32 + lane] = s;
+  }
+}
+
+// out[c] = scale * sum_p part[p][c]: warp w sums a contiguous run of partials, warp 0 adds the 8 runs in order
+__global__ void __launch_bounds__(256) k_colsum_reduce(const float* __restrict__ part, int P, float scale,
+                                                       float* __restrict__ out) {
+  __shared__ float red[8][33];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int per = (P + 7) / 8, p0 = warp * per, p1 = min(P, p0 + per);
+  float s = 0.f;
+  for (int p = p0; p < p1; ++p) s += part[(int64_t)p * 32 + lane];
+  red[warp][lane] = s;
+  __syncthreads();
+  if (warp == 0) {
+    float t = red[0][lane];
+#pragma unroll
+    for (int w = 1; w < 8; ++w) t += red[w][lane];
+    out[lane] = t * scale;
+  }
+}
+
+static int colsum_grid(int64_t N) {
+  const int64_t blocks = ceil_div(N > 0 ? N : 1, kColsumRows);
+  return (int)(blocks < (int64_t)kNumSMs * 8 ? blocks : (int64_t)kNumSMs * 8);
+}
+
+size_t mask_bits_colsum_workspace_floats(int64_t N) { return (size_t)colsum_grid(N) * 32; }
+
+int launch_mask_bits_colsum(const float* gy, const uint32_t* bits, float scale, int64_t N, float* d_bias, float* ws,
+                            void* stream) {
+  const int P = colsum_grid(N);
+  MGCN_LAUNCH(k_mask_bits_colsum, P, 256, 0, stream, gy, bits, N, ws);
+  MGCN_LAUNCH(k_colsum_reduce, 1, 256, 0, stream, ws, P, scale, d_bias);
+  return MGCN_OK;
 }
 
 }  // namespace mgcn

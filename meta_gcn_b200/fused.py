@@ -193,18 +193,22 @@ class _ResidualGCNStack32(torch.autograd.Function):
 
 
 class _ResidualGCNStack32AT(torch.autograd.Function):
-    """hidden width 32, no node-model bias, AGGREGATE-THEN-TRANSFORM: (A_hat x) W instead of A_hat (x W).  One
+    """hidden width 32, with or without node-model bias, AGGREGATE-THEN-TRANSFORM: (A_hat x) W instead of A_hat (x W).  One
     tcgen05 launch per layer forward (csrc/gcn_fwd_tc.cu) that reads one [N,32] array and writes one: activations are
     stored as z_n = sigma (.) x_n (sigma = the per-source degree factor, 1 where that factor is 0 — such a row is
     never a source when the degree is the graph's own out-degree), so the gather needs no per-edge weight and no
     separate message array; the row-local terms divide sigma out per row.  Saved per layer: z_n and one mask word
     per row.  Backward: dW_n = x_n^T (A_hat^T ga), dx = (A_hat^T ga) W_n^T + gy R_n — the transposed aggregation of
-    the masked gradient, then the row-local tcgen05 launch."""
+    the masked gradient, then the row-local tcgen05 launch.  Parameters per layer: (W, [b], R, r); the bias adds
+    before the ReLU in the layer kernels, and its gradient is the column sum of gy under the layer's mask word times
+    the dropout scale (post does not enter it)."""
 
     @staticmethod
-    def forward(ctx, x, graph, pre, post, last_relu, p, *params):
-        L = len(params) // 3
-        layers = [params[i * 3:(i + 1) * 3] for i in range(L)]
+    def forward(ctx, x, graph, pre, post, has_bias, last_relu, p, *params):
+        per = 4 if has_bias else 3
+        L = len(params) // per
+        layers = [params[i * per:(i + 1) * per] for i in range(L)]
+        bias = (lambda n: layers[n][1]) if has_bias else (lambda n: None)
         fwd = graph.fwd_plain
         x0 = x.contiguous()
         sigma = None
@@ -220,8 +224,8 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             xs0 = x0 * pre.unsqueeze(1) if pre is not None else x0            # pre_j x_j, one rounding as in the gather
             s0 = ops.spmm_impl(fwd, xs0)                                      # [N, H_in]
             z, _, hm = ops.gcn_first_layer_fwd_impl(
-                s0, x0, layers[0][0], layers[0][1], layers[0][2], None, None, post,
-                1 if (last_relu or L > 1) else 0, out_scale=sigma if L > 1 else None, **drop(0))
+                s0, x0, layers[0][0], layers[0][-2], layers[0][-1], None, None, post,
+                1 if (last_relu or L > 1) else 0, out_scale=sigma if L > 1 else None, bias=bias(0), **drop(0))
             zs.append(None)
             hmasks.append(hm)
             first = 1
@@ -231,11 +235,12 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         for n in range(first, L):
             zs.append(z)
             z, hm = ops.gcn_layer_fwd_tc_impl(
-                fwd, z, layers[n][0], layers[n][1], layers[n][2], None, sigma, post,
+                fwd, z, layers[n][0], layers[n][-2], layers[n][-1], bias(n), sigma, post,
                 sigma if n < L - 1 else None, 1 if (last_relu or n < L - 1) else 0, **drop(n))
             hmasks.append(hm)
         ctx.agg_first = agg_first
-        ctx.graph, ctx.cfg = graph, (L, last_relu)
+        ctx.graph, ctx.cfg = graph, (L, per, has_bias, last_relu)
+        ctx.bias_scale = 1.0 if scale is None else scale
         # the backward reads `post` only where it scales a gradient by the mask words: the dropout scale goes there
         ctx.save_for_backward(x0, s0, pre, _scaled_post(post, scale, x0.size(0), x0), sigma, z if last_relu else None,
                               *[t for t in zs if t is not None], *hmasks, *params)
@@ -243,7 +248,7 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        L, last_relu = ctx.cfg
+        L, per, has_bias, last_relu = ctx.cfg
         saved = ctx.saved_tensors
         x0, s0, pre, post, sigma, out = saved[:6]
         nz = L - 1 if ctx.agg_first else L
@@ -252,7 +257,7 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             zs = [None] + zs
         hmasks = saved[6 + nz:6 + nz + L]
         params = saved[6 + nz + L:]
-        layers = [params[i * 3:(i + 1) * 3] for i in range(L)]
+        layers = [params[i * per:(i + 1) * per] for i in range(L)]
         bwd = ctx.graph.bwd_plain
         grads = [None] * len(params)
         gy = g.contiguous()
@@ -262,22 +267,33 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         last = 1 if ctx.agg_first else 0
         for n in range(L - 1, last - 1, -1):
             want_prev = n > 0
-            if BWD_FUSED:
+            w, res_w = layers[n][0], layers[n][-2]
+            if has_bias:
+                # the one-launch backward (BWD_FUSED) has no bias gradient: a model with bias takes the two launches
+                dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
+                gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
+                    dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, hmasks[n], post, ctx.bias_scale,
+                    want_prev, x_scale=sigma)
+                grads[per * n + 1] = db
+            elif BWD_FUSED:
                 gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_fused_impl(
-                    bwd, gs, gy, zs[n], layers[n][0], layers[n][1], hmasks[n - 1] if want_prev else None, post,
+                    bwd, gs, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
                     row_scale=pre, x_scale=sigma, want_prev=want_prev)
             else:
                 dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
                 gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_impl(
-                    dxw, gy, zs[n], layers[n][0], layers[n][1], hmasks[n - 1] if want_prev else None, post,
+                    dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
                     want_prev, True, x_scale=sigma)
-            grads[3 * n], grads[3 * n + 1], grads[3 * n + 2] = dw, drw, drb
+            grads[per * n], grads[per * n + per - 2], grads[per * n + per - 1] = dw, drw, drb
             if want_prev:
                 gy, gs = gy_prev, gs_prev
         if ctx.agg_first:
-            grads[1], grads[2] = ops.linear_wgrad_impl(x0, gy, True, True)
+            grads[per - 2], grads[per - 1] = ops.linear_wgrad_impl(x0, gy, True, True)
             grads[0] = ops.linear_wgrad_impl(s0, gs, False, False)[0]    # dW0 = s0^T gs0
-        return (None, None, None, None, None, None, *grads)
+            if has_bias:
+                # no row-local launch for layer 0: its bias gradient is a pass of its own
+                grads[1] = ops.mask_bits_colsum_impl(gy, hmasks[0], ctx.bias_scale)
+        return (None, None, None, None, None, None, None, *grads)
 
 
 def residual_gcn_stack(x, graph, pre, post, layer_params, has_bias, last_relu=False, aggregate_first=True,
@@ -291,9 +307,10 @@ def residual_gcn_stack(x, graph, pre, post, layer_params, has_bias, last_relu=Fa
         raise ValueError(f"dropout must be in [0, 1), got {dropout}")
     flat = [p for lp in layer_params for p in lp]
     widths = {lp[0].size(1) for lp in layer_params} | {lp[0].size(0) for lp in layer_params[1:]}
+    if widths == {32} and FORWARD_AGGREGATE_FIRST and aggregate_first and not x.requires_grad and \
+            (x.size(1) <= 4 or x.size(1) == 32):
+        return _ResidualGCNStack32AT.apply(x, graph, pre, post, has_bias, last_relu, dropout, *flat)
     if not has_bias and widths == {32}:
-        if FORWARD_AGGREGATE_FIRST and aggregate_first and not x.requires_grad and (x.size(1) <= 4 or x.size(1) == 32):
-            return _ResidualGCNStack32AT.apply(x, graph, pre, post, last_relu, dropout, *flat)
         if dropout > 0:
             return None
         return _ResidualGCNStack32.apply(x, graph, pre, post, last_relu, *flat)

@@ -486,11 +486,13 @@ def gcn_layer_fwd_impl(csr, m, x, resid, res_w, res_b, w_next, bias, pre, post, 
 
 
 def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_out, out_scale=None, keep=None,
-                             keep_scale=1.0):
+                             keep_scale=1.0, bias=None):
     """first layer with a narrow input (mgcn_gcn_first_layer_fwd_ex): s = aggregated input [N,Hin], x = layer input
     [N,Hin]; returns (x_next [N,32], m_next | None, hmask int32[N]); out_scale [N]: x_next rows leave scaled;
-    keep int32 [N] (w_next None only): dropout keep bits of the layer, kept entries of h multiplied by keep_scale"""
-    _need_cuda(s, x, w_in, res_w, res_b, w_next, pre, post, out_scale, keep)
+    keep int32 [N] (w_next None only): dropout keep bits of the layer, kept entries of h multiplied by keep_scale;
+    bias [32]: the node-model bias, h = relu(post (s W) + bias) (mgcn_gcn_first_layer_fwd_bias)"""
+    _need_cuda(s, x, w_in, res_w, res_b, w_next, pre, post, out_scale, keep, bias)
+    bias = _f32c(bias, "bias")
     out_scale = _f32c(out_scale, "out_scale")
     s = _f32c(s, "s")
     x = _f32c(x, "x")
@@ -509,7 +511,16 @@ def gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_ou
     m_next = torch.empty(N, H, dtype=torch.float32, device=dev) if w_next is not None else None
     hmask = torch.empty(N, dtype=torch.int32, device=dev)
     keep = _keep_rows(keep, N, 1)
-    _lib.check(_lib.load().mgcn_gcn_first_layer_fwd_ex(
+    lib = _lib.load()
+    if bias is not None:
+        if bias.numel() != H:
+            raise ValueError(f"bias must have {H} entries, got {bias.numel()}")
+        _lib.check(lib.mgcn_gcn_first_layer_fwd_bias(
+            _ptr(s), _ptr(x), N, Hin, _ptr(w_in), _ptr(res_w), _ptr(res_b), _ptr(bias), _ptr(w_next), _ptr(pre),
+            _ptr(post), _ptr(out_scale), _ptr(keep), float(keep_scale), int(act_out), H, _ptr(x_next), _ptr(m_next),
+            _ptr(hmask), _stream()))
+        return x_next, m_next, hmask
+    _lib.check(lib.mgcn_gcn_first_layer_fwd_ex(
         _ptr(s), _ptr(x), N, Hin, _ptr(w_in), _ptr(res_w), _ptr(res_b), _ptr(w_next), _ptr(pre), _ptr(post),
         _ptr(out_scale), _ptr(keep), float(keep_scale), int(act_out), H, _ptr(x_next), _ptr(m_next), _ptr(hmask),
         _stream()))
@@ -596,6 +607,53 @@ def gcn_layer_bwd_impl(dxw, gy, x, w, res_w, hmask_prev, post, want_prev=True, t
     ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
     _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
     return gy_prev, gs_prev, dw, drw, drb
+
+
+def gcn_layer_bwd_bias_impl(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, bias_scale=1.0, want_prev=True,
+                            x_scale=None):
+    """gcn_layer_bwd_impl on tcgen05 plus the node-model bias gradient (mgcn_gcn_layer_bwd_tc_ex): returns
+    (gy_prev | None, gs_prev | None, dw, d_res_w, d_res_b, d_bias) with
+    d_bias[c] = bias_scale * sum_i bit c of hmask_cur[i] * gy[i,c]   (hmask_cur: this layer's mask words)"""
+    _need_cuda(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, x_scale)
+    if hmask_cur is None:
+        raise ValueError("the bias gradient needs this layer's mask words (hmask_cur)")
+    x_scale = _f32c(x_scale, "x_scale")
+    dxw = _f32c(dxw, "dxw")
+    gy = _f32c(gy, "gy")
+    x = _f32c(x, "x")
+    w = _f32c(w, "w")
+    res_w = _f32c(res_w, "res_w")
+    post = _f32c(post, "post")
+    hmask_cur = _keep_rows(hmask_cur, x.size(0), 1)
+    N, H = x.shape
+    dev = x.device
+    gy_prev = torch.empty_like(x) if want_prev else None
+    gs_prev = torch.empty_like(x) if want_prev else None
+    dw = torch.empty(H, H, dtype=torch.float32, device=dev)
+    drw = torch.empty(H, H, dtype=torch.float32, device=dev)
+    drb = torch.empty(H, dtype=torch.float32, device=dev)
+    db = torch.empty(H, dtype=torch.float32, device=dev)
+    lib = _lib.load()
+    args = (_ptr(dxw), _ptr(gy), _ptr(x), _ptr(x_scale), _ptr(w), _ptr(res_w), _ptr(hmask_prev) if want_prev else None,
+            _ptr(hmask_cur), _ptr(post), float(bias_scale), N, H, _ptr(gy_prev), _ptr(gs_prev), _ptr(dw), _ptr(drw),
+            _ptr(drb), _ptr(db))
+    fn = lib.mgcn_gcn_layer_bwd_tc_ex
+    ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
+    _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
+    return gy_prev, gs_prev, dw, drw, drb, db
+
+
+def mask_bits_colsum_impl(gy, bits, scale=1.0):
+    """d_bias[c] = scale * sum_i bit c of bits[i] * gy[i,c]   (H = 32; fixed order, mgcn_mask_bits_colsum)"""
+    _need_cuda(gy, bits)
+    gy = _f32c(gy, "gy")
+    bits = _keep_rows(bits, gy.size(0), 1)
+    d_bias = torch.empty(gy.size(1), dtype=torch.float32, device=gy.device)
+    lib = _lib.load()
+    args = (_ptr(gy), _ptr(bits), float(scale), gy.size(0), gy.size(1), _ptr(d_bias))
+    ws, nbytes = _workspace(lambda w_, nb, stm: lib.mgcn_mask_bits_colsum(*args, w_, nb, stm), gy.device)
+    _lib.check(lib.mgcn_mask_bits_colsum(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
+    return d_bias
 
 
 def gcn_layer_bwd_fused_impl(csr_t, gs, gy, z, w, res_w, hmask_prev, post, row_scale=None, x_scale=None, want_prev=True):
@@ -1001,6 +1059,12 @@ _LIBDEF.define("gcn_first_layer_fwd(Tensor s, Tensor x, Tensor w_in, Tensor res_
 _LIBDEF.define("gcn_layer_bwd(Tensor dxw, Tensor gy, Tensor x, Tensor w, Tensor res_w, Tensor? hmask_prev, Tensor? post, "
                "bool want_prev, bool tensor_memory, Tensor? x_scale) -> (Tensor, Tensor, Tensor, Tensor, Tensor)")
 _LIBDEF.define("mask_bits_scale(Tensor gy, Tensor bits, Tensor? post) -> Tensor")
+_LIBDEF.define("gcn_first_layer_fwd_bias(Tensor s, Tensor x, Tensor w_in, Tensor res_w, Tensor? res_b, Tensor bias, "
+               "Tensor? w_next, Tensor? pre, Tensor? post, int act_out, Tensor? out_scale) -> (Tensor, Tensor, Tensor)")
+_LIBDEF.define("gcn_layer_bwd_bias(Tensor dxw, Tensor gy, Tensor x, Tensor w, Tensor res_w, Tensor? hmask_prev, "
+               "Tensor hmask_cur, Tensor? post, float bias_scale, bool want_prev, Tensor? x_scale) "
+               "-> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)")
+_LIBDEF.define("mask_bits_colsum(Tensor gy, Tensor bits, float scale) -> Tensor")
 _LIBDEF.define("dropout_keep_bits(Tensor seed, int L, int N, int W, float p) -> Tensor")
 _LIBDEF.define("segment_max(Tensor[] csr, int hub_threshold, Tensor x, bool gather_perm, Tensor? edge_val) -> (Tensor, Tensor)")
 _LIBDEF.define("segment_max_bwd(Tensor[] csr_t, int hub_threshold, Tensor grad, Tensor arg, Tensor? edge_val) -> Tensor")
@@ -1033,6 +1097,17 @@ def _op_layer_bwd(dxw, gy, x, w, res_w, hmask_prev, post, want_prev, tensor_memo
     return _none_to_empty(gyp, dw), _none_to_empty(gsp, dw), dw, drw, drb
 
 
+def _op_first_layer_fwd_bias(s, x, w_in, res_w, res_b, bias, w_next, pre, post, act_out, out_scale):
+    xn, mn, hm = gcn_first_layer_fwd_impl(s, x, w_in, res_w, res_b, w_next, pre, post, act_out, out_scale, bias=bias)
+    return xn, _none_to_empty(mn, xn), hm
+
+
+def _op_layer_bwd_bias(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, bias_scale, want_prev, x_scale):
+    gyp, gsp, dw, drw, drb, db = gcn_layer_bwd_bias_impl(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, bias_scale,
+                                                         want_prev, x_scale)
+    return _none_to_empty(gyp, dw), _none_to_empty(gsp, dw), dw, drw, drb, db
+
+
 def _op_edge_fingerprint(edge_index):
     _need_cuda(edge_index)
     ei = edge_index.contiguous()
@@ -1052,6 +1127,9 @@ _IMPLS2 = {
     "gcn_first_layer_fwd": _op_first_layer_fwd,
     "gcn_layer_bwd": _op_layer_bwd,
     "mask_bits_scale": mask_bits_scale_impl,
+    "gcn_first_layer_fwd_bias": _op_first_layer_fwd_bias,
+    "gcn_layer_bwd_bias": _op_layer_bwd_bias,
+    "mask_bits_colsum": mask_bits_colsum_impl,
     "dropout_keep_bits": dropout_keep_bits_impl,
     "segment_max": lambda csr, ht, x, gp, ev: segment_max_impl(_as_csr(csr, ht), x, gp, ev),
     "segment_max_bwd": lambda csr_t, ht, grad, arg, ev: segment_max_bwd_impl(_as_csr(csr_t, ht), grad, arg, ev),
@@ -1098,6 +1176,28 @@ def _(dxw, gy, x, w, res_w, hmask_prev, post, want_prev, tensor_memory, x_scale)
 @torch.library.register_fake("mgcn::mask_bits_scale")
 def _(gy, bits, post):
     return torch.empty_like(gy)
+
+
+@torch.library.register_fake("mgcn::gcn_first_layer_fwd_bias")
+def _(s, x, w_in, res_w, res_b, bias, w_next, pre, post, act_out, out_scale):
+    n, h = x.size(0), w_in.size(1)
+    return (torch.empty(n, h, dtype=torch.float32, device=x.device),
+            torch.empty((n, h) if w_next is not None else (0,), dtype=torch.float32, device=x.device),
+            torch.empty(n, dtype=torch.int32, device=x.device))
+
+
+@torch.library.register_fake("mgcn::gcn_layer_bwd_bias")
+def _(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, bias_scale, want_prev, x_scale):
+    h = x.size(1)
+    prev = torch.empty_like(x) if want_prev else torch.empty(0, dtype=torch.float32, device=x.device)
+    f = dict(dtype=torch.float32, device=x.device)
+    return (prev, torch.empty_like(prev), torch.empty(h, h, **f), torch.empty(h, h, **f), torch.empty(h, **f),
+            torch.empty(h, **f))
+
+
+@torch.library.register_fake("mgcn::mask_bits_colsum")
+def _(gy, bits, scale):
+    return torch.empty(gy.size(1), dtype=torch.float32, device=gy.device)
 
 
 @torch.library.register_fake("mgcn::dropout_keep_bits")
