@@ -342,6 +342,17 @@ int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int64_t n_in, 
                              const float* res_b, const float* bias, const float* in_scale, const float* post,
                              const float* out_scale, const uint32_t* keep, float keep_scale, int act_out, int64_t H,
                              float* z_next, uint32_t* hmask, void* workspace, size_t* workspace_bytes, void* stream);
+/* The same layer with an edge gate (EdgeGateProj, gcn_base_models.py:322-369) on every gathered row:
+ *     s_i = post_i * sum_{e: col[e]=i} g_e z[row[e]],   g_e = sigmoid(a_j + (b_i + c))   (j = row[e])
+ * gate_ab float2 [n_in] = per-node scores (a, b) from mgcn_gate_scores, gate_c [1] = the gate bias on the device (NULL =
+ * 0).  A gate is formed from the two endpoints while the row is gathered: no [E] array, no edge ids; hub segments are
+ * gated before their partials are stored.  Everything after the gather is the contract of mgcn_gcn_layer_fwd_tc_ex.
+ * gate_ab == NULL: exactly mgcn_gcn_layer_fwd_tc_ex (gate_c unused).  No allocation, capture-safe. */
+int mgcn_gcn_layer_fwd_tc_gate(const mgcn_csr_t* g, const float* z, int64_t n_in, const float* w, const float* res_w,
+                               const float* res_b, const float* bias, const float* in_scale, const float* post,
+                               const float* out_scale, const uint32_t* keep, float keep_scale, const float* gate_ab,
+                               const float* gate_c, int act_out, int64_t H, float* z_next, uint32_t* hmask,
+                               void* workspace, size_t* workspace_bytes, void* stream);
 /* The same layer with the A operands of its products in TENSOR MEMORY (csrc/gcn_fwd_tm.cu): the gather lanes write
  * their sums with tcgen05.st.16x256b, the products are tcgen05.mma with A from TMEM — no operand image passes
  * through shared memory (the layer kernels are bound by the LSU data pipe).  Same contract, same results within
@@ -400,6 +411,44 @@ int mgcn_gcn_layer_bwd_fused(const mgcn_csr_t* gt, const float* gs, const float*
                              const uint32_t* hmask_prev, const float* post, int64_t H,
                              float* gy_prev, float* gs_prev, float* dw, float* d_res_w, float* d_res_b, void* workspace,
                              size_t* workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Edge gates of the hidden-32 stack (csrc/gate.cu; EdgeGateProj, gcn_base_models.py:322-369, with in_edgedim None).
+ * The gate of an edge j -> i depends on its endpoints only: g_ij = sigmoid(a_j + (b_i + c)) with per-node scores
+ *     a_j = (x_j w) . u,   b_i = (x_i w) . v            (u = linsrc.weight[0], v = lintgt.weight[0], c = the gate bias)
+ * Every entry point forms g from the same operands in the same order, so all of them see the same gate bits.
+ * Sums run in edge_index order per row (hub rows: segment partials added in a fixed order): deterministic, no atomics.
+ *
+ * Scores: ab[i] = ((x_i . (w u)) / in_scale_i, (x_i . (w v)) / in_scale_i) as float2 [N] (w u formed per block in a fixed
+ * order).  x [N,H] with H <= 32 (H = 32 for the stored z = in_scale (.) x of the stack, in_scale [N] or NULL = 1);
+ * w [H][32] (in,out), u / v [32].  One launch, no workspace, capture-safe. */
+int mgcn_gate_scores(const float* x, int64_t N, int64_t H, const float* in_scale, const float* w, const float* u,
+                     const float* v, float* ab, void* stream);
+/* Gated aggregation of a narrow input (H <= 4: the first layer, aggregated before its transform):
+ *     out_i = sum_{e: col[e]=i} g_e x[row[e]]       over g's rowptr / nbr (row order = edge_index order)
+ * ab / c as above (c NULL = 0).  One warp per row, lane-strided partial sums added in a fixed tree order.  One launch,
+ * capture-safe. */
+int mgcn_gate_spmm_narrow(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, const float* ab,
+                          const float* c, float* out, void* stream);
+/* Backward of the gate, by target (g = the structure of the forward, grouped by target).  gs [N,32] = the masked,
+ * post-scaled gradient of the layer (mgcn_mask_bits_scale), m [N,32] = z w (= pre_j x_j w: the message before its gate):
+ *     dt_ij = <gs_i, m_j> * g_ij (1 - g_ij)                     (the gradient at the sigmoid's input)
+ *     db_i  = sum_{j: j->i} dt_ij                               -> db [N]
+ * Workspace: one float per hub segment (query with workspace == NULL).  Two launches with hub rows, else one;
+ * no allocation, capture-safe. */
+int mgcn_gate_grad_by_target(const mgcn_csr_t* g, const float* gs, const float* m, const float* ab, const float* c,
+                             float* db, void* workspace, size_t* workspace_bytes, void* stream);
+/* Backward of the gated aggregation by source (gt = grouped by source; the forward's structure when it is symmetric).
+ * With dt_ij computed exactly as in mgcn_gate_grad_by_target (the same bits) and db from it:
+ *     da_j  = sum_{i: j->i} dt_ij
+ *     dxw_j = pre_j * sum_{i: j->i} g_ij gs_i + da_j u + db_j v     (= dL / d(x_j w); pre NULL = 1)
+ *     dsc_j = (da_j / sigma_j, db_j / sigma_j, db_j)                 (sigma NULL = 1) -> dsc [N,3]
+ * so that [du | dv] = m^T dsc[:, 0:2] and dc = colsum(dsc[:, 2]) (one mgcn_linear_wgrad).  dxw enters
+ * mgcn_gcn_layer_bwd_tc(_ex) as the transposed aggregation would.  Workspace: one [33] float row per hub segment.
+ * Two launches with hub rows, else one; no allocation, capture-safe. */
+int mgcn_gate_grad_by_source(const mgcn_csr_t* gt, const float* gs, const float* m, const float* ab, const float* c,
+                             const float* db, const float* pre, const float* u, const float* v, const float* sigma,
+                             float* dxw, float* dsc, void* workspace, size_t* workspace_bytes, void* stream);
 
 /* gs[i,c] = post[i] * gy[i,c] * bit c of bits[i]   (H = 32; post may be NULL) */
 int mgcn_mask_bits_scale(const float* gy, const uint32_t* bits, const float* post, int64_t N,

@@ -75,6 +75,14 @@ SIGNATURES = {
                                       c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_fwd_tc_ex": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                          c_f32, c_int, c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
+    "mgcn_gcn_layer_fwd_tc_gate": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                           c_ptr, c_f32, c_ptr, c_ptr, c_int, c_i64, c_ptr, c_ptr, c_ptr, c_size_p,
+                                           c_ptr]),
+    "mgcn_gate_scores": (c_int, [c_ptr, c_i64, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "mgcn_gate_spmm_narrow": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "mgcn_gate_grad_by_target": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
+    "mgcn_gate_grad_by_source": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                         c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_fwd_tm": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int,
                                       c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_segment_max": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_int, c_ptr, c_ptr, c_ptr, c_ptr]),

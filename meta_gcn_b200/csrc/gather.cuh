@@ -74,14 +74,26 @@ __device__ __forceinline__ Row8 ld_row8_l1(const float* p) {
   return r;
 }
 
-template <bool kL1 = false>
+// Gate of an edge j -> i from two per-node scores (EdgeGateProj, gcn_base_models.py:322-369):
+// sigmoid(a_j + t_i) with t_i = b_i + c formed once per row.  Every kernel that needs a gate forms it with this one
+// function from the same two operands, so the gates of the forward and of both backward passes are the same bits.
+// ex2.approx and one rounded reciprocal (a few ulp of fp32, relative): an IEEE exp / divide costs the gated forward
+// layer kernel spills at its 80-register cap.
+__device__ __forceinline__ float edge_gate(float a_j, float t_i) {
+  return __frcp_rn(__fadd_rn(1.f, __expf(-__fadd_rn(a_j, t_i))));
+}
+
+// kGate: every gathered row is weighted by edge_gate(ab[j].x, gate_t) before it is added (one rounded multiply)
+template <bool kL1 = false, bool kGate = false>
 __device__ __forceinline__ Row8 gather_sum(const float* __restrict__ m, const int32_t* __restrict__ nbr_w,
                                            int beg, int end, int gi, int gi_n, int sub, int grp_lane0,
-                                           unsigned gmask, int col, uint64_t pol) {
+                                           unsigned gmask, int col, uint64_t pol,
+                                           const float2* __restrict__ ab = nullptr, float gate_t = 0.f) {
   Row8 acc;
 #pragma unroll
   for (int q = 0; q < 8; ++q) acc.v[q] = 0.f;
-  constexpr int U = MGCN_GATHER_U;
+  // gated: two rows in flight instead of four (with four, the gated forward layer kernel spills at its 80 registers)
+  constexpr int U = kGate ? 2 : MGCN_GATHER_U;
   int e = beg;
   while (e < end) {
     const int cnt = min(4, end - e);
@@ -95,13 +107,24 @@ __device__ __forceinline__ Row8 gather_sum(const float* __restrict__ m, const in
 #pragma unroll
         for (int u = 0; u < U; ++u) j[u] = __shfl_sync(gmask, gi, grp_lane0 + ((t0 + u) & 3));
         Row8 xv[U];
+        float sa[U];
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           if (t0 + u < cnt) xv[u] = kL1 ? ld_row8_l1(m + (int64_t)j[u] * kGH + col) : ld_row8(m + (int64_t)j[u] * kGH + col);
+          if constexpr (kGate) {
+            if (t0 + u < cnt) sa[u] = __ldg(&ab[j[u]].x);
+          }
         }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-          if (t0 + u < cnt) row8_add(acc, xv[u]);
+          if (t0 + u < cnt) {
+            if constexpr (kGate) {
+              const float gt = edge_gate(sa[u], gate_t);
+#pragma unroll
+              for (int q = 0; q < 8; ++q) xv[u].v[q] = __fmul_rn(gt, xv[u].v[q]);
+            }
+            row8_add(acc, xv[u]);
+          }
         }
       }
     }

@@ -98,6 +98,8 @@ struct FwdTcArgs {
   int64_t hub_cap;
   int act_out;
   int hub_threshold;
+  const float2* gate_ab;    // [n_in] per-node gate scores (a, b) (k_gcn_fwd_tc<0, true> only)
+  const float* gate_c;      // [1] gate bias or NULL
 };
 
 __device__ __forceinline__ int sw128_off(int r, int q) {   // bytes; 16-byte chunk q of row r, SWIZZLE_128B K-major
@@ -134,7 +136,9 @@ __device__ __forceinline__ void ft_tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
                : "r"(taddr));
 }
 
-template <int kMode>   // 0: tiles of the work order (rows + hub segments), 1: tiles of the hub list
+// kGate (mode 0): each gathered row j of row i weighted by edge_gate(a_j, b_i + c) — segments too, so the hub finish
+// (mode 1) sums gated partials unchanged
+template <int kMode, bool kGate = false>   // 0: tiles of the work order (rows + hub segments), 1: tiles of the hub list
 __global__ void __launch_bounds__(kFtThreads, 1) k_gcn_fwd_tc(const FwdTcArgs a) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -272,7 +276,13 @@ __global__ void __launch_bounds__(kFtThreads, 1) k_gcn_fwd_tc(const FwdTcArgs a)
       for (int q = 0; q < 8; ++q) acc.v[q] = 0.f;
       if (kMode == 0) {
         if (rowp >= 0) {
-          acc = gather_sum(a.z, a.nbr_w, pc.beg, pc.end, pc.gi, pc.gin, sub, grp_lane0, gmask, col, pol);
+          if constexpr (kGate) {
+            const float gc = a.gate_c ? __ldg(a.gate_c) : 0.f;
+            acc = gather_sum<false, true>(a.z, a.nbr_w, pc.beg, pc.end, pc.gi, pc.gin, sub, grp_lane0, gmask, col,
+                                          pol, a.gate_ab, __fadd_rn(__ldg(&a.gate_ab[rowp].y), gc));
+          } else {
+            acc = gather_sum(a.z, a.nbr_w, pc.beg, pc.end, pc.gi, pc.gin, sub, grp_lane0, gmask, col, pol);
+          }
           if (slot != 0) store_partial(a.partial, slot, col, acc);
         }
         // first round of the NEXT pass: its index batch was fetched before this gather and has arrived by now
@@ -444,6 +454,16 @@ extern "C" int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int
                                         const float* in_scale, const float* post, const float* out_scale,
                                         const uint32_t* keep, float keep_scale, int act_out, int64_t H, float* z_next,
                                         uint32_t* hmask, void* workspace, size_t* workspace_bytes, void* stream) {
+  return mgcn_gcn_layer_fwd_tc_gate(g, z, n_in, w, res_w, res_b, bias, in_scale, post, out_scale, keep, keep_scale,
+                                    nullptr, nullptr, act_out, H, z_next, hmask, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mgcn_gcn_layer_fwd_tc_gate(const mgcn_csr_t* g, const float* z, int64_t n_in, const float* w,
+                                          const float* res_w, const float* res_b, const float* bias,
+                                          const float* in_scale, const float* post, const float* out_scale,
+                                          const uint32_t* keep, float keep_scale, const float* gate_ab,
+                                          const float* gate_c, int act_out, int64_t H, float* z_next, uint32_t* hmask,
+                                          void* workspace, size_t* workspace_bytes, void* stream) {
   MGCN_REQUIRE(workspace_bytes != nullptr && g != nullptr, MGCN_ERR_NULL);
   MGCN_REQUIRE(H == kGH, MGCN_ERR_SHAPE);
   MGCN_REQUIRE(act_out == 0 || act_out == 1, MGCN_ERR_SHAPE);
@@ -460,6 +480,7 @@ extern "C" int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int
   MGCN_REQUIRE(z && w && res_w && z_next && hmask && g->rowptr && g->tasks, MGCN_ERR_NULL);
   MGCN_REQUIRE(g->nnz_cap == 0 || g->nbr_w, MGCN_ERR_NULL);
   MGCN_REQUIRE((reinterpret_cast<uintptr_t>(z) & 31u) == 0, MGCN_ERR_ALIGN);   // 256-bit row gathers
+  MGCN_REQUIRE((reinterpret_cast<uintptr_t>(gate_ab) & 7u) == 0, MGCN_ERR_ALIGN);
   MGCN_REQUIRE(aligned16(g->tasks) && aligned16(z_next) && aligned16(partial), MGCN_ERR_ALIGN);
   FwdTcArgs a{};
   a.tasks = reinterpret_cast<const int4*>(g->tasks);
@@ -473,6 +494,7 @@ extern "C" int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int
   a.z = z; a.w = w; a.res_w = res_w; a.res_b = res_b; a.bias = bias;
   a.in_scale = in_scale; a.post = post; a.out_scale = out_scale;
   a.keep = keep; a.keep_scale = keep_scale;
+  a.gate_ab = reinterpret_cast<const float2*>(gate_ab); a.gate_c = gate_c;
   a.z_next = z_next; a.hmask = hmask; a.partial = partial;
   a.n_rows = g->n_rows;
   a.seg_cap = hubs ? g->seg_cap : 0;
@@ -484,7 +506,13 @@ extern "C" int mgcn_gcn_layer_fwd_tc_ex(const mgcn_csr_t* g, const float* z, int
   MGCN_CHECK_CUDA(cudaFuncSetAttribute(k_gcn_fwd_tc<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFtSmem));
   MGCN_CHECK_CUDA(cudaFuncSetAttribute(k_gcn_fwd_tc<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFtSmem));
   int64_t tiles = ceil_div(a.n_rows + a.seg_cap, kFtRows);
-  MGCN_LAUNCH(k_gcn_fwd_tc<0>, (unsigned)(tiles < sms ? tiles : sms), kFtThreads, kFtSmem, stream, a);
+  if (gate_ab) {
+    void (*gated)(const FwdTcArgs) = k_gcn_fwd_tc<0, true>;
+    MGCN_CHECK_CUDA(cudaFuncSetAttribute(gated, cudaFuncAttributeMaxDynamicSharedMemorySize, kFtSmem));
+    MGCN_LAUNCH(gated, (unsigned)(tiles < sms ? tiles : sms), kFtThreads, kFtSmem, stream, a);
+  } else {
+    MGCN_LAUNCH(k_gcn_fwd_tc<0>, (unsigned)(tiles < sms ? tiles : sms), kFtThreads, kFtSmem, stream, a);
+  }
   if (hubs) {
     tiles = ceil_div(a.hub_cap, kFtRows);
     MGCN_LAUNCH(k_gcn_fwd_tc<1>, (unsigned)(tiles < sms ? tiles : sms), kFtThreads, kFtSmem, stream, a);

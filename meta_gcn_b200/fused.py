@@ -201,14 +201,22 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
     per row.  Backward: dW_n = x_n^T (A_hat^T ga), dx = (A_hat^T ga) W_n^T + gy R_n — the transposed aggregation of
     the masked gradient, then the row-local tcgen05 launch.  Parameters per layer: (W, [b], R, r); the bias adds
     before the ReLU in the layer kernels, and its gradient is the column sum of gy under the layer's mask word times
-    the dropout scale (post does not enter it)."""
+    the dropout scale (post does not enter it).  With edge gates (EdgeGateProj) the parameters per layer are
+    (W, [b], u, v, c, R, r): every gathered row is weighted by sigmoid(a_j + b_i + c) formed from per-node scores
+    (csrc/gate.cu), and the backward adds the gate's two passes (by target, by source) before the row-local launch."""
 
     @staticmethod
     def forward(ctx, x, graph, pre, post, has_bias, last_relu, p, *params):
-        per = 4 if has_bias else 3
+        return _ResidualGCNStack32AT._forward(ctx, x, graph, pre, post, has_bias, last_relu, p, False, *params)
+
+    @staticmethod
+    def _forward(ctx, x, graph, pre, post, has_bias, last_relu, p, gated, *params):
+        per = (4 if has_bias else 3) + (3 if gated else 0)
         L = len(params) // per
         layers = [params[i * per:(i + 1) * per] for i in range(L)]
         bias = (lambda n: layers[n][1]) if has_bias else (lambda n: None)
+        hb = 1 if has_bias else 0
+        gate = (lambda n: layers[n][1 + hb:4 + hb]) if gated else (lambda n: None)   # (u [1,32], v [1,32], c [1])
         fwd = graph.fwd_plain
         x0 = x.contiguous()
         sigma = None
@@ -217,12 +225,17 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         # dropout: applied in the layer kernels' epilogues, the dropped entries cleared in the ReLU mask words
         keep, scale = _dropout_masks(x0, L, 1, p)
         drop = (lambda n: {"keep": keep[n], "keep_scale": scale}) if keep is not None else (lambda n: {})
-        zs, hmasks = [], []
+        zs, hmasks, abs_ = [], [], []
         agg_first = x0.size(1) <= 4
         s0 = None
         if agg_first:
             xs0 = x0 * pre.unsqueeze(1) if pre is not None else x0            # pre_j x_j, one rounding as in the gather
-            s0 = ops.spmm_impl(fwd, xs0)                                      # [N, H_in]
+            if gated:
+                u, v, c = gate(0)
+                abs_.append(ops.gate_scores_impl(x0, layers[0][0], u, v))
+                s0 = ops.gate_spmm_narrow_impl(fwd, xs0, abs_[0], c)          # [N, H_in]
+            else:
+                s0 = ops.spmm_impl(fwd, xs0)                                  # [N, H_in]
             z, _, hm = ops.gcn_first_layer_fwd_impl(
                 s0, x0, layers[0][0], layers[0][-2], layers[0][-1], None, None, post,
                 1 if (last_relu or L > 1) else 0, out_scale=sigma if L > 1 else None, bias=bias(0), **drop(0))
@@ -234,12 +247,18 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             first = 0
         for n in range(first, L):
             zs.append(z)
+            gk = {}
+            if gated:
+                u, v, c = gate(n)
+                abs_.append(ops.gate_scores_impl(z, layers[n][0], u, v, sigma))
+                gk = {"gate_ab": abs_[-1], "gate_c": c}
             z, hm = ops.gcn_layer_fwd_tc_impl(
                 fwd, z, layers[n][0], layers[n][-2], layers[n][-1], bias(n), sigma, post,
-                sigma if n < L - 1 else None, 1 if (last_relu or n < L - 1) else 0, **drop(n))
+                sigma if n < L - 1 else None, 1 if (last_relu or n < L - 1) else 0, **drop(n), **gk)
             hmasks.append(hm)
         ctx.agg_first = agg_first
-        ctx.graph, ctx.cfg = graph, (L, per, has_bias, last_relu)
+        ctx.abs = abs_
+        ctx.graph, ctx.cfg = graph, (L, per, has_bias, last_relu, gated)
         ctx.bias_scale = 1.0 if scale is None else scale
         # the backward reads `post` only where it scales a gradient by the mask words: the dropout scale goes there
         ctx.save_for_backward(x0, s0, pre, _scaled_post(post, scale, x0.size(0), x0), sigma, z if last_relu else None,
@@ -248,7 +267,7 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        L, per, has_bias, last_relu = ctx.cfg
+        L, per, has_bias, last_relu, gated = ctx.cfg
         saved = ctx.saved_tensors
         x0, s0, pre, post, sigma, out = saved[:6]
         nz = L - 1 if ctx.agg_first else L
@@ -258,8 +277,25 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         hmasks = saved[6 + nz:6 + nz + L]
         params = saved[6 + nz + L:]
         layers = [params[i * per:(i + 1) * per] for i in range(L)]
-        bwd = ctx.graph.bwd_plain
+        fwd, bwd = ctx.graph.fwd_plain, ctx.graph.bwd_plain
         grads = [None] * len(params)
+        hb = 1 if has_bias else 0
+
+        def gate_backward(n, m, gs, xw=None):
+            """dxw of layer n with its gate (m = the layer's messages before their gates, z W); the gate's gradients
+            into grads: [du | dv] = (x W)^T d(a, b), dc = sum db (one fixed-order reduction).  x W = m / sigma for the
+            stored z (a row with pre = 0 has sigma = 1 and z = x there); xw: x W given directly (the narrow first layer,
+            whose m = pre (.) x W is 0 on such a row while its db is not)"""
+            u, v, c = layers[n][1 + hb:4 + hb]
+            ab = ctx.abs[n]
+            db = ops.gate_grad_by_target_impl(fwd, gs, m, ab, c)
+            dxw, dsc = ops.gate_grad_by_source_impl(bwd, gs, m, ab, c, db, pre, u, v, sigma if xw is None else None)
+            dg, dgb = ops.linear_wgrad_impl(m if xw is None else xw, dsc, False, True)
+            grads[per * n + 1 + hb] = dg[:, 0].reshape(u.shape)
+            grads[per * n + 2 + hb] = dg[:, 1].reshape(v.shape)
+            grads[per * n + 3 + hb] = dgb[2:3].reshape(c.shape)
+            return dxw
+
         gy = g.contiguous()
         if last_relu:
             gy = ops.relu_backward_impl(gy, out)
@@ -268,7 +304,19 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
         for n in range(L - 1, last - 1, -1):
             want_prev = n > 0
             w, res_w = layers[n][0], layers[n][-2]
-            if has_bias:
+            if gated:
+                # the gate's passes form dxw; the row-local launch takes it as the transposed aggregation's
+                dxw = gate_backward(n, ops.linear_impl(zs[n], w, False), gs)
+                if has_bias:
+                    gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
+                        dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, hmasks[n], post,
+                        ctx.bias_scale, want_prev, x_scale=sigma)
+                    grads[per * n + 1] = db
+                else:
+                    gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_impl(
+                        dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
+                        want_prev, True, x_scale=sigma)
+            elif has_bias:
                 # the one-launch backward (BWD_FUSED) has no bias gradient: a model with bias takes the two launches
                 dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
                 gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
@@ -289,27 +337,51 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
                 gy, gs = gy_prev, gs_prev
         if ctx.agg_first:
             grads[per - 2], grads[per - 1] = ops.linear_wgrad_impl(x0, gy, True, True)
-            grads[0] = ops.linear_wgrad_impl(s0, gs, False, False)[0]    # dW0 = s0^T gs0
+            if gated:
+                # W0 enters the scores too: dW0 = x0^T dxw0 with dxw0 = d / d(x0 W0), messages and scores together
+                xw0 = ops.linear_impl(x0, layers[0][0], False)
+                m0 = ops.linear_impl(x0, layers[0][0], False, row_scale=pre) if pre is not None else xw0
+                dxw = gate_backward(0, m0, gs, xw=xw0)
+                grads[0] = ops.linear_wgrad_impl(x0, dxw, False, False)[0]
+            else:
+                grads[0] = ops.linear_wgrad_impl(s0, gs, False, False)[0]    # dW0 = s0^T gs0
             if has_bias:
                 # no row-local launch for layer 0: its bias gradient is a pass of its own
                 grads[1] = ops.mask_bits_colsum_impl(gy, hmasks[0], ctx.bias_scale)
         return (None, None, None, None, None, None, None, *grads)
 
 
+class _GatedResidualGCNStack32AT(torch.autograd.Function):
+    """_ResidualGCNStack32AT with EdgeGateProj on every layer: parameters per layer (W, [b], u, v, c, R, r)"""
+
+    @staticmethod
+    def forward(ctx, x, graph, pre, post, has_bias, last_relu, p, *params):
+        return _ResidualGCNStack32AT._forward(ctx, x, graph, pre, post, has_bias, last_relu, p, True, *params)
+
+    @staticmethod
+    def backward(ctx, g):
+        return _ResidualGCNStack32AT.backward(ctx, g)
+
+
 def residual_gcn_stack(x, graph, pre, post, layer_params, has_bias, last_relu=False, aggregate_first=True,
-                       dropout=0.0):
+                       dropout=0.0, gated=False):
     """layer_params: per layer (weight_node [Hin,H], [bias [H]], residual.weight [H,Hin],
-    residual.bias [H]).  pre/post: per-source / per-target degree factors (either may be None).
-    dropout: p of nn.Dropout on every layer's node-model output (0 <= p < 1; pass 0 outside training).
-    Returns None where the stack does not take dropout (the round-1 hidden-32 kernels, chosen for an x that requires
-    grad or a degree with zeros): the caller then composes the layers one by one."""
+    residual.bias [H]); with gated, (weight_node, [bias], linsrc.weight [1,H], lintgt.weight [1,H], gate bias [1],
+    residual.weight, residual.bias): EdgeGateProj on every layer.  pre/post: per-source / per-target degree factors
+    (either may be None).  dropout: p of nn.Dropout on every layer's node-model output (0 <= p < 1; pass 0 outside
+    training).  Returns None where the stack does not take dropout (the round-1 hidden-32 kernels, chosen for an x
+    that requires grad or a degree with zeros) or gates (anything but the hidden-32 aggregate-then-transform stack):
+    the caller then composes the layers one by one."""
     if not 0.0 <= dropout < 1.0:
         raise ValueError(f"dropout must be in [0, 1), got {dropout}")
     flat = [p for lp in layer_params for p in lp]
     widths = {lp[0].size(1) for lp in layer_params} | {lp[0].size(0) for lp in layer_params[1:]}
     if widths == {32} and FORWARD_AGGREGATE_FIRST and aggregate_first and not x.requires_grad and \
             (x.size(1) <= 4 or x.size(1) == 32):
-        return _ResidualGCNStack32AT.apply(x, graph, pre, post, has_bias, last_relu, dropout, *flat)
+        stack = _GatedResidualGCNStack32AT if gated else _ResidualGCNStack32AT
+        return stack.apply(x, graph, pre, post, has_bias, last_relu, dropout, *flat)
+    if gated:
+        return None
     if not has_bias and widths == {32}:
         if dropout > 0:
             return None

@@ -17,6 +17,15 @@ from .gcn_base_models import NodeModelBase
 from .gcn_multi_kernel import GCNMultiKernel
 
 
+def _stack_gate(nm):
+    """edge gate of a node model as the residual stack sees it: None (no gate), True (EdgeGateProj on node scores only,
+    with its bias: the stack's gated kernels) or False (any other gate: the per-layer path)"""
+    eg = nm.edge_gate
+    if eg is None:
+        return None
+    return type(eg).__name__ == "EdgeGateProj" and eg.in_edgedim is None and eg.bias is not None
+
+
 class GCNLayer(nn.Module):
     def __init__(self, in_channels, out_channels, in_edgedim=None, deg_norm="sm", edge_gate=None,
                  aggr="add", bias=True, num_kernel=1, nodemodel="additive", non_linear="relu", **kwargs):
@@ -127,8 +136,9 @@ class GCNModel(nn.Module):
         if any(len(m) != 1 or layer.gcn.kernel_combine != "add" for m, layer in zip(nms, self.gcn_net)):
             return False
         first = nms[0][0]
-        return all(type(m[0]).__name__ == "NodeModelAdditive" and m[0].aggr == "add" and m[0].edge_gate is None and m[0].deg_norm == first.deg_norm and m[0].in_edgedim is None
-                   and (m[0].bias is None) == (first.bias is None) for m in nms)
+        return all(type(m[0]).__name__ == "NodeModelAdditive" and m[0].aggr == "add" and m[0].deg_norm == first.deg_norm and m[0].in_edgedim is None
+                   and (m[0].bias is None) == (first.bias is None)
+                   and _stack_gate(m[0]) is not False and _stack_gate(m[0]) == _stack_gate(first) for m in nms)
 
     def _forward_stack(self, x, edge_index, dis, deg=None):
         nm0 = self.gcn_net[0].gcn.node_models[0]
@@ -141,14 +151,16 @@ class GCNModel(nn.Module):
         pre = dis
         post = dis if nm0.deg_norm == "sm" else None
         has_bias = nm0.bias is not None
+        gated = _stack_gate(nm0) is True
         params = []
         for layer, lin in zip(self.gcn_net, self.residuals):
             nm = layer.gcn.node_models[0]
-            params.append((nm.weight_node, nm.bias, lin.weight, lin.bias) if has_bias
-                          else (nm.weight_node, lin.weight, lin.bias))
-        # None: the stack chosen for these inputs does not take dropout (fused.residual_gcn_stack)
+            eg = nm.edge_gate
+            params.append((nm.weight_node,) + ((nm.bias,) if has_bias else ())
+                          + ((eg.linsrc.weight, eg.lintgt.weight, eg.bias) if gated else ()) + (lin.weight, lin.bias))
+        # None: the stack chosen for these inputs does not take dropout or gates (fused.residual_gcn_stack)
         return fused.residual_gcn_stack(x, graph, pre, post, params, has_bias, aggregate_first=aggregate_first,
-                                        dropout=self.dropout.p if self.training else 0.0)
+                                        dropout=self.dropout.p if self.training else 0.0, gated=gated)
 
     def forward(self, x, edge_index_K, edge_attr_K=None, deg_K=None, edge_weight_K=None, **kwargs):
         hidden = kwargs.pop("_hidden", False)        # forward_loss: stop before the output layer

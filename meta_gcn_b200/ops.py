@@ -542,15 +542,16 @@ FWD_TMEM_OPERANDS = False
 
 
 def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, tmem_operands=None,
-                          keep=None, keep_scale=1.0):
+                          keep=None, keep_scale=1.0, gate_ab=None, gate_c=None):
     """one aggregate-then-transform forward layer at hidden 32 on tcgen05 (mgcn_gcn_layer_fwd_tc_ex): z = in_scale (.) x
     [N,32]; returns (z_next = out_scale (.) x_next [N,32], hmask int32[N]).  keep int32 [N]: dropout keep bits of the
-    layer (kept entries of h multiplied by keep_scale, dropped ones cleared in hmask too)"""
-    _need_cuda(z, w, res_w, res_b, bias, in_scale, post, out_scale, keep)
+    layer (kept entries of h multiplied by keep_scale, dropped ones cleared in hmask too).  gate_ab [N,2] (from
+    gate_scores_impl) and gate_c [1]: every gathered row weighted by its edge gate (mgcn_gcn_layer_fwd_tc_gate)"""
+    _need_cuda(z, w, res_w, res_b, bias, in_scale, post, out_scale, keep, gate_ab, gate_c)
     tmem = FWD_TMEM_OPERANDS if tmem_operands is None else tmem_operands
-    if keep is not None and tmem:
-        raise ValueError("dropout keep bits need the shared-memory operand forward (mgcn_gcn_layer_fwd_tc_ex), "
-                         "not the TMEM-operand kernel")
+    if (keep is not None or gate_ab is not None) and tmem:
+        raise ValueError("dropout keep bits and edge gates need the shared-memory operand forward "
+                         "(mgcn_gcn_layer_fwd_tc_gate), not the TMEM-operand kernel")
     z = _f32c(z, "z")
     w = _f32c(w, "w")
     res_w = _f32c(res_w, "res_w")
@@ -571,12 +572,93 @@ def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_sca
     tail = (int(act_out), H, _ptr(z_next), _ptr(hmask))
     if tmem:
         fn, args = lib.mgcn_gcn_layer_fwd_tm, lead + tail
+    elif gate_ab is not None:
+        keep = _keep_rows(keep, n_rows, 1)
+        gate_ab, gate_c = _gate_operands(gate_ab, gate_c, z.size(0))
+        fn, args = lib.mgcn_gcn_layer_fwd_tc_gate, lead + (_ptr(keep), float(keep_scale), _ptr(gate_ab),
+                                                          _ptr(gate_c)) + tail
     else:
         keep = _keep_rows(keep, n_rows, 1)
         fn, args = lib.mgcn_gcn_layer_fwd_tc_ex, lead + (_ptr(keep), float(keep_scale)) + tail
     ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
     _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
     return z_next, hmask
+
+
+def _gate_operands(ab, c, n):
+    ab = _f32c(ab, "gate_ab")
+    c = _f32c(c, "gate_c")
+    if tuple(ab.shape) != (n, 2):
+        raise ValueError(f"gate_ab must be [{n}, 2], got {tuple(ab.shape)}")
+    if c is not None and c.numel() != 1:
+        raise ValueError("gate_c must have one entry")
+    return ab, c
+
+
+def gate_scores_impl(x, w, u, v, in_scale=None):
+    """per-node gate scores (mgcn_gate_scores): [N,2] = ((x w) . u, (x w) . v) / in_scale for x [N,H<=32] (x = the
+    stored z = in_scale (.) x of the stack), w [H,32], u / v with 32 entries"""
+    _need_cuda(x, w, u, v, in_scale)
+    x = _f32c(x, "x")
+    w = _f32c(w, "w")
+    u = _f32c(u, "u")
+    v = _f32c(v, "v")
+    in_scale = _f32c(in_scale, "in_scale")
+    N, H = x.shape
+    if tuple(w.shape) != (H, 32) or u.numel() != 32 or v.numel() != 32:
+        raise ValueError("gate_scores needs w [H,32] and u, v with 32 entries")
+    ab = torch.empty(N, 2, dtype=torch.float32, device=x.device)
+    _lib.check(_lib.load().mgcn_gate_scores(_ptr(x), N, H, _ptr(in_scale), _ptr(w), _ptr(u), _ptr(v), _ptr(ab),
+                                            _stream()))
+    return ab
+
+
+def gate_spmm_narrow_impl(csr, x, ab, c):
+    """out_i = sum_{j -> i} gate_ij x_j for x [n_in, H<=4] (mgcn_gate_spmm_narrow)"""
+    _need_cuda(csr.rowptr, x, ab, c)
+    x = _f32c(x, "x")
+    ab, c = _gate_operands(ab, c, x.size(0))
+    out = torch.empty(csr.n_rows, x.size(1), dtype=torch.float32, device=x.device)
+    _lib.check(_lib.load().mgcn_gate_spmm_narrow(ctypes.byref(csr.struct()), _ptr(x), x.size(0), x.size(1), _ptr(ab),
+                                                 _ptr(c), _ptr(out), _stream()))
+    return out
+
+
+def gate_grad_by_target_impl(csr, gs, m, ab, c):
+    """db [N]: db_i = sum_{j -> i} <gs_i, m_j> g_ij (1 - g_ij) over the forward structure (mgcn_gate_grad_by_target)"""
+    _need_cuda(csr.rowptr, gs, m, ab, c)
+    gs = _f32c(gs, "gs")
+    m = _f32c(m, "m")
+    ab, c = _gate_operands(ab, c, m.size(0))
+    db = torch.empty(csr.n_rows, dtype=torch.float32, device=gs.device)
+    lib = _lib.load()
+    args = (ctypes.byref(csr.struct()), _ptr(gs), _ptr(m), _ptr(ab), _ptr(c), _ptr(db))
+    ws, nbytes = _workspace(lambda w_, nb, stm: lib.mgcn_gate_grad_by_target(*args, w_, nb, stm), gs.device)
+    _lib.check(lib.mgcn_gate_grad_by_target(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
+    return db
+
+
+def gate_grad_by_source_impl(csr_t, gs, m, ab, c, db, pre, u, v, sigma):
+    """(dxw [N,32], dsc [N,3]) of mgcn_gate_grad_by_source: dxw_j = pre_j sum_i g_ij gs_i + da_j u + db_j v and
+    dsc_j = (da_j / sigma_j, db_j / sigma_j, db_j)"""
+    _need_cuda(csr_t.rowptr, gs, m, ab, c, db, pre, u, v, sigma)
+    gs = _f32c(gs, "gs")
+    m = _f32c(m, "m")
+    ab, c = _gate_operands(ab, c, m.size(0))
+    db = _f32c(db, "db")
+    pre = _f32c(pre, "pre")
+    u = _f32c(u, "u")
+    v = _f32c(v, "v")
+    sigma = _f32c(sigma, "sigma")
+    n = csr_t.n_rows
+    dxw = torch.empty(n, 32, dtype=torch.float32, device=gs.device)
+    dsc = torch.empty(n, 3, dtype=torch.float32, device=gs.device)
+    lib = _lib.load()
+    args = (ctypes.byref(csr_t.struct()), _ptr(gs), _ptr(m), _ptr(ab), _ptr(c), _ptr(db), _ptr(pre), _ptr(u), _ptr(v),
+            _ptr(sigma), _ptr(dxw), _ptr(dsc))
+    ws, nbytes = _workspace(lambda w_, nb, stm: lib.mgcn_gate_grad_by_source(*args, w_, nb, stm), gs.device)
+    _lib.check(lib.mgcn_gate_grad_by_source(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
+    return dxw, dsc
 
 
 def gcn_layer_bwd_impl(dxw, gy, x, w, res_w, hmask_prev, post, want_prev=True, tensor_memory=False, x_scale=None):
@@ -1065,6 +1147,15 @@ _LIBDEF.define("gcn_layer_bwd_bias(Tensor dxw, Tensor gy, Tensor x, Tensor w, Te
                "Tensor hmask_cur, Tensor? post, float bias_scale, bool want_prev, Tensor? x_scale) "
                "-> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)")
 _LIBDEF.define("mask_bits_colsum(Tensor gy, Tensor bits, float scale) -> Tensor")
+_LIBDEF.define("gate_scores(Tensor x, Tensor w, Tensor u, Tensor v, Tensor? in_scale) -> Tensor")
+_LIBDEF.define("gcn_layer_fwd_tc_gate(Tensor[] csr, int hub_threshold, Tensor z, Tensor w, Tensor res_w, Tensor? res_b, "
+               "Tensor? bias, Tensor? in_scale, Tensor? post, Tensor? out_scale, int act_out, Tensor? keep, "
+               "float keep_scale, Tensor gate_ab, Tensor? gate_c) -> (Tensor, Tensor)")
+_LIBDEF.define("gate_spmm_narrow(Tensor[] csr, int hub_threshold, Tensor x, Tensor ab, Tensor? c) -> Tensor")
+_LIBDEF.define("gate_grad_by_target(Tensor[] csr, int hub_threshold, Tensor gs, Tensor m, Tensor ab, Tensor? c) "
+               "-> Tensor")
+_LIBDEF.define("gate_grad_by_source(Tensor[] csr_t, int hub_threshold, Tensor gs, Tensor m, Tensor ab, Tensor? c, "
+               "Tensor db, Tensor? pre, Tensor u, Tensor v, Tensor? sigma) -> (Tensor, Tensor)")
 _LIBDEF.define("dropout_keep_bits(Tensor seed, int L, int N, int W, float p) -> Tensor")
 _LIBDEF.define("segment_max(Tensor[] csr, int hub_threshold, Tensor x, bool gather_perm, Tensor? edge_val) -> (Tensor, Tensor)")
 _LIBDEF.define("segment_max_bwd(Tensor[] csr_t, int hub_threshold, Tensor grad, Tensor arg, Tensor? edge_val) -> Tensor")
@@ -1122,7 +1213,20 @@ def _op_propagate(csr, csr_t, hub_threshold, x, nbr_scale, row_scale, act):
     return spmm_impl(_as_csr(csr, hub_threshold), x, False, None, nbr_scale, row_scale, 0, None, None, act)
 
 
+def _op_layer_fwd_tc_gate(csr, hub_threshold, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, keep,
+                          keep_scale, gate_ab, gate_c):
+    return gcn_layer_fwd_tc_impl(_as_csr(csr, hub_threshold), z, w, res_w, res_b, bias, in_scale, post, out_scale,
+                                 act_out, tmem_operands=False, keep=keep, keep_scale=keep_scale, gate_ab=gate_ab,
+                                 gate_c=gate_c)
+
+
 _IMPLS2 = {
+    "gate_scores": gate_scores_impl,
+    "gcn_layer_fwd_tc_gate": _op_layer_fwd_tc_gate,
+    "gate_spmm_narrow": lambda csr, ht, x, ab, c: gate_spmm_narrow_impl(_as_csr(csr, ht), x, ab, c),
+    "gate_grad_by_target": lambda csr, ht, gs, m, ab, c: gate_grad_by_target_impl(_as_csr(csr, ht), gs, m, ab, c),
+    "gate_grad_by_source": lambda csr_t, ht, gs, m, ab, c, db, pre, u, v, sigma: gate_grad_by_source_impl(
+        _as_csr(csr_t, ht), gs, m, ab, c, db, pre, u, v, sigma),
     "gcn_layer_fwd_tc": _op_layer_fwd_tc,
     "gcn_first_layer_fwd": _op_first_layer_fwd,
     "gcn_layer_bwd": _op_layer_bwd,
@@ -1198,6 +1302,36 @@ def _(dxw, gy, x, w, res_w, hmask_prev, hmask_cur, post, bias_scale, want_prev, 
 @torch.library.register_fake("mgcn::mask_bits_colsum")
 def _(gy, bits, scale):
     return torch.empty(gy.size(1), dtype=torch.float32, device=gy.device)
+
+
+@torch.library.register_fake("mgcn::gate_scores")
+def _(x, w, u, v, in_scale):
+    return torch.empty(x.size(0), 2, dtype=torch.float32, device=x.device)
+
+
+@torch.library.register_fake("mgcn::gcn_layer_fwd_tc_gate")
+def _(csr, hub_threshold, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, keep, keep_scale, gate_ab,
+      gate_c):
+    n = _rows_of(csr)
+    return (torch.empty(n, z.size(1), dtype=torch.float32, device=z.device),
+            torch.empty(n, dtype=torch.int32, device=z.device))
+
+
+@torch.library.register_fake("mgcn::gate_spmm_narrow")
+def _(csr, hub_threshold, x, ab, c):
+    return torch.empty(_rows_of(csr), x.size(1), dtype=torch.float32, device=x.device)
+
+
+@torch.library.register_fake("mgcn::gate_grad_by_target")
+def _(csr, hub_threshold, gs, m, ab, c):
+    return torch.empty(_rows_of(csr), dtype=torch.float32, device=gs.device)
+
+
+@torch.library.register_fake("mgcn::gate_grad_by_source")
+def _(csr_t, hub_threshold, gs, m, ab, c, db, pre, u, v, sigma):
+    n = _rows_of(csr_t)
+    return (torch.empty(n, 32, dtype=torch.float32, device=gs.device),
+            torch.empty(n, 3, dtype=torch.float32, device=gs.device))
 
 
 @torch.library.register_fake("mgcn::dropout_keep_bits")
