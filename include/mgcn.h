@@ -42,9 +42,19 @@ extern "C" {
 #define MGCN_ERR_WORKSPACE (-5) /* workspace smaller than the queried size            */
 
 /* Rows longer than this are "hubs": they are cut into segments of this many entries, each summed by
- * one lane group like an ordinary row, and the partial sums are combined left to right.  Rows at or
- * below it are summed by one lane group sequentially in edge_index order (bit-identical to the
- * reference's CPU scatter_add). */
+ * one lane group like an ordinary row (from 0, in row order).  Rows at or below it are summed by one
+ * lane group sequentially in edge_index order (bit-identical to the reference's CPU scatter_add).
+ * The ns segment sums p_0 .. p_{ns-1} of a hub are combined in one of two fixed orders:
+ *   left to right       ((p_0 + p_1) + p_2) + ...            mgcn_spmm; mgcn_aggregate_prescaled except below
+ *   runs                R_g = sum of p_{g*per} .. p_{min(ns, g*per+per)-1}, each from 0, left to right;
+ *                       then ((R_0 + R_1) + R_2) + ... over the non-empty runs, with
+ *                       per = ceil(ns/8) (8 runs) if ns <= 32, per = ceil(ns/64) (64 runs) if ns > 32
+ *                       — mgcn_aggregate_prescaled at H = 32 without mean / bias / residual on a 32-byte
+ *                       aligned x, and mgcn_gcn_layer_fwd
+ *   8 runs              the same with per = ceil(ns/8) for every ns — the tcgen05 hidden-32 layer kernels
+ *                       (mgcn_gcn_layer_fwd_tc*, mgcn_gcn_layer_fwd_tm, mgcn_gcn_layer_bwd_fused)
+ * Each is independent of the grid, the device and the order of the hub table, so results are identical
+ * from run to run and across devices; they give different bits for hubs of more than 2 segments. */
 #define MGCN_DEFAULT_HUB_THRESHOLD 64
 
 /* A row-owned adjacency (CSR when built by source, CSC when built by target).  All pointer members
@@ -210,8 +220,11 @@ int mgcn_spmm(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H, int 
 /* The same aggregation for inputs that already carry the per-source factor (x~ = nbr_scale * x,
  * written by the producing transform): no per-edge weight at all,
  *   out_i = act( post_scale[i] * sum_k x~[nbr[k], :] (/ len_i) + bias + residual_i ),
- * rows visited in g->order.  Same summation order as mgcn_spmm; differs from it only in where the
- * factors are rounded (x*(d_i d_j) vs (x d_j) summed, then * d_i).  H must be 16, 32, 64 or 128. */
+ * rows visited in g->order.  Same summation order as mgcn_spmm inside rows and hub segments; differs from it in
+ * where the factors are rounded (x*(d_i d_j) vs (x d_j) summed, then * d_i) and, at H = 32 without reduce / bias /
+ * residual on a 32-byte aligned x, in the combine order of hub segments ("runs", see MGCN_DEFAULT_HUB_THRESHOLD).
+ * Epilogue order: * post_scale, / max(len_i, 1), + bias, + residual, act.  H must be 16, 32, 64 or 128; x, out,
+ * bias and residual 16-byte aligned (else MGCN_ERR_ALIGN). */
 int mgcn_aggregate_prescaled(const mgcn_csr_t* g, const float* x, int64_t n_in, int64_t H,
                              const float* post_scale, int reduce, const float* bias,
                              const float* residual, int act, float* out, void* workspace,
@@ -277,7 +290,8 @@ int mgcn_relu_backward(const float* g, const float* y, int64_t count, float* g_i
  *            x_next = act_out ? relu(y) : y
  *            m_next = pre * (x_next w_next)       (w_next may be NULL: last layer)
  *            hmask[i] bit c = (h[i,c] > 0)
- * Sums run in edge_index order per row (hub rows: per segment, segments left to right); the dense
+ * Sums run in edge_index order per row (hub rows: per segment, segments combined in runs — see
+ * MGCN_DEFAULT_HUB_THRESHOLD); the dense
  * products run on the tensor pipe as 3xTF32 with separately accumulated correction terms.
  * Row-local mode, g == NULL: m[i] is the finished pre-activation of row i (n_in rows) — used for a first
  * layer of small input width, which is aggregated BEFORE its transform: (A_hat x) W instead of A_hat (x W).

@@ -159,70 +159,76 @@ __global__ void __launch_bounds__(256) k_hub_reduce(const int32_t* __restrict__ 
   __shared__ int n_giant;
   __shared__ __align__(16) float red[64][kH];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, sub = lane & 3, grp = lane >> 2, col = sub * 8;
-  if (threadIdx.x == 0) n_giant = 0;
-  __syncthreads();
   int64_t nh = *hub_count;
   if (nh > hub_cap) nh = hub_cap;
   const int64_t W = (int64_t)gridDim.x * 8;
-  for (int64_t k = (int64_t)blockIdx.x * 8 + warp; k < nh; k += W) {
-    const int64_t row = __ldg(hub_rows + k);
-    const int s0 = __ldg(hub_seg0 + k);
-    const int len = __ldg(rowptr + row + 1) - __ldg(rowptr + row);
-    const int ns = (len + hub_threshold - 1) / hub_threshold;
-    if (ns <= 1) continue;
-    if (ns > kGiantSegs) {   // queue for the CTA-wide pass below (the slot order never reaches the results)
-      int slot = 0;
-      if (lane == 0) slot = atomicAdd(&n_giant, 1);
-      slot = __shfl_sync(0xffffffffu, slot, 0);
-      if (slot < kGiantList) {
+  int64_t k = (int64_t)blockIdx.x * 8 + warp;
+  // rounds: a warp that finds the giant list full stops at that hub and resumes there after the list is drained, so
+  // every giant gets the 64-run grouping whatever the grid (and hence the device's SM count) and the hub table order
+  bool more = true;
+  while (more) {
+    if (threadIdx.x == 0) n_giant = 0;
+    __syncthreads();
+    for (; k < nh; k += W) {
+      const int64_t row = __ldg(hub_rows + k);
+      const int s0 = __ldg(hub_seg0 + k);
+      const int len = __ldg(rowptr + row + 1) - __ldg(rowptr + row);
+      const int ns = (len + hub_threshold - 1) / hub_threshold;
+      if (ns <= 1) continue;
+      if (ns > kGiantSegs) {   // queue for the CTA-wide pass below (the slot order never reaches the results)
+        int slot = 0;
+        if (lane == 0) slot = atomicAdd(&n_giant, 1);
+        slot = __shfl_sync(0xffffffffu, slot, 0);
+        if (slot >= kGiantList) break;   // list full: this hub waits for the next round
         if (lane == 0) giant_k[slot] = (int)k;
         continue;
       }
-    }
-    const int per = (ns + 7) >> 3;
-    const Row8 run = hub_run_sum(partial, s0, grp * per, min(ns, grp * per + per), col);
-    Row8 tot = run;   // group 0: its own run; then runs 1..7 in order
+      const int per = (ns + 7) >> 3;
+      const Row8 run = hub_run_sum(partial, s0, grp * per, min(ns, grp * per + per), col);
+      Row8 tot = run;   // group 0: its own run; then runs 1..7 in order
 #pragma unroll
-    for (int g = 1; g < 8; ++g) {
-      Row8 other;
+      for (int g = 1; g < 8; ++g) {
+        Row8 other;
 #pragma unroll
-      for (int q = 0; q < 8; ++q) other.v[q] = __shfl_sync(0xffffffffu, run.v[q], 4 * g + sub);
-      if (g * per < ns) row8_add(tot, other);
-    }
-    if (grp == 0) {
-      float* o = partial + (int64_t)s0 * kH + col;
-      *reinterpret_cast<float4*>(o) = make_float4(tot.v[0], tot.v[1], tot.v[2], tot.v[3]);
-      *reinterpret_cast<float4*>(o + 4) = make_float4(tot.v[4], tot.v[5], tot.v[6], tot.v[7]);
-    }
-  }
-  __syncthreads();
-  // giants: 64 lane groups of the CTA sum 64 contiguous runs concurrently, group 0 adds the 64 run sums in order
-  const int ng = min(n_giant, kGiantList);
-  for (int gi = 0; gi < ng; ++gi) {
-    const int64_t k = giant_k[gi];
-    const int64_t row = __ldg(hub_rows + k);
-    const int s0 = __ldg(hub_seg0 + k);
-    const int len = __ldg(rowptr + row + 1) - __ldg(rowptr + row);
-    const int ns = (len + hub_threshold - 1) / hub_threshold;
-    const int per = (ns + 63) >> 6, gid = warp * 8 + grp;
-    const Row8 run = hub_run_sum(partial, s0, gid * per, min(ns, gid * per + per), col);
-    *reinterpret_cast<float4*>(&red[gid][col]) = make_float4(run.v[0], run.v[1], run.v[2], run.v[3]);
-    *reinterpret_cast<float4*>(&red[gid][col + 4]) = make_float4(run.v[4], run.v[5], run.v[6], run.v[7]);
-    __syncthreads();   // also: every read of the hub's first slot (run 0) has completed
-    if (warp == 0 && grp == 0) {
-      Row8 tot = run;
-      for (int g = 1; g < 64 && g * per < ns; ++g) {
-        const float4 lo = *reinterpret_cast<const float4*>(&red[g][col]), hi = *reinterpret_cast<const float4*>(&red[g][col + 4]);
-        Row8 o;
-        o.v[0] = lo.x; o.v[1] = lo.y; o.v[2] = lo.z; o.v[3] = lo.w;
-        o.v[4] = hi.x; o.v[5] = hi.y; o.v[6] = hi.z; o.v[7] = hi.w;
-        row8_add(tot, o);
+        for (int q = 0; q < 8; ++q) other.v[q] = __shfl_sync(0xffffffffu, run.v[q], 4 * g + sub);
+        if (g * per < ns) row8_add(tot, other);
       }
-      float* o = partial + (int64_t)s0 * kH + col;
-      *reinterpret_cast<float4*>(o) = make_float4(tot.v[0], tot.v[1], tot.v[2], tot.v[3]);
-      *reinterpret_cast<float4*>(o + 4) = make_float4(tot.v[4], tot.v[5], tot.v[6], tot.v[7]);
+      if (grp == 0) {
+        float* o = partial + (int64_t)s0 * kH + col;
+        *reinterpret_cast<float4*>(o) = make_float4(tot.v[0], tot.v[1], tot.v[2], tot.v[3]);
+        *reinterpret_cast<float4*>(o + 4) = make_float4(tot.v[4], tot.v[5], tot.v[6], tot.v[7]);
+      }
     }
     __syncthreads();
+    // giants: 64 lane groups of the CTA sum 64 contiguous runs concurrently, group 0 adds the 64 run sums in order
+    const int ng = min(n_giant, kGiantList);
+    for (int gi = 0; gi < ng; ++gi) {
+      const int64_t k = giant_k[gi];
+      const int64_t row = __ldg(hub_rows + k);
+      const int s0 = __ldg(hub_seg0 + k);
+      const int len = __ldg(rowptr + row + 1) - __ldg(rowptr + row);
+      const int ns = (len + hub_threshold - 1) / hub_threshold;
+      const int per = (ns + 63) >> 6, gid = warp * 8 + grp;
+      const Row8 run = hub_run_sum(partial, s0, gid * per, min(ns, gid * per + per), col);
+      *reinterpret_cast<float4*>(&red[gid][col]) = make_float4(run.v[0], run.v[1], run.v[2], run.v[3]);
+      *reinterpret_cast<float4*>(&red[gid][col + 4]) = make_float4(run.v[4], run.v[5], run.v[6], run.v[7]);
+      __syncthreads();   // also: every read of the hub's first slot (run 0) has completed
+      if (warp == 0 && grp == 0) {
+        Row8 tot = run;
+        for (int g = 1; g < 64 && g * per < ns; ++g) {
+          const float4 lo = *reinterpret_cast<const float4*>(&red[g][col]), hi = *reinterpret_cast<const float4*>(&red[g][col + 4]);
+          Row8 o;
+          o.v[0] = lo.x; o.v[1] = lo.y; o.v[2] = lo.z; o.v[3] = lo.w;
+          o.v[4] = hi.x; o.v[5] = hi.y; o.v[6] = hi.z; o.v[7] = hi.w;
+          row8_add(tot, o);
+        }
+        float* o = partial + (int64_t)s0 * kH + col;
+        *reinterpret_cast<float4*>(o) = make_float4(tot.v[0], tot.v[1], tot.v[2], tot.v[3]);
+        *reinterpret_cast<float4*>(o + 4) = make_float4(tot.v[4], tot.v[5], tot.v[6], tot.v[7]);
+      }
+      __syncthreads();
+    }
+    more = __syncthreads_or(k < nh) != 0;   // also: n_giant is read above by every thread before it is reset
   }
 }
 
@@ -684,69 +690,74 @@ __global__ void __launch_bounds__(256) k_agg_flat_hub_finish(const AggFlatArgs a
   __shared__ int n_giant;
   __shared__ __align__(16) float red[64][kH];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, sub = lane & 3, grp = lane >> 2, col = sub * 8;
-  if (threadIdx.x == 0) n_giant = 0;
-  __syncthreads();
   int64_t nh = *a.hub_count;
   if (nh > a.hub_cap) nh = a.hub_cap;
   const uint64_t pol = policy_evict_first();
   const int64_t W = (int64_t)gridDim.x * 8;
-  for (int64_t k = (int64_t)blockIdx.x * 8 + warp; k < nh; k += W) {
-    const int64_t row = __ldg(a.hub_rows + k);
-    const int s0 = __ldg(a.hub_seg0 + k);
-    const int len = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
-    const int ns = (len + a.hub_threshold - 1) / a.hub_threshold;
-    if (ns > kGiantSegs) {   // queue for the CTA-wide pass below (the slot order never reaches the results)
-      int slot = 0;
-      if (lane == 0) slot = atomicAdd(&n_giant, 1);
-      slot = __shfl_sync(0xffffffffu, slot, 0);
-      if (slot < kGiantList) {
+  int64_t k = (int64_t)blockIdx.x * 8 + warp;
+  // rounds, as in k_hub_reduce: every giant gets the 64-run grouping whatever the grid and the hub table order
+  bool more = true;
+  while (more) {
+    if (threadIdx.x == 0) n_giant = 0;
+    __syncthreads();
+    for (; k < nh; k += W) {
+      const int64_t row = __ldg(a.hub_rows + k);
+      const int s0 = __ldg(a.hub_seg0 + k);
+      const int len = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
+      const int ns = (len + a.hub_threshold - 1) / a.hub_threshold;
+      if (ns > kGiantSegs) {   // queue for the CTA-wide pass below (the slot order never reaches the results)
+        int slot = 0;
+        if (lane == 0) slot = atomicAdd(&n_giant, 1);
+        slot = __shfl_sync(0xffffffffu, slot, 0);
+        if (slot >= kGiantList) break;   // list full: this hub waits for the next round
         if (lane == 0) giant_k[slot] = (int)k;
         continue;
       }
-    }
-    Row8 tot;
-    if (ns <= 1) {
-      tot = sum_partials(a.partial, s0, 1, col);
-    } else {
-      const int per = (ns + 7) >> 3;
-      const Row8 run = hub_run_sum(a.partial, s0, grp * per, min(ns, grp * per + per), col);
-      tot = run;   // group 0: its own run; then runs 1..7 in order
+      Row8 tot;
+      if (ns <= 1) {
+        tot = sum_partials(a.partial, s0, 1, col);
+      } else {
+        const int per = (ns + 7) >> 3;
+        const Row8 run = hub_run_sum(a.partial, s0, grp * per, min(ns, grp * per + per), col);
+        tot = run;   // group 0: its own run; then runs 1..7 in order
 #pragma unroll
-      for (int g = 1; g < 8; ++g) {
-        Row8 other;
+        for (int g = 1; g < 8; ++g) {
+          Row8 other;
 #pragma unroll
-        for (int q = 0; q < 8; ++q) other.v[q] = __shfl_sync(0xffffffffu, run.v[q], 4 * g + sub);
-        if (g * per < ns) row8_add(tot, other);
+          for (int q = 0; q < 8; ++q) other.v[q] = __shfl_sync(0xffffffffu, run.v[q], 4 * g + sub);
+          if (g * per < ns) row8_add(tot, other);
+        }
       }
-    }
-    if (grp == 0) agg_finish_row(a, tot, a.post ? __ldg(a.post + row) : 1.f, row, col, pol);
-  }
-  __syncthreads();
-  // giants: 64 lane groups of the CTA sum 64 contiguous runs concurrently, group 0 adds the 64 run sums in order
-  const int ng = min(n_giant, kGiantList);
-  for (int gi = 0; gi < ng; ++gi) {
-    const int64_t k = giant_k[gi];
-    const int64_t row = __ldg(a.hub_rows + k);
-    const int s0 = __ldg(a.hub_seg0 + k);
-    const int len = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
-    const int ns = (len + a.hub_threshold - 1) / a.hub_threshold;
-    const int per = (ns + 63) >> 6, gid = warp * 8 + grp;
-    const Row8 run = hub_run_sum(a.partial, s0, gid * per, min(ns, gid * per + per), col);
-    *reinterpret_cast<float4*>(&red[gid][col]) = make_float4(run.v[0], run.v[1], run.v[2], run.v[3]);
-    *reinterpret_cast<float4*>(&red[gid][col + 4]) = make_float4(run.v[4], run.v[5], run.v[6], run.v[7]);
-    __syncthreads();
-    if (warp == 0 && grp == 0) {
-      Row8 tot = run;
-      for (int g = 1; g < 64 && g * per < ns; ++g) {
-        const float4 lo = *reinterpret_cast<const float4*>(&red[g][col]), hi = *reinterpret_cast<const float4*>(&red[g][col + 4]);
-        Row8 o;
-        o.v[0] = lo.x; o.v[1] = lo.y; o.v[2] = lo.z; o.v[3] = lo.w;
-        o.v[4] = hi.x; o.v[5] = hi.y; o.v[6] = hi.z; o.v[7] = hi.w;
-        row8_add(tot, o);
-      }
-      agg_finish_row(a, tot, a.post ? __ldg(a.post + row) : 1.f, row, col, pol);
+      if (grp == 0) agg_finish_row(a, tot, a.post ? __ldg(a.post + row) : 1.f, row, col, pol);
     }
     __syncthreads();
+    // giants: 64 lane groups of the CTA sum 64 contiguous runs concurrently, group 0 adds the 64 run sums in order
+    const int ng = min(n_giant, kGiantList);
+    for (int gi = 0; gi < ng; ++gi) {
+      const int64_t k = giant_k[gi];
+      const int64_t row = __ldg(a.hub_rows + k);
+      const int s0 = __ldg(a.hub_seg0 + k);
+      const int len = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
+      const int ns = (len + a.hub_threshold - 1) / a.hub_threshold;
+      const int per = (ns + 63) >> 6, gid = warp * 8 + grp;
+      const Row8 run = hub_run_sum(a.partial, s0, gid * per, min(ns, gid * per + per), col);
+      *reinterpret_cast<float4*>(&red[gid][col]) = make_float4(run.v[0], run.v[1], run.v[2], run.v[3]);
+      *reinterpret_cast<float4*>(&red[gid][col + 4]) = make_float4(run.v[4], run.v[5], run.v[6], run.v[7]);
+      __syncthreads();
+      if (warp == 0 && grp == 0) {
+        Row8 tot = run;
+        for (int g = 1; g < 64 && g * per < ns; ++g) {
+          const float4 lo = *reinterpret_cast<const float4*>(&red[g][col]), hi = *reinterpret_cast<const float4*>(&red[g][col + 4]);
+          Row8 o;
+          o.v[0] = lo.x; o.v[1] = lo.y; o.v[2] = lo.z; o.v[3] = lo.w;
+          o.v[4] = hi.x; o.v[5] = hi.y; o.v[6] = hi.z; o.v[7] = hi.w;
+          row8_add(tot, o);
+        }
+        agg_finish_row(a, tot, a.post ? __ldg(a.post + row) : 1.f, row, col, pol);
+      }
+      __syncthreads();
+    }
+    more = __syncthreads_or(k < nh) != 0;
   }
 }
 
