@@ -52,7 +52,7 @@ extern "C" {
  *                       — mgcn_aggregate_prescaled at H = 32 without mean / bias / residual on a 32-byte
  *                       aligned x, and mgcn_gcn_layer_fwd
  *   8 runs              the same with per = ceil(ns/8) for every ns — the tcgen05 hidden-32 layer kernels
- *                       (mgcn_gcn_layer_fwd_tc*, mgcn_gcn_layer_fwd_tm, mgcn_gcn_layer_bwd_fused)
+ *                       (mgcn_gcn_layer_fwd_tc*)
  * Each is independent of the grid, the device and the order of the hub table, so results are identical
  * from run to run and across devices; they give different bits for hubs of more than 2 segments. */
 #define MGCN_DEFAULT_HUB_THRESHOLD 64
@@ -367,30 +367,16 @@ int mgcn_gcn_layer_fwd_tc_gate(const mgcn_csr_t* g, const float* z, int64_t n_in
                                const float* out_scale, const uint32_t* keep, float keep_scale, const float* gate_ab,
                                const float* gate_c, int act_out, int64_t H, float* z_next, uint32_t* hmask,
                                void* workspace, size_t* workspace_bytes, void* stream);
-/* The same layer with the A operands of its products in TENSOR MEMORY (csrc/gcn_fwd_tm.cu): the gather lanes write
- * their sums with tcgen05.st.16x256b, the products are tcgen05.mma with A from TMEM — no operand image passes
- * through shared memory (the layer kernels are bound by the LSU data pipe).  Same contract, same results within
- * rounding (the contraction index is summed in a permuted order inside the tensor core). */
-int mgcn_gcn_layer_fwd_tm(const mgcn_csr_t* g, const float* z, int64_t n_in, const float* w, const float* res_w,
-                          const float* res_b, const float* bias, const float* in_scale, const float* post,
-                          const float* out_scale, int act_out, int64_t H, float* z_next, uint32_t* hmask,
-                          void* workspace, size_t* workspace_bytes, void* stream);
 
 /* backward, row-local part of layer n (dxw = pre * A^T gs comes from mgcn_aggregate_prescaled on the
  * structure built by source):
  *   G = dxw w^T + gy res_w;  dw = x^T dxw;  d_res_w = gy^T x;  d_res_b = colsum(gy)
  *   gy_prev = G * (x > 0);   gs_prev = post * gy_prev * bits(hmask_prev)      (both NULL: not wanted)
- * Weight gradients are reduced in a fixed order (deterministic, no atomics). */
-int mgcn_gcn_layer_bwd(const float* dxw, const float* gy, const float* x, const float* w,
-                       const float* res_w, const uint32_t* hmask_prev, const float* post, int64_t N,
-                       int64_t H, float* gy_prev, float* gs_prev, float* dw, float* d_res_w,
-                       float* d_res_b, void* workspace, size_t* workspace_bytes, void* stream);
-
-/* mgcn_gcn_layer_bwd on tcgen05.mma / tensor memory — the default of the hidden-32 stack.  Every operand is split
- * once into tf32 hi/lo images in shared memory (K-major images for the row-local products, SWIZZLE_128B_BASE32B
- * images for the transposed ones); a persistent CTA per SM runs producer / issuer / epilogue roles over two operand
- * stages and two accumulator buffers (csrc/gcn_layer_tc.cu).  Same contract and the same results within rounding
- * as mgcn_gcn_layer_bwd; 0.58 ms against 0.81 ms per layer at the botnet batch (profiles/r1b_layer_summary.md).
+ * Weight gradients are reduced in a fixed order (deterministic, no atomics).
+ * Runs on tcgen05.mma / tensor memory.  Every operand is split once into tf32 hi/lo images in shared memory (K-major
+ * images for the row-local products, SWIZZLE_128B_BASE32B images for the transposed ones); a persistent CTA per SM
+ * runs producer / issuer / epilogue roles over two operand stages and two accumulator buffers (csrc/gcn_layer_tc.cu).
+ * 0.58 ms per layer at the botnet batch (profiles/r1b_layer_summary.md).
  * x_scale [N] or NULL: the array passed as x holds x_scale (.) x (the stored format of mgcn_gcn_layer_fwd_tc); the
  * factor is divided out as the rows are loaded. */
 int mgcn_gcn_layer_bwd_tc(const float* dxw, const float* gy, const float* x, const float* x_scale, const float* w,
@@ -412,19 +398,6 @@ int mgcn_gcn_layer_bwd_tc_ex(const float* dxw, const float* gy, const float* x, 
                              const float* post, float bias_scale, int64_t N, int64_t H, float* gy_prev,
                              float* gs_prev, float* dw, float* d_res_w, float* d_res_b, float* d_bias,
                              void* workspace, size_t* workspace_bytes, void* stream);
-
-/* The backward of one hidden-32 layer as ONE launch (csrc/gcn_bwd_fused.cu): mgcn_aggregate_prescaled over the
- * by-source structure `gt` followed by mgcn_gcn_layer_bwd_tc, without the [N,32] array between them —
- *     dxw_j = row_scale_j * sum_{e: row[e]=j} gs[col[e]]     (autograd of gcn_base_models.py:237-241, the transposed
- *                                                             scatter; row_scale = the per-source degree factor or NULL)
- *     then the contract of mgcn_gcn_layer_bwd_tc with x = z / x_scale (z = the stored input of mgcn_gcn_layer_fwd_tc).
- * The gather warps write their sums into the tensor core's operand images; per layer the launch reads gs (gathered),
- * gy and z and writes gy_prev and gs_prev (both NULL: weight gradients only).  gt needs tasks / nbr_w (work order). */
-int mgcn_gcn_layer_bwd_fused(const mgcn_csr_t* gt, const float* gs, const float* gy, const float* z,
-                             const float* x_scale, const float* row_scale, const float* w, const float* res_w,
-                             const uint32_t* hmask_prev, const float* post, int64_t H,
-                             float* gy_prev, float* gs_prev, float* dw, float* d_res_w, float* d_res_b, void* workspace,
-                             size_t* workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Edge gates of the hidden-32 stack (csrc/gate.cu; EdgeGateProj, gcn_base_models.py:322-369, with in_edgedim None).

@@ -83,8 +83,6 @@ SIGNATURES = {
     "mgcn_gate_grad_by_target": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gate_grad_by_source": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                          c_ptr, c_ptr, c_size_p, c_ptr]),
-    "mgcn_gcn_layer_fwd_tm": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int,
-                                      c_i64, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_segment_max": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
     "mgcn_segment_max_ex": (c_int, [CSR_P, c_ptr, c_i64, c_i64, c_int, c_ptr, c_f32, c_ptr, c_ptr, c_ptr]),
     "mgcn_segment_max_bwd": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
@@ -111,14 +109,10 @@ SIGNATURES = {
                                   c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_fwd": (c_int, [CSR_P, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                    c_ptr, c_int, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
-    "mgcn_gcn_layer_bwd": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr,
-                                   c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_bwd_tc": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr,
                                       c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_gcn_layer_bwd_tc_ex": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_f32, c_i64,
                                          c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
-    "mgcn_gcn_layer_bwd_fused": (c_int, [CSR_P, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64,
-                                         c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_mask_bits_scale": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_ptr]),
     "mgcn_mask_bits_colsum": (c_int, [c_ptr, c_ptr, c_f32, c_i64, c_i64, c_ptr, c_ptr, c_size_p, c_ptr]),
     "mgcn_dropout_keep_bits": (c_int, [c_ptr, c_i64, c_i64, c_i64, c_f32, c_ptr, c_ptr]),

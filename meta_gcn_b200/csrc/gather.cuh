@@ -1,4 +1,4 @@
-// Row gather shared by the aggregation kernels (gcn_layer.cu, gcn_fwd_tc.cu, gcn_bwd_fused.cu).
+// Row gather shared by the aggregation kernels (gcn_layer.cu, gcn_fwd_tc.cu, gate.cu).
 #pragma once
 #include "common.cuh"
 

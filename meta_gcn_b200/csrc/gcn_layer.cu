@@ -12,12 +12,11 @@
 //     two dense products run on the tensor pipe (mma.sync m16n8k8, 3xTF32) out of shared memory, so
 //     per layer the forward reads m (gathered) and x once and writes x' and m' once.
 //   k_agg_plain   (agg_pipelined.cu; backward, transposed aggregation)   dxw = pre * A^T gs
-//   k_layer_bwd   (backward, row-local):
+//   k_layer_bwd_tc (gcn_layer_tc.cu, entry points mgcn_gcn_layer_bwd_tc* below; backward, row-local):
 //       G       = dxw W_n^T + gy R_n;   dW_n = x_n^T dxw;   dR_n = gy^T x_n;   dr_n = colsum(gy)
 //       gy_prev = G * (x_n > 0);        gs_prev = post * gy_prev * bits_{n-1}
 //     gy is the gradient w.r.t. y_n (outer ReLU already applied), gs the operand of the transposed
-//     aggregation of layer n-1.  Weight gradients accumulate in registers over all tiles of a warp and
-//     are reduced warp -> CTA -> grid in a fixed order (deterministic, no atomics).
+//     aggregation of layer n-1.  Weight gradients are reduced in a fixed order (deterministic, no atomics).
 //
 // Why the tensor pipe at H = 32: 6 products of [N,32]x[32,32] per layer are 0.53 TFLOP per step at the
 // botnet batch; the FP32 FMA peak (74 TFLOP/s) alone would cost 7 ms against a 5 ms HBM bound for the
@@ -796,180 +795,6 @@ int launch_agg_flat32(const mgcn_csr_t* g, const float* x, const float* post, in
 // -------------------------------------------------------------------------------------------------
 // backward, row-local
 // -------------------------------------------------------------------------------------------------
-struct LayerBwdArgs {
-  const float* dxw;          // [N,32]  pre * A^T gs          (transposed aggregation)
-  const float* gy;           // [N,32]  gradient w.r.t. y_n
-  const float* x;            // [N,32]  layer input x_n
-  const float* w;            // weight_node (in, out)
-  const float* res_w;        // residual weight (out, in)
-  const uint32_t* hmask_prev;  // bits of h_{n-1} > 0
-  const float* post;         // per-target factor or NULL
-  float* gy_prev;            // [N,32] or NULL
-  float* gs_prev;            // [N,32] or NULL
-  float* part_w;             // [grid][32*32]
-  float* part_r;             // [grid][32*32]
-  float* part_b;             // [grid][32]
-  int64_t n_rows;
-};
-
-constexpr int kBwdWarps = 8;
-constexpr int kBwdRows = 16 * kBwdWarps;  // rows per CTA tile
-constexpr int kLdx = kH + 8;              // x tile: only ever a transposed-product operand
-constexpr int kBwdSmemFloats = 4 * kPlane + kBwdRows * (2 * kLda + kLdx);
-
-template <int LD>
-__device__ __forceinline__ void stage_rows_async(const float* __restrict__ src, int64_t row0, int64_t N,
-                                                 float (*dst)[LD], int tid, uint64_t pol) {
-#pragma unroll
-  for (int i = 0; i < kBwdRows * 8 / (kBwdWarps * 32); ++i) {
-    const int c = i * (kBwdWarps * 32) + tid;
-    const int r = c >> 3, q = c & 7;
-    const int64_t gr = row0 + r;
-    cp_async16_hint(&dst[r][4 * q], src + (gr < N ? gr : 0) * kH + 4 * q, gr < N ? 16 : 0, pol);
-  }
-}
-
-// 16 rows of a tile -> global, 128 bytes per row, 4 rows per instruction
-__device__ __forceinline__ void store_rows16(float* __restrict__ dst, int64_t row0, int64_t N,
-                                             const float (*src)[kLda], int lane, uint64_t pol) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int c = i * 32 + lane;
-    const int r = c >> 3, q = c & 7;
-    const int64_t gr = row0 + r;
-    if (gr < N) st_f4_hint(dst + gr * kH + 4 * q, *reinterpret_cast<const float4*>(&src[r][4 * q]), pol);
-  }
-}
-
-// One CTA walks 128-row tiles.  Row-local products (G): warp w owns rows [16w, 16w+16).  Weight
-// gradients: warp w owns one 16x16 block of dW (w < 4) or dR (w >= 4) over all 128 rows of the tile,
-// so the persistent accumulators are 8 registers per thread and no cross-warp reduction is needed.
-__global__ void __launch_bounds__(kBwdWarps * 32, 2) k_layer_bwd(const LayerBwdArgs a) {
-  extern __shared__ __align__(16) float smem[];
-  float* planes = smem;  // W^T hi/lo, R hi/lo
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int g = lane >> 2, t = lane & 3;
-  float (*Dw)[kLda] = reinterpret_cast<float (*)[kLda]>(smem + 4 * kPlane);
-  float (*Gy)[kLda] = Dw + kBwdRows;
-  float (*Xs)[kLdx] = reinterpret_cast<float (*)[kLdx]>(smem + 4 * kPlane + 2 * kBwdRows * kLda);
-  fill_plane(a.w, 1, kH, planes, planes + kPlane, tid, kBwdWarps * 32);                  // (k=c, n=j) = W[j][c]
-  fill_plane(a.res_w, kH, 1, planes + 2 * kPlane, planes + 3 * kPlane, tid, kBwdWarps * 32);  // (k=c, n=j) = R[c][j]
-  const int prod = warp >> 2;            // 0: dW = x^T dxw, 1: dR = gy^T x
-  const int m0 = ((warp >> 1) & 1) * 16, n0 = (warp & 1) * 16;
-  float acc_blk[2][4];
-#pragma unroll
-  for (int j = 0; j < 2; ++j)
-#pragma unroll
-    for (int q = 0; q < 4; ++q) acc_blk[j][q] = 0.f;
-  float acc_b = 0.f;
-  const bool want_prev = a.gy_prev != nullptr;
-  const uint64_t pol = policy_evict_first();
-  const int64_t ntiles = (a.n_rows + kBwdRows - 1) / kBwdRows;
-  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int64_t row0 = tile * kBwdRows;
-    __syncthreads();  // previous tile fully consumed (also orders the plane fill)
-    stage_rows_async<kLda>(a.dxw, row0, a.n_rows, Dw, tid, pol);
-    stage_rows_async<kLda>(a.gy, row0, a.n_rows, Gy, tid, pol);
-    stage_rows_async<kLdx>(a.x, row0, a.n_rows, Xs, tid, pol);
-    uint32_t mybits = 0;
-    float mypost = 1.f;
-    const int64_t myrow = row0 + warp * 16 + lane;
-    if (want_prev && lane < 16 && myrow < a.n_rows) {
-      mybits = __ldg(a.hmask_prev + myrow);
-      if (a.post) mypost = __ldg(a.post + myrow);
-    }
-    cp_async_wait_all();
-    __syncthreads();
-    // weight-gradient block of this warp over the 128 rows, flushed to the RN accumulators every 32
-    {
-      const float* As = prod == 0 ? &Xs[0][0] : &Gy[0][0];
-      const int lda = prod == 0 ? kLdx : kLda;
-      const float* Bs = prod == 0 ? &Dw[0][0] : &Xs[0][0];
-      const int ldb = prod == 0 ? kLda : kLdx;
-#pragma unroll 1
-      for (int rc = 0; rc < kBwdRows; rc += 32) {
-        float mainc[2][4], corr[2][4];
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-          for (int q = 0; q < 4; ++q) mainc[j][q] = corr[j][q] = 0.f;
-#pragma unroll
-        for (int r0 = rc; r0 < rc + 32; r0 += 8) {
-          uint32_t ahi[4], alo[4];
-          split_tf32(As[(r0 + t) * lda + m0 + g], ahi[0], alo[0]);
-          split_tf32(As[(r0 + t) * lda + m0 + g + 8], ahi[1], alo[1]);
-          split_tf32(As[(r0 + t + 4) * lda + m0 + g], ahi[2], alo[2]);
-          split_tf32(As[(r0 + t + 4) * lda + m0 + g + 8], ahi[3], alo[3]);
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            uint32_t bhi[2], blo[2];
-            split_tf32(Bs[(r0 + t) * ldb + n0 + 8 * j + g], bhi[0], blo[0]);
-            split_tf32(Bs[(r0 + t + 4) * ldb + n0 + 8 * j + g], bhi[1], blo[1]);
-            mma_tf32_16x8x8(corr[j], alo, bhi);
-            mma_tf32_16x8x8(corr[j], ahi, blo);
-            mma_tf32_16x8x8(mainc[j], ahi, bhi);
-          }
-        }
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-          for (int q = 0; q < 4; ++q) acc_blk[j][q] += mainc[j][q] + corr[j][q];
-      }
-      float colsum = 0.f;
-#pragma unroll
-      for (int r = 0; r < 16; ++r) colsum += Gy[warp * 16 + r][lane];
-      acc_b += colsum;
-    }
-    if (want_prev) {
-      __syncthreads();  // every warp is done reading all rows of Dw / Gy
-      float (*Dt)[kLda] = Dw + warp * 16;
-      float (*Gt)[kLda] = Gy + warp * 16;
-      float accg[4][4], second[4][4];
-      warp_gemm16<kH, kH>(&Dt[0][0], kLda, planes, planes + kPlane, kLdb, accg, lane);
-      warp_gemm16<kH, kH>(&Gt[0][0], kLda, planes + 2 * kPlane, planes + 3 * kPlane, kLdb, second, lane);
-      __syncwarp();  // all fragment reads of this warp's rows are done
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        const int rr = g + 8 * half;
-        const uint32_t bits = __shfl_sync(0xffffffffu, mybits, rr);
-        const float ps = __shfl_sync(0xffffffffu, mypost, rr);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int c = 8 * j + 2 * t;
-          const float2 xv = *reinterpret_cast<const float2*>(&Xs[warp * 16 + rr][c]);
-          const float g0 = xv.x > 0.f ? accg[j][2 * half] + second[j][2 * half] : 0.f;
-          const float g1 = xv.y > 0.f ? accg[j][2 * half + 1] + second[j][2 * half + 1] : 0.f;
-          *reinterpret_cast<float2*>(&Dt[rr][c]) = make_float2(g0, g1);
-          const float s0 = ((bits >> c) & 1u) ? g0 * ps : 0.f;
-          const float s1 = ((bits >> (c + 1)) & 1u) ? g1 * ps : 0.f;
-          *reinterpret_cast<float2*>(&Gt[rr][c]) = make_float2(s0, s1);
-        }
-      }
-      __syncwarp();
-      store_rows16(a.gy_prev, row0 + warp * 16, a.n_rows, Dt, lane, pol);
-      store_rows16(a.gs_prev, row0 + warp * 16, a.n_rows, Gt, lane, pol);
-    }
-  }
-  // this warp's 16x16 block of dW (row = input j, col = output c) or dR (row = output c, col = input j)
-  float* part = (prod == 0 ? a.part_w : a.part_r) + (int64_t)blockIdx.x * kH * kH;
-#pragma unroll
-  for (int j = 0; j < 2; ++j) {
-    const int c = n0 + 8 * j + 2 * t;
-    *reinterpret_cast<float2*>(part + (m0 + g) * kH + c) = make_float2(acc_blk[j][0], acc_blk[j][1]);
-    *reinterpret_cast<float2*>(part + (m0 + g + 8) * kH + c) = make_float2(acc_blk[j][2], acc_blk[j][3]);
-  }
-  __syncthreads();
-  float* red = smem + 4 * kPlane;
-  red[warp * 32 + lane] = acc_b;
-  __syncthreads();
-  if (tid < 32) {
-    float s = red[tid];
-#pragma unroll
-    for (int w = 1; w < kBwdWarps; ++w) s += red[w * 32 + tid];
-    a.part_b[(int64_t)blockIdx.x * kH + tid] = s;
-  }
-}
-
 // gs = post * gy * bits   (seed of the backward: last layer has no outer ReLU)
 __global__ void __launch_bounds__(256) k_mask_bits_scale(const float* __restrict__ gy,
                                                          const uint32_t* __restrict__ bits,
@@ -989,12 +814,6 @@ __global__ void __launch_bounds__(256) k_mask_bits_scale(const float* __restrict
     v.w = (b & 8u) ? v.w * s : 0.f;
     reinterpret_cast<float4*>(gs)[i] = v;
   }
-}
-
-static int bwd_grid(int64_t N) {
-  const int64_t tiles = ceil_div(N > 0 ? N : 1, kBwdRows);
-  const int64_t p = (int64_t)kNumSMs * 2;
-  return (int)(tiles < p ? tiles : p);
 }
 
 }  // namespace mgcn
@@ -1144,53 +963,8 @@ extern "C" int mgcn_gcn_first_layer_fwd_bias(const float* s, const float* x, int
   return MGCN_OK;
 }
 
-extern "C" int mgcn_gcn_layer_bwd(const float* dxw, const float* gy, const float* x, const float* w,
-                                  const float* res_w, const uint32_t* hmask_prev, const float* post,
-                                  int64_t N, int64_t H, float* gy_prev, float* gs_prev, float* dw,
-                                  float* d_res_w, float* d_res_b, void* workspace,
-                                  size_t* workspace_bytes, void* stream) {
-  MGCN_REQUIRE(workspace_bytes != nullptr, MGCN_ERR_NULL);
-  MGCN_REQUIRE(H == kH, MGCN_ERR_SHAPE);
-  MGCN_REQUIRE(N >= 0 && N < (int64_t(1) << 31), MGCN_ERR_RANGE);
-  const int P = bwd_grid(N);
-  WorkspaceCarver ws(workspace);
-  float* part_w = ws.take<float>((size_t)P * kH * kH);
-  float* part_r = ws.take<float>((size_t)P * kH * kH);
-  float* part_b = ws.take<float>((size_t)P * kH);
-  if (workspace == nullptr) {
-    *workspace_bytes = ws.bytes();
-    return MGCN_OK;
-  }
-  MGCN_REQUIRE(*workspace_bytes >= ws.bytes(), MGCN_ERR_WORKSPACE);
-  MGCN_REQUIRE(dxw && gy && x && w && res_w && dw && d_res_w && d_res_b, MGCN_ERR_NULL);
-  MGCN_REQUIRE((gy_prev == nullptr) == (gs_prev == nullptr), MGCN_ERR_NULL);
-  MGCN_REQUIRE(!gy_prev || hmask_prev, MGCN_ERR_NULL);
-  MGCN_REQUIRE(aligned16(dxw) && aligned16(gy) && aligned16(x) && (!gy_prev || aligned16(gy_prev)) &&
-                   (!gs_prev || aligned16(gs_prev)),
-               MGCN_ERR_ALIGN);
-  if (N == 0) return MGCN_OK;
-  LayerBwdArgs a{};
-  a.dxw = dxw; a.gy = gy; a.x = x; a.w = w; a.res_w = res_w; a.hmask_prev = hmask_prev; a.post = post;
-  a.gy_prev = gy_prev; a.gs_prev = gs_prev;
-  a.part_w = part_w; a.part_r = part_r; a.part_b = part_b;
-  a.n_rows = N;
-  const size_t smem = sizeof(float) * kBwdSmemFloats;
-  // the attribute belongs to (function, device): set on every call (cheap), so a second GPU in the same process
-  // gets it too and a failure is reported every time
-  cudaError_t attr_err = cudaSuccess;
-  {
-    attr_err = cudaFuncSetAttribute(k_layer_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  }
-  MGCN_CHECK_CUDA(attr_err);
-  MGCN_LAUNCH(k_layer_bwd, P, kBwdWarps * 32, smem, stream, a);
-  int rc = launch_reduce_partials(part_w, P, kH * kH, kH, dw, kH, 1, stream);
-  if (rc == MGCN_OK) rc = launch_reduce_partials(part_r, P, kH * kH, kH, d_res_w, kH, 1, stream);
-  if (rc == MGCN_OK) rc = launch_reduce_partials(part_b, P, kH, kH, d_res_b, 0, 1, stream);
-  return rc;
-}
-
-// Same contract on tcgen05 / TMEM (gcn_layer_tc.cu).  Measured 0.99 ms against 0.83 ms for the mma.sync
-// kernel above at the botnet batch (profiles/r1_layer_summary.md): correct, not yet the default.
+// Row-local backward of the hidden-32 stack (contract: the header comment above, include/mgcn.h) on tcgen05 / TMEM
+// (gcn_layer_tc.cu).  x_scale [N] or NULL: x holds x_scale (.) x.
 extern "C" int mgcn_gcn_layer_bwd_tc(const float* dxw, const float* gy, const float* x, const float* x_scale,
                                      const float* w, const float* res_w, const uint32_t* hmask_prev, const float* post,
                                      int64_t N, int64_t H, float* gy_prev, float* gs_prev, float* dw,

@@ -1,5 +1,5 @@
 // Row-local backward of one residual GCN layer at hidden 32 on the 5th-generation tensor cores
-// (tcgen05.mma, accumulators in tensor memory) — same contract as k_layer_bwd (gcn_layer.cu):
+// (tcgen05.mma, accumulators in tensor memory), entry points mgcn_gcn_layer_bwd_tc* (gcn_layer.cu):
 //     G = dxw W^T + gy R;   dW = x^T dxw;   dR = gy^T x;   dr = colsum(gy)
 //     gy_prev = G * (x > 0);   gs_prev = post * gy_prev * bits(hmask_prev)
 // Every operand element is split ONCE into hi/lo tf32 images in shared memory and one thread issues 24
@@ -25,7 +25,7 @@
 //   barriers   full[stage] producers -> issuer, done[pair buffer][set] tensor core -> producers + epilogue,
 //              tfree[pair buffer] epilogue -> issuers   (done is per pair buffer so that no waiter can be lapped)
 // Measured at the botnet batch (profiles/r1b_layer_summary.md): 0.99 ms as CTA-wide phases -> 0.58 ms, against 0.81 ms
-// for the mma.sync kernel; 4.0 TB/s of algorithmic bytes.  The limiter is now the shared-memory data pipe
+// for the mma.sync kernel it replaced; 4.0 TB/s of algorithmic bytes.  The limiter is now the shared-memory data pipe
 // (l1tex__data_pipe_lsu_wavefronts 83 %: 47 M store wavefronts for the ten images + the tensor core's operand
 // reads), not HBM (48 %) or the tensor pipe (23 %).
 #include <mutex>

@@ -9,24 +9,14 @@ masks of the backward are folded into operand loads; no autograd graph, no [N,H]
 beyond the saved layer outputs.  Per layer: forward = transform, aggregation, residual transform
 (3 launches); backward = weight-gradient x2, transform x2, mask/scale, transposed aggregation.
 """
-import os
-
 import torch
 
 from . import ops
 
 FUSED_WIDTHS = (16, 32, 64, 128)
-# row-local backward of the hidden-32 stack: tcgen05 / TMEM pipeline (0.64 ms per layer at the botnet batch)
-# or the mma.sync kernel (0.81 ms); both pass the same parity tests
-BWD_TENSOR_MEMORY = True
 # hidden-32 stack: aggregate-then-transform forward on tcgen05 (csrc/gcn_fwd_tc.cu; one [N,32] read + one write per
 # layer) or the transform-then-aggregate kernels of round 1 (csrc/gcn_layer.cu); both pass the same parity tests
 FORWARD_AGGREGATE_FIRST = True
-# aggregate-then-transform stack: transposed aggregation + row-local backward as ONE launch per layer
-# (csrc/gcn_bwd_fused.cu: no dxw array, 0.9 GB less DRAM traffic per layer) instead of two.  Same parity tests,
-# identical from run to run — but measured SLOWER at the botnet batch (1.45 ms against 0.48 + 0.61 ms: the per-row
-# operand-image work needs more warps than fit next to a 16-warp gather), so it is off by default
-BWD_FUSED = os.environ.get("MGCN_BWD_FUSED", "0") == "1"
 
 
 def dropout_seed(device):
@@ -176,7 +166,7 @@ class _ResidualGCNStack32(torch.autograd.Function):
         for n in range(L - 1, 0, -1):
             dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
             gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_impl(
-                dxw, gy, xs[n], layers[n][0], layers[n][1], hmasks[n - 1], post, True, BWD_TENSOR_MEMORY)
+                dxw, gy, xs[n], layers[n][0], layers[n][1], hmasks[n - 1], post, True)
             grads[3 * n], grads[3 * n + 1], grads[3 * n + 2] = dw, drw, drb
             gy, gs = gy_prev, gs_prev
         grads[1], grads[2] = ops.linear_wgrad_impl(xs[0], gy, True, True)
@@ -307,31 +297,16 @@ class _ResidualGCNStack32AT(torch.autograd.Function):
             if gated:
                 # the gate's passes form dxw; the row-local launch takes it as the transposed aggregation's
                 dxw = gate_backward(n, ops.linear_impl(zs[n], w, False), gs)
-                if has_bias:
-                    gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
-                        dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, hmasks[n], post,
-                        ctx.bias_scale, want_prev, x_scale=sigma)
-                    grads[per * n + 1] = db
-                else:
-                    gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_impl(
-                        dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
-                        want_prev, True, x_scale=sigma)
-            elif has_bias:
-                # the one-launch backward (BWD_FUSED) has no bias gradient: a model with bias takes the two launches
-                dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
-                gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
-                    dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, hmasks[n], post, ctx.bias_scale,
-                    want_prev, x_scale=sigma)
-                grads[per * n + 1] = db
-            elif BWD_FUSED:
-                gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_fused_impl(
-                    bwd, gs, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
-                    row_scale=pre, x_scale=sigma, want_prev=want_prev)
             else:
                 dxw = ops.aggregate_prescaled_impl(bwd, gs, pre, 0, None, None, 0)
+            hmask_prev = hmasks[n - 1] if want_prev else None
+            if has_bias:
+                gy_prev, gs_prev, dw, drw, drb, db = ops.gcn_layer_bwd_bias_impl(
+                    dxw, gy, zs[n], w, res_w, hmask_prev, hmasks[n], post, ctx.bias_scale, want_prev, x_scale=sigma)
+                grads[per * n + 1] = db
+            else:
                 gy_prev, gs_prev, dw, drw, drb = ops.gcn_layer_bwd_impl(
-                    dxw, gy, zs[n], w, res_w, hmasks[n - 1] if want_prev else None, post,
-                    want_prev, True, x_scale=sigma)
+                    dxw, gy, zs[n], w, res_w, hmask_prev, post, want_prev, x_scale=sigma)
             grads[per * n], grads[per * n + per - 2], grads[per * n + per - 1] = dw, drw, drb
             if want_prev:
                 gy, gs = gy_prev, gs_prev

@@ -536,22 +536,13 @@ def _keep_rows(keep, N, W):
     return keep.contiguous()
 
 
-# forward layer of the hidden-32 stack: A operands through tensor memory (csrc/gcn_fwd_tm.cu) or as shared-memory
-# images (csrc/gcn_fwd_tc.cu); both pass the same parity tests
-FWD_TMEM_OPERANDS = False
-
-
-def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, tmem_operands=None,
-                          keep=None, keep_scale=1.0, gate_ab=None, gate_c=None):
+def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, keep=None,
+                          keep_scale=1.0, gate_ab=None, gate_c=None):
     """one aggregate-then-transform forward layer at hidden 32 on tcgen05 (mgcn_gcn_layer_fwd_tc_ex): z = in_scale (.) x
     [N,32]; returns (z_next = out_scale (.) x_next [N,32], hmask int32[N]).  keep int32 [N]: dropout keep bits of the
     layer (kept entries of h multiplied by keep_scale, dropped ones cleared in hmask too).  gate_ab [N,2] (from
     gate_scores_impl) and gate_c [1]: every gathered row weighted by its edge gate (mgcn_gcn_layer_fwd_tc_gate)"""
     _need_cuda(z, w, res_w, res_b, bias, in_scale, post, out_scale, keep, gate_ab, gate_c)
-    tmem = FWD_TMEM_OPERANDS if tmem_operands is None else tmem_operands
-    if (keep is not None or gate_ab is not None) and tmem:
-        raise ValueError("dropout keep bits and edge gates need the shared-memory operand forward "
-                         "(mgcn_gcn_layer_fwd_tc_gate), not the TMEM-operand kernel")
     z = _f32c(z, "z")
     w = _f32c(w, "w")
     res_w = _f32c(res_w, "res_w")
@@ -570,9 +561,7 @@ def gcn_layer_fwd_tc_impl(csr, z, w, res_w, res_b, bias, in_scale, post, out_sca
     lead = (ctypes.byref(csr.struct()), _ptr(z), z.size(0), _ptr(w), _ptr(res_w), _ptr(res_b), _ptr(bias),
             _ptr(in_scale), _ptr(post), _ptr(out_scale))
     tail = (int(act_out), H, _ptr(z_next), _ptr(hmask))
-    if tmem:
-        fn, args = lib.mgcn_gcn_layer_fwd_tm, lead + tail
-    elif gate_ab is not None:
+    if gate_ab is not None:
         keep = _keep_rows(keep, n_rows, 1)
         gate_ab, gate_c = _gate_operands(gate_ab, gate_c, z.size(0))
         fn, args = lib.mgcn_gcn_layer_fwd_tc_gate, lead + (_ptr(keep), float(keep_scale), _ptr(gate_ab),
@@ -661,12 +650,14 @@ def gate_grad_by_source_impl(csr_t, gs, m, ab, c, db, pre, u, v, sigma):
     return dxw, dsc
 
 
-def gcn_layer_bwd_impl(dxw, gy, x, w, res_w, hmask_prev, post, want_prev=True, tensor_memory=False, x_scale=None):
-    """row-local backward of one layer at hidden 32 (mgcn_gcn_layer_bwd): returns
-    (gy_prev | None, gs_prev | None, dw, d_res_w, d_res_b).  x_scale [N] (tensor_memory only): x holds x_scale (.) x"""
+def gcn_layer_bwd_impl(dxw, gy, x, w, res_w, hmask_prev, post, want_prev=True, tensor_memory=True, x_scale=None):
+    """row-local backward of one layer at hidden 32 on tcgen05 (mgcn_gcn_layer_bwd_tc): returns
+    (gy_prev | None, gs_prev | None, dw, d_res_w, d_res_b).  x_scale [N]: x holds x_scale (.) x.  tensor_memory is
+    kept only for existing positional callers; False raises ValueError"""
+    if not tensor_memory:
+        raise ValueError("the mma.sync row-local backward was removed: gcn_layer_bwd runs on tcgen05 only "
+                         "(tensor_memory=True)")
     _need_cuda(dxw, gy, x, w, res_w, hmask_prev, post, x_scale)
-    if x_scale is not None and not tensor_memory:
-        raise ValueError("x_scale needs the tcgen05 backward")
     x_scale = _f32c(x_scale, "x_scale")
     dxw = _f32c(dxw, "dxw")
     gy = _f32c(gy, "gy")
@@ -682,10 +673,9 @@ def gcn_layer_bwd_impl(dxw, gy, x, w, res_w, hmask_prev, post, want_prev=True, t
     drw = torch.empty(H, H, dtype=torch.float32, device=dev)
     drb = torch.empty(H, dtype=torch.float32, device=dev)
     lib = _lib.load()
-    args = (_ptr(dxw), _ptr(gy), _ptr(x), *((_ptr(x_scale),) if tensor_memory else ()), _ptr(w), _ptr(res_w),
-            _ptr(hmask_prev) if want_prev else None,
+    args = (_ptr(dxw), _ptr(gy), _ptr(x), _ptr(x_scale), _ptr(w), _ptr(res_w), _ptr(hmask_prev) if want_prev else None,
             _ptr(post), N, H, _ptr(gy_prev), _ptr(gs_prev), _ptr(dw), _ptr(drw), _ptr(drb))
-    fn = lib.mgcn_gcn_layer_bwd_tc if tensor_memory else lib.mgcn_gcn_layer_bwd
+    fn = lib.mgcn_gcn_layer_bwd_tc
     ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
     _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
     return gy_prev, gs_prev, dw, drw, drb
@@ -736,38 +726,6 @@ def mask_bits_colsum_impl(gy, bits, scale=1.0):
     ws, nbytes = _workspace(lambda w_, nb, stm: lib.mgcn_mask_bits_colsum(*args, w_, nb, stm), gy.device)
     _lib.check(lib.mgcn_mask_bits_colsum(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
     return d_bias
-
-
-def gcn_layer_bwd_fused_impl(csr_t, gs, gy, z, w, res_w, hmask_prev, post, row_scale=None, x_scale=None, want_prev=True):
-    """the whole backward of one hidden-32 layer in one launch (mgcn_gcn_layer_bwd_fused): transposed aggregation of gs
-    over the by-source structure csr_t (scaled by row_scale) + the row-local products with x = z / x_scale; returns
-    (gy_prev | None, gs_prev | None, dw, d_res_w, d_res_b)"""
-    _need_cuda(gs, gy, z, w, res_w, hmask_prev, post, row_scale, x_scale)
-    gs = _f32c(gs, "gs")
-    gy = _f32c(gy, "gy")
-    z = _f32c(z, "z")
-    w = _f32c(w, "w")
-    res_w = _f32c(res_w, "res_w")
-    post = _f32c(post, "post")
-    row_scale = _f32c(row_scale, "row_scale")
-    x_scale = _f32c(x_scale, "x_scale")
-    N, H = z.shape
-    if csr_t.n_rows != N or gs.size(0) != N or gy.size(0) != N:
-        raise ValueError("gcn_layer_bwd_fused needs a square structure and [N,32] operands")
-    dev = z.device
-    gy_prev = torch.empty_like(z) if want_prev else None
-    gs_prev = torch.empty_like(z) if want_prev else None
-    dw = torch.empty(H, H, dtype=torch.float32, device=dev)
-    drw = torch.empty(H, H, dtype=torch.float32, device=dev)
-    drb = torch.empty(H, dtype=torch.float32, device=dev)
-    lib = _lib.load()
-    args = (ctypes.byref(csr_t.struct()), _ptr(gs), _ptr(gy), _ptr(z), _ptr(x_scale), _ptr(row_scale), _ptr(w),
-            _ptr(res_w), _ptr(hmask_prev) if want_prev else None, _ptr(post), H, _ptr(gy_prev), _ptr(gs_prev),
-            _ptr(dw), _ptr(drw), _ptr(drb))
-    fn = lib.mgcn_gcn_layer_bwd_fused
-    ws, nbytes = _workspace(lambda w_, nb, stm: fn(*args, w_, nb, stm), dev)
-    _lib.check(fn(*args, _ptr(ws), ctypes.byref(nbytes), _stream()))
-    return gy_prev, gs_prev, dw, drw, drb
 
 
 def mask_bits_scale_impl(gy, bits, post):
@@ -1216,8 +1174,7 @@ def _op_propagate(csr, csr_t, hub_threshold, x, nbr_scale, row_scale, act):
 def _op_layer_fwd_tc_gate(csr, hub_threshold, z, w, res_w, res_b, bias, in_scale, post, out_scale, act_out, keep,
                           keep_scale, gate_ab, gate_c):
     return gcn_layer_fwd_tc_impl(_as_csr(csr, hub_threshold), z, w, res_w, res_b, bias, in_scale, post, out_scale,
-                                 act_out, tmem_operands=False, keep=keep, keep_scale=keep_scale, gate_ab=gate_ab,
-                                 gate_c=gate_c)
+                                 act_out, keep=keep, keep_scale=keep_scale, gate_ab=gate_ab, gate_c=gate_c)
 
 
 _IMPLS2 = {

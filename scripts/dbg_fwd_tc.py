@@ -12,8 +12,6 @@ from meta_gcn_b200.graph import GraphStructure
 
 dev = "cuda"
 H = 32
-if "--tmem" in sys.argv:
-    ops.FWD_TMEM_OPERANDS = True
 torch.manual_seed(0)
 
 

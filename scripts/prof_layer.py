@@ -59,8 +59,6 @@ timeit("layer_fwd (gather+2 products)", lambda: ops.gcn_layer_fwd_impl(gs.fwd, m
 if hasattr(ops, "gcn_layer_fwd_tc_impl"):
     timeit("layer_fwd_tc (aggregate-then-transform)",
            lambda: ops.gcn_layer_fwd_tc_impl(gs.fwd, x, w, r, rb, None, dis, dis, dis, 1), b_agg(n, e, H))
-    timeit("layer_fwd_tm (A operands in TMEM)",
-           lambda: ops.gcn_layer_fwd_tc_impl(gs.fwd, x, w, r, rb, None, dis, dis, dis, 1, tmem_operands=True), b_agg(n, e, H))
 timeit("layer_fwd last (no next)", lambda: ops.gcn_layer_fwd_impl(gs.fwd, m, x, None, r, rb, None, None, dis, dis, 0),
        4 * e + 8 * n + 3 * nh)
 x1 = torch.ones(n, 1, device=dev)
@@ -71,11 +69,7 @@ timeit("agg_plain bwd structure", lambda: ops.aggregate_prescaled_impl(gs.bwd, g
        b_agg(n, e, H))
 timeit("agg_plain fwd structure", lambda: ops.aggregate_prescaled_impl(gs.fwd, gy, dis, 0, None, None, 1),
        b_agg(n, e, H))
-timeit("layer_bwd (row-local, 4 products)", lambda: ops.gcn_layer_bwd_impl(m, gy, x, w, r, bits, dis, True), 5 * nh + 8 * n)
-timeit("layer_bwd tcgen05 variant", lambda: ops.gcn_layer_bwd_impl(m, gy, x, w, r, bits, dis, True, True), 5 * nh + 8 * n)
-if hasattr(ops, "gcn_layer_bwd_fused_impl"):
-    timeit("layer_bwd fused (gather + 4 products)",
-           lambda: ops.gcn_layer_bwd_fused_impl(gs.bwd, m, gy, x, w, r, bits, dis, row_scale=dis, x_scale=dis), b_agg(n, e, H) + nh)
+timeit("layer_bwd (row-local, tcgen05)", lambda: ops.gcn_layer_bwd_impl(m, gy, x, w, r, bits, dis, True), 5 * nh + 8 * n)
 timeit("mask_bits_scale", lambda: ops.mask_bits_scale_impl(gy, bits, dis), 2 * nh + 8 * n)
 timeit("torch copy", lambda: m.copy_(x), 2 * nh)
 # the step's first and last stages (H_in = 1 first layer, output layer + loss)

@@ -58,11 +58,7 @@ def assert_parity_arbitrated(actual, ref32, ref64, what, rtol=1e-5):
     return rel, rel32
 
 
-@pytest.mark.parametrize("bwd_fused", [False, True])
-def test_c1_full_graph_12_layers_vs_oracle(bwd_fused, monkeypatch):
-    """bwd_fused: the layer backward as one launch (csrc/gcn_bwd_fused.cu, fused.BWD_FUSED) instead of two"""
-    from meta_gcn_b200 import fused
-    monkeypatch.setattr(fused, "BWD_FUSED", bwd_fused)
+def test_c1_full_graph_12_layers_vs_oracle():
     g = D.synth_botnet_graph(seed=0)
     x = torch.from_numpy(g["x"])
     ei = torch.from_numpy(g["edge_index"])

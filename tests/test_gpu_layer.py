@@ -95,9 +95,8 @@ def test_layer_fwd_is_deterministic_and_order_exact():
     assert_bitexact(outs[0], torch.relu(ref), "edge-order sum")
 
 
-@pytest.mark.parametrize("tensor_memory", [False, True])
 @pytest.mark.parametrize("n,want_prev", [(1000, True), (1003, True), (131, False), (7, True), (40000, True), (300001, True), (151617, False)])
-def test_layer_bwd(n, want_prev, tensor_memory):
+def test_layer_bwd(n, want_prev):
     gen = torch.Generator().manual_seed(n)
     dxw = torch.randn(n, H, generator=gen)
     gy = torch.randn(n, H, generator=gen)
@@ -108,7 +107,7 @@ def test_layer_bwd(n, want_prev, tensor_memory):
     bits = torch.randint(-2 ** 31, 2 ** 31 - 1, (n,), generator=gen, dtype=torch.int64).to(torch.int32)
     d = lambda t: t.to(DEV)
     gyp, gsp, dw, drw, drb = ops.gcn_layer_bwd_impl(d(dxw), d(gy), d(x), d(w), d(res_w), d(bits), d(post),
-                                                    want_prev, tensor_memory)
+                                                    want_prev)
     D = lambda t: t.double()
     assert_parity(dw, D(x).t() @ D(dxw), "dW")
     assert_parity(drw, D(gy).t() @ D(x), "dR")
@@ -221,10 +220,8 @@ def _giant_hub_graph(n=4000):
     (4000, -1, 1, True, False),      # giant hubs (141 / 55 / 8 segments)
     (300001, 1500000, 1, True, False),
 ])
-@pytest.mark.parametrize("tmem_operands", [False, True])
-def test_layer_fwd_tc_aggregate_then_transform(n, e, act_out, scaled, with_bias, tmem_operands):
-    """mgcn_gcn_layer_fwd_tc (operand images in shared memory) and mgcn_gcn_layer_fwd_tm (operands in tensor memory)
-    against an fp64 dense / sparse restatement of gcn_model.py:89-106 +
+def test_layer_fwd_tc_aggregate_then_transform(n, e, act_out, scaled, with_bias):
+    """mgcn_gcn_layer_fwd_tc against an fp64 dense / sparse restatement of gcn_model.py:89-106 +
     gcn_base_models.py:199-243 with the stored format z = sigma (.) x: outputs (scaled by out_scale), mask words;
     ragged tile counts, empty rows, isolated nodes, hub rows, several tiles per CTA."""
     if e == -1:
@@ -244,7 +241,7 @@ def test_layer_fwd_tc_aggregate_then_transform(n, e, act_out, scaled, with_bias,
     gs = GraphStructure(ei.to(DEV), n, hub_threshold=64)
     d = lambda t: None if t is None else t.to(DEV)
     zn, hm = ops.gcn_layer_fwd_tc_impl(gs.fwd, d(z), d(w), d(res_w), d(res_b), d(bias), d(sigma), d(post), d(outs),
-                                       act_out, tmem_operands=tmem_operands)
+                                       act_out)
     D = lambda t: t.double()
     agg = torch.zeros(n, H, dtype=torch.float64).index_add_(0, ei[1], D(z)[ei[0]])
     s = D(post).view(-1, 1) * agg
@@ -263,7 +260,7 @@ def test_layer_fwd_tc_aggregate_then_transform(n, e, act_out, scaled, with_bias,
     assert (got[sure] == (hn[sure] > 0)).all()
     # run-to-run identical (fixed summation orders, no atomics on data)
     zn2, hm2 = ops.gcn_layer_fwd_tc_impl(gs.fwd, d(z), d(w), d(res_w), d(res_b), d(bias), d(sigma), d(post), d(outs),
-                                         act_out, tmem_operands=tmem_operands)
+                                         act_out)
     assert_bitexact(zn, zn2, "run-to-run")
     assert_bitexact(hm, hm2, "run-to-run mask")
 
@@ -301,11 +298,11 @@ def test_layer_bwd_tc_scaled_input(n):
     (300001, 1500000, True, True),
     (151617, 700000, True, False),
 ])
-def test_layer_bwd_fused(n, e, scaled, want_prev):
-    """mgcn_gcn_layer_bwd_fused (transposed aggregation + row-local products in one launch) against an fp64 restatement
-    of the autograd of gcn_model.py:89-106 / gcn_base_models.py:199-243 in the stored format z = sigma (.) x: dxw is
-    never materialised, so it is checked through dW, gy_prev and gs_prev; ragged tile counts, rows without entries,
-    hub rows, several tiles per CTA; and the two-launch path (mgcn_aggregate_prescaled + mgcn_gcn_layer_bwd_tc)."""
+def test_layer_bwd_two_launch(n, e, scaled, want_prev):
+    """the layer backward of the hidden-32 stack as it runs there, mgcn_aggregate_prescaled over the by-source structure
+    followed by mgcn_gcn_layer_bwd_tc, against an fp64 restatement of the autograd of gcn_model.py:89-106 /
+    gcn_base_models.py:199-243 in the stored format z = sigma (.) x: ragged tile counts, rows without entries, hub rows,
+    several tiles per CTA."""
     if e == -1:
         ei = _giant_hub_graph(n)
     else:
@@ -323,8 +320,12 @@ def test_layer_bwd_fused(n, e, scaled, want_prev):
     z = x * sigma.view(-1, 1) if scaled else x
     struct = GraphStructure(ei.to(DEV), n, hub_threshold=64)
     d = lambda t: None if t is None else t.to(DEV)
-    args = (struct.bwd, d(gs_in), d(gy), d(z), d(w), d(res_w), d(bits), d(post))
-    gyp, gsp, dw, drw, drb = ops.gcn_layer_bwd_fused_impl(*args, row_scale=d(pre), x_scale=d(sigma), want_prev=want_prev)
+
+    def backward():
+        dxw = ops.aggregate_prescaled_impl(struct.bwd, d(gs_in), d(pre), 0, None, None, 0)
+        return ops.gcn_layer_bwd_impl(dxw, d(gy), d(z), d(w), d(res_w), d(bits), d(post), want_prev, x_scale=d(sigma))
+
+    gyp, gsp, dw, drw, drb = backward()
     D = lambda t: t.double()
     # dxw_j = pre_j * sum over edges j -> i of gs_i
     dxw = torch.zeros(n, H, dtype=torch.float64).index_add_(0, ei[0], D(gs_in)[ei[1]])
@@ -343,13 +344,6 @@ def test_layer_bwd_fused(n, e, scaled, want_prev):
     b = ((bits.numpy().astype(np.uint32)[:, None] >> np.arange(H, dtype=np.uint32)[None, :]) & 1).astype(np.float64)
     assert_parity(gsp, D(post).view(-1, 1) * gy_ref * torch.from_numpy(b), "gs_prev")
     # run-to-run identical (fixed summation orders, no atomics on data)
-    again = ops.gcn_layer_bwd_fused_impl(*args, row_scale=d(pre), x_scale=d(sigma), want_prev=want_prev)
+    again = backward()
     for got, ref, name in zip((gyp, gsp, dw, drw, drb), again, ("gy_prev", "gs_prev", "dW", "dR", "dr")):
         assert_bitexact(got, ref, "run-to-run " + name)
-    # the two-launch path computes the same thing
-    if n > 0:
-        dxw2 = ops.aggregate_prescaled_impl(struct.bwd, d(gs_in), d(pre), 0, None, None, 0)
-        gyp2, gsp2, dw2, drw2, drb2 = ops.gcn_layer_bwd_impl(dxw2, d(gy), d(z), d(w), d(res_w), d(bits), d(post), True, True,
-                                                             x_scale=d(sigma))
-        assert_parity(gyp, gyp2.double().cpu(), "gy_prev vs two launches")
-        assert_parity(dw, dw2.double().cpu(), "dW vs two launches")

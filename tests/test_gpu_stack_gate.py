@@ -152,8 +152,7 @@ def test_gated_forward_layer_vs_fp64_and_null_gate(dropout):
     keep = torch.randint(-2 ** 31, 2 ** 31 - 1, (n,), generator=gen, dtype=torch.int64).to(torch.int32).to(DEV) \
         if dropout else None
     ks = 2.0 if dropout else 1.0
-    ref_ex = ops.gcn_layer_fwd_tc_impl(fwd, z, w, rw, rb, b, in_scale, post, out_scale, 1, tmem_operands=False,
-                                       keep=keep, keep_scale=ks)
+    ref_ex = ops.gcn_layer_fwd_tc_impl(fwd, z, w, rw, rb, b, in_scale, post, out_scale, 1, keep=keep, keep_scale=ks)
     null = _layer_fwd_tc_gate(fwd, z, w, rw, rb, b, in_scale, post, out_scale, keep, ks, None, None)
     assert_bitexact(null[0], ref_ex[0], "z_next, gate NULL")
     assert torch.equal(null[1], ref_ex[1])
@@ -295,13 +294,13 @@ def _ungate_layer1(model):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case, want", [
-    ("sm", 4), ("rw", 4), ("no_norm", 4), ("no_bias", 4), ("bwd_fused", 4),
+    ("sm", 4), ("rw", 4), ("no_norm", 4), ("no_bias", 4),
     ("width16", 0), ("x_requires_grad", 0), ("edge_gate_free", 0), ("mixed", 0), ("mean", 0), ("max", 0),
     ("edge_attr", 0), ("edge_weight", 0), ("degree_with_zeros", 0)])
 def test_gated_routing(monkeypatch, case, want):
-    """the gated stack (one by-source gate pass per layer) for sm / rw / no normalisation, with or without bias and
-    under MGCN_BWD_FUSED; the per-layer path for every excluded configuration"""
-    from meta_gcn_b200 import fused, ops
+    """the gated stack (one by-source gate pass per layer) for sm / rw / no normalisation, with or without bias; the
+    per-layer path for every excluded configuration"""
+    from meta_gcn_b200 import ops
     from meta_gcn_b200.gcn_meta.models import GCNModel
     from test_gpu_dropout import _graph, _inputs
     g = _graph(seed=5, num_nodes=6000, edge_entries=50000, evil=400)
@@ -314,8 +313,6 @@ def test_gated_routing(monkeypatch, case, want):
     cfg.update({"rw": dict(deg_norm="rw"), "no_norm": dict(deg_norm=None), "no_bias": dict(bias=False),
                 "width16": dict(enc_sizes=[16] * 4), "mean": dict(aggr="mean"), "max": dict(aggr="max"),
                 "edge_attr": dict(in_edgedim=3)}.get(case, {}))
-    if case == "bwd_fused":
-        monkeypatch.setattr(fused, "BWD_FUSED", True)
     torch.manual_seed(0)
     model = GCNModel(**cfg)
     if case == "edge_gate_free":

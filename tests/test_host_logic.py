@@ -109,6 +109,14 @@ def test_ops_refuse_cpu_tensors():
         GCNModel(1, [8], 2)(torch.ones(2, 1), ei)
 
 
+def test_layer_bwd_refuses_the_removed_mma_sync_kernel():
+    """ops.gcn_layer_bwd_impl runs on tcgen05 only: tensor_memory=False is refused before any tensor is looked at"""
+    from meta_gcn_b200 import ops
+    t, m = torch.ones(4, 32), torch.ones(32, 32)
+    with pytest.raises(ValueError, match="mma.sync"):
+        ops.gcn_layer_bwd_impl(t, t, t, m, m, None, None, False, False)
+
+
 def test_ops_trace_with_fake_tensors():
     import meta_gcn_b200.ops  # noqa: F401
     from torch._subclasses.fake_tensor import FakeTensorMode
